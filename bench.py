@@ -3,17 +3,19 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--only headline,gs_1024,...]
 
-ONE JSON line.  Its top level is the headline workload -- BASELINE.json configs[1]: gradient descent, 100 iterations,
-1024x1024, followed by the wavefront-mask add + 8-bit quantisation; a *step* is one batch of 32 such holograms per GPU,
-inputs resident in HBM, `value` = iterations/s summed over the ranks (weak scaling: every rank runs its own batch, the
-path has no collective).  `verified` says whether plane 0 of the timed batch reproduced the reference's error curve and
-8-bit frame (tests/golden/gd_noise_1024x1024_curves.npz, made by the unmodified reference).
+ONE JSON line on stdout.  Its top level is the headline workload -- BASELINE.json configs[1]: gradient descent, 100
+iterations, 1024x1024, followed by the wavefront-mask add + 8-bit quantisation; a *step* is one batch of 32 such
+holograms per GPU, inputs resident in HBM, `value` = iterations/s summed over the ranks (weak scaling: every rank runs
+its own batch, the path has no collective).  `verified` says whether plane 0 of the timed batch reproduced the
+reference's error curve and 8-bit frame (tests/golden/gd_noise_1024x1024_curves.npz, made by the unmodified reference).
 
 `e2e` is the same work through the reference-facing API with HOST buffers (algorithms.gradient_descent(target, args) ->
 numpy, then display_holograms.hologram_to_grey), host<->device copies inside the timed region, summed over the ranks.
 
-`configs` holds one sub-record per further workload of BASELINE.json, each timed like the headline (device events,
-warm-up, max over ranks):
+The line stays under 4 KB (tools that collect a run's output may keep only its tail): it ends with `summary`, one flat
+object with the main figure of every further workload.  The full record -- the same keys with every sub-record, the
+kernels' rooflines and notes -- is written to stderr as one JSON line.  Its `configs` holds one sub-record per further
+workload of BASELINE.json, each timed like the headline (device events, warm-up, max over ranks):
     gs_1024   Gerchberg-Saxton, batch 32 x 1024^2 x 100 iterations (the metric names GS and GD)
     fp64      GD and GS at 1024^2 in the fp64 parity mode
     config1   ONE 512x512 GS hologram, 20 iterations: device latency and through gerchberg_saxton(target, args)
@@ -28,6 +30,13 @@ warm-up, max over ranks):
 
 `--impl reference` times the CPU implementation (the oracle's numpy restatement of the reference, scipy.fft with all
 host threads) on a bounded sample of the headline workload.
+
+`--dump-outputs DIR` writes what the headline's last timed step computed on rank 0, so that two builds can be compared
+output for output (the inputs are seeded: the same arguments give the same inputs):
+    hologram.npy  float64 [batch, n]      the holograms at n pixels per plane (n <= 65536, the same pixels for every
+                                          plane, drawn without replacement by np.random.default_rng(0), in ascending order)
+    frames.npy    float32 [batch, n]      the 8-bit SLM frames (mask add + quantisation) at the same pixels
+    errors.npy    float64 [batch, loops]  every plane's error curve
 """
 from __future__ import annotations
 
@@ -69,7 +78,14 @@ def parse():
     p.add_argument("--slab-size", type=int, default=16384)
     p.add_argument("--workload", default="batch", choices=["batch", "slab"],
                    help="slab: only config5 as the line's own workload (one --size^2 plane row-split over the ranks)")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", default="",
+                   help="write the headline's outputs of its last timed step to DIR/<name>.npy (see the module docstring)")
+    a = p.parse_args()
+    if a.steps < 1:
+        p.error("--steps must be at least 1")
+    if a.dump_outputs and (a.impl != "b200" or a.workload != "batch"):
+        p.error("--dump-outputs writes the headline's outputs: it needs --impl b200 --workload batch")
+    return a
 
 
 def env_rank():
@@ -368,6 +384,7 @@ def batched_loop_record(h, a, alg, precision, shape, batch, loops, steps, warmup
 
     n0 = eng.launch_count()
     ms, step_ms, out = h.time_steps(step, max(warmup, 3), steps)
+    timed_res = state["res"]                         # the profiled re-run below replaces state["res"]
     launches = (eng.launch_count() - n0) * steps // (max(warmup, 3) + steps)
     iters = batch * loops * steps * h.world
     per_iter_s = ms * 1e-3 / (batch * loops * steps)
@@ -392,7 +409,7 @@ def batched_loop_record(h, a, alg, precision, shape, batch, loops, steps, warmup
             roof["note"] = ("one launch does what round 1's two did (max pass: read + write the transform, 16 B/px; gradient pass: 20 B/px -- "
                             "0.104 + 0.164 = 0.268 ms): it moves 20 B/px in 0.24 ms and is bound by the planes' barriers and the SM "
                             "(issue slots 32 % busy), not by DRAM; the whole iteration's fractions are in iteration_roofline")
-    state.update(eng=eng, targets=targets, norms=norms, during=during, x0=x0, x=x, out=out, step=step)
+    state.update(eng=eng, targets=targets, norms=norms, during=during, x0=x0, x=x, res=timed_res, out=out, step=step)
     return rec, state
 
 
@@ -415,6 +432,22 @@ def verify_headline(state, shape, loops, precision):
     ok = bool(ok_len and curve < tol and d.max() <= 1 and frac <= 2e-3)
     return ok, {"error_curve_max_rel": curve, "curve_tolerance": tol, "frame_max_lsb": int(d.max()), "frame_fraction_differing": frac, "frame_fraction_allowed": 2e-3,
                 "fixture": "tests/golden/gd_noise_1024x1024_curves.npz (unmodified reference, algorithms.py:60-112 + move_traps.py:135-140)"}
+
+
+def dump_outputs(out_dir, state):
+    """--dump-outputs: the headline's last timed step (module docstring), at most 64 MB in all."""
+    import torch
+    res, frames = state["res"], state["out"]
+    batch = frames.shape[0]
+    npx = frames[0].numel()
+    n = min(npx, 1 << 16, (48 << 20) // (12 * batch))            # 8 B (hologram) + 4 B (frame) per sampled pixel
+    idx = torch.from_numpy(np.sort(np.random.default_rng(0).choice(npx, size=n, replace=False))).to(frames.device)
+    arrays = {"hologram": res.hologram.reshape(batch, -1).index_select(1, idx).cpu().numpy(),
+              "frames": frames.reshape(batch, -1).index_select(1, idx).float().cpu().numpy(),
+              "errors": np.stack(res.errors).astype(np.float64)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, arr in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), arr)
 
 
 def run_b200(a):
@@ -451,6 +484,8 @@ def run_b200(a):
         verified, verification = verify_headline(st, shape, a.loops, a.precision)
     if verified is not None:
         verified = h.all_ok(verified)
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, st)
     csz = 8 if a.precision == "fp32" else 16
     line = {
         "metric": "GS/GD iterations/sec at 1024^2", "value": head["value"], "unit": "iterations/s", "n_gpus": world,
@@ -566,7 +601,9 @@ def run_b200(a):
     line["cpu_baseline"] = cpu
     line["configs"] = configs
     if rank == 0:
-        emit(line)
+        sys.stderr.write(json.dumps(line) + "\n")
+        sys.stderr.flush()
+        emit(result_line(line))
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
@@ -750,6 +787,52 @@ def run_slab(a):
         dist.destroy_process_group()
 
 
+# (summary key, path into the full record): the main figure of every further workload, in the order the run makes them
+SUMMARY = [
+    ("iteration_frac", ("iteration_roofline", "survey_model", "frac")),
+    ("single_ms", ("single_hologram", "ms_per_hologram")),
+    ("gs_1024_its", ("configs", "gs_1024", "value")),
+    ("fp64_gd_its", ("configs", "fp64", "gd", "value")),
+    ("fp64_gd_verified", ("configs", "fp64", "gd", "verified")),
+    ("fp64_gs_its", ("configs", "fp64", "gs", "value")),
+    ("s4096_gd_its", ("configs", "size_4096", "gd", "value")),
+    ("s4096_gs_its", ("configs", "size_4096", "gs", "value")),
+    ("c1_dev_ms", ("configs", "config1", "device_ms_per_hologram")),
+    ("c1_e2e_ms", ("configs", "config1", "e2e_ms_per_hologram")),
+    ("c3_u8_hps", ("configs", "config3", "uint8_frames", "holograms_per_s")),
+    ("c3_f64_hps", ("configs", "config3", "float64_holograms", "holograms_per_s")),
+    ("c3_u8_raster_hps", ("configs", "config3", "uint8_frames_device_rasterised", "holograms_per_s")),
+    ("c4_hps", ("configs", "config4", "holograms_per_s")),
+    ("c5_gs_its", ("configs", "config5", "value")),
+    ("c5_gd_its", ("configs", "config5_gd", "value")),
+]
+
+
+def result_line(full: dict) -> dict:
+    """The stdout line of the batch workload (module docstring): the headline's own keys without the prose, then
+    `summary`."""
+    line = {k: full[k] for k in ("metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per_step", "higher_is_better",
+                                 "scaling", "vs_baseline", "dtype", "data", "holograms_per_s", "gpu_launches", "clocks",
+                                 "verified")}
+    line["config"] = {k: full["config"][k] for k in ("workload", "algorithm", "shape", "batch_per_gpu", "iterations", "gd_form")}
+    line["verification"] = {k: v for k, v in full["verification"].items() if k != "fixture"}
+    if full.get("roofline"):
+        line["roofline"] = {k: v for k, v in full["roofline"].items() if k != "note"}
+    if full.get("cpu_baseline"):
+        line["cpu_baseline"] = {k: full["cpu_baseline"][k] for k in ("value", "unit", "cores", "kind")}
+    if full.get("e2e"):
+        line["e2e"] = {k: full["e2e"][k] for k in ("value", "unit", "h2d_bytes_per_step", "d2h_bytes_per_step", "ms_per_hologram")}
+    summary = {}
+    for key, path in SUMMARY:
+        v = full
+        for p in path:
+            v = v.get(p) if isinstance(v, dict) else None
+        if v is not None:
+            summary[key] = v
+    line["summary"] = summary
+    return line
+
+
 def emit(line: dict) -> None:
     """The ONE JSON line of this run, on the process's real stdout."""
     os.write(_REAL_STDOUT, (json.dumps(line) + "\n").encode())
@@ -758,6 +841,7 @@ def emit(line: dict) -> None:
 _REAL_STDOUT = 1
 
 if __name__ == "__main__":
+    sys.dont_write_bytecode = True      # a run leaves nothing in the source tree (which may be read-only)
     args = parse()
     # watchdog: a run that takes absurdly long (default 20 min; SLM_BENCH_WATCHDOG=seconds) dumps every thread's stack
     # to stderr and exits instead of hanging its launcher

@@ -1,5 +1,5 @@
-import sys, time, argparse, contextlib, io
-sys.path.insert(0,'/root/repo')
+import os, sys, time, argparse, contextlib, io
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
 from spatial_light_modulator_module_b200 import algorithms, display_holograms, host_logic as hl, synthetic
 from spatial_light_modulator_module_b200.engine import get_engine

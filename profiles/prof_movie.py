@@ -1,5 +1,5 @@
-import cProfile, pstats, sys, time, io
-sys.path.insert(0, "/root/repo")
+import os, cProfile, pstats, sys, time, io
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
 from spatial_light_modulator_module_b200 import generate_hologram_sequence as ghs, synthetic
 n = int(sys.argv[1]) if len(sys.argv) > 1 else 512

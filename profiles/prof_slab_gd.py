@@ -1,6 +1,6 @@
 """torchrun --nproc-per-node N profiles/prof_slab_gd.py [n]: per-kernel device times of slab GD iterations."""
 import os, sys, time
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch, torch.distributed as dist
 rank, local, world = int(os.environ.get("RANK", 0)), int(os.environ.get("LOCAL_RANK", 0)), int(os.environ.get("WORLD_SIZE", 1))
 torch.cuda.set_device(local)

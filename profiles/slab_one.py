@@ -1,7 +1,7 @@
 """One 16384^2 plane through the slab path on ONE GPU (world = 1), a few iterations of GS and GD: the command the ncu
 captures of the slab kernels are taken from (profiles/r2_ncu_slab.md)."""
-import sys
-sys.path.insert(0, "/root/repo")
+import os, sys
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
 from spatial_light_modulator_module_b200 import host_logic as hl
 from spatial_light_modulator_module_b200.slab import SlabEngine
