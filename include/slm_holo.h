@@ -115,8 +115,10 @@ int slm_trap_frames(slm_ctx* ctx, uint8_t* frames, int n_frames, int H, int W, c
 /* ---- one very large plane split by rows over the ranks (BASELINE config 5): slab-decomposed 2-D transform ----
  * Rank p owns `rows` = N/P rows of the N x N field.  A 2-D transform is: line transforms on the row slab,
  * exchange (pack -> all-to-all -> the peers' blocks side by side = the "exchange layout"), line transforms
- * on the received columns (now contiguous lines), exchange back.  The library supplies the kernels; the
- * all-to-all and the 4-scalar all-reduce are the caller's (NCCL through torch.distributed in slab.py).
+ * on the received columns (now contiguous lines), exchange back.  The library supplies the kernels.  The
+ * all-to-all and the 4-scalar all-gather are either the caller's collectives (NCCL through torch.distributed in
+ * slab.py) or this library's stores into the peers' memory (slm_transpose_blocks_peer, slm_rows_reduce with peers),
+ * ordered by the caller's device-side barriers.
  * GS does not depend on the transform's scale (only angle(A) is used), so these transforms are unnormalised. */
 int slm_rows_create(slm_ctx** out, int device, int rows, int W, int precision, void* cuda_stream);
 /* plain line transforms of every row: `in` complex<R> (or in_u8 + host lut[256] -> real input, algorithms.py:21,27);
@@ -130,18 +132,11 @@ int slm_rows_fft(slm_ctx* ctx, const void* in, const uint8_t* in_u8, const doubl
 int slm_rows_gs_row_pass(slm_ctx* ctx, const void* in, void* out, const void* inc_amp, int in_is_field, int final_pass,
                          double* hologram);
 /* Fourier-plane step (algorithms.py:31-38) on received columns in the exchange layout: finishes fft2, replaces
- * the amplitude, starts ifft2; per-line sums (max |C|^2, sum r^2, sum r*u, sum u^2 against scale_prev) go to
+ * the amplitude, starts ifft2; per-line sums (max |C|^2, sum r^2, sum r*u, sum u^2 against the previous iteration's
+ * scale, read from device memory at scale_prev_dev: the loop state stays on the device, see slm_rows_close) go to
  * partial[rows][4]; intensity (nullable, device double, same layout) receives |C|^2. */
 int slm_rows_gs_fourier_pass(slm_ctx* ctx, const void* in, void* out, int block_w, const uint8_t* target_u8,
-                             const double* amp_lut, double scale_prev, double* partial, double* intensity);
-/* The same with the previous iteration's scale read from device memory (loop state kept on the device: no host
- * round trip per iteration; see slm_rows_close). */
-int slm_rows_gs_fourier_pass_dev(slm_ctx* ctx, const void* in, void* out, int block_w, const uint8_t* target_u8,
-                                 const double* amp_lut, const double* scale_prev_dev, double* partial, double* intensity,
-                                 int line0, int nlines /* 0: all lines; else a part, so the way back of finished lines can start */);
-/* slm_rows_gs_row_pass (not the final pass, uniform illumination) on rows [row0, row0 + nrows) of the slab only: the
- * transposing stores of finished rows (slm_transpose_blocks_peer with a part) run beside the pass over the next rows. */
-int slm_rows_gs_row_pass_part(slm_ctx* ctx, const void* in, void* out, int in_is_field, int row0, int nrows);
+                             const double* amp_lut, const double* scale_prev_dev, double* partial, double* intensity);
 /* partial[rows][4] -> out4 (device double[4]: max, three sums) by one CTA in a fixed order.  With n_peers > 0 the four
  * numbers are also stored into every peer's gathered[self] (peer_gathered[r] = rank r's device double[n_peers][4],
  * mapped into this process: peer memory over NVLink) -- otherwise the caller all-gathers out4. */
@@ -178,15 +173,7 @@ int slm_transpose_blocks(slm_ctx* ctx, const void* in, void* out, int rows, int 
  * of it is written; from_exchange = 1: peers[q] is rank q's row slab, columns [self*rows, (self+1)*rows) are written.
  * The caller orders the ranks (a device-side barrier before the consumers run and before the buffers are reused). */
 int slm_transpose_blocks_peer(slm_ctx* ctx, const void* in, const void* const* peers, int n_peers, int self, int rows, int W,
-                              int elem_bytes, int from_exchange, int first, int count /* 0: everything; else rows (way out) or
-                              lines (way back) [first, first + count) */);
-
-/* Strided device-to-device copy on the context's stream (cudaMemcpy2DAsync): `rows` runs of width_bytes.  dst may be
- * peer memory; the copy engines move the blocks while the SMs compute (the slab path's overlapped exchange). */
-int slm_copy2d_async(slm_ctx* ctx, void* dst, size_t dst_pitch, const void* src, size_t src_pitch, size_t width_bytes, size_t rows);
-/* n such copies of one geometry (one block per peer) in one call. */
-int slm_copy2d_multi(slm_ctx* ctx, int n, void* const* dst, const void* const* src, size_t dst_pitch, size_t src_pitch,
-                     size_t width_bytes, size_t rows);
+                              int elem_bytes, int from_exchange);
 
 /* error_evolution and its length per plane (algorithms.py:25,39,93) of the last run.
  * err: host double[batch][max_loops]; iters: host int[batch].  Synchronises the stream. */

@@ -8,11 +8,8 @@ if world > 1:
     dist.init_process_group("nccl", device_id=torch.device("cuda", local))
 from spatial_light_modulator_module_b200.slab import SlabEngine
 n = int(sys.argv[1]) if len(sys.argv) > 1 else 16384
-for mode in ("copy", "store", "peer1", "coll"):
-    for k in ("SLM_SLAB_NO_PEER", "SLM_SLAB_PARTS", "SLM_SLAB_EXCHANGE"):
-        os.environ.pop(k, None)
-    os.environ.update({"copy": {"SLM_SLAB_PARTS": "4"}, "store": {"SLM_SLAB_PARTS": "4", "SLM_SLAB_EXCHANGE": "store"}, "peer1": {}, "coll": {"SLM_SLAB_NO_PEER": "1"}}[mode])
-    eng = SlabEngine(n, world, rank, "fp32")
+for mode in ("peer", "coll"):
+    eng = SlabEngine(n, world, rank, "fp32", peer=None if mode == "peer" else False)
     rows = n // world
     slab = eng._mem_upload((np.random.default_rng(100 + rank).random((rows, n)) * 255).astype(np.uint8))
     eng.gs(slab, 2, want_expected=False, on_device=True)
@@ -47,41 +44,6 @@ for mode in ("copy", "store", "peer1", "coll"):
     for _ in range(10): eng._exchange_back(S, Rv, X, cs, "X")
     e1.record(); torch.cuda.synchronize()
     if rank == 0: print(f"    exchange back: {e0.elapsed_time(e1)/10:.3f} ms each")
-    if peer and getattr(eng, "_how", "") == "copy":
-        B = eng._peer["comm_stream"]
-        part = rows // eng._parts
-        for rows_part, name in ((True, "copy engines, way out (strided runs)"), (False, "copy engines, way back (contiguous)")):
-            torch.cuda.synchronize(); dist.barrier()
-            e0.record(B)
-            for _ in range(5):
-                for j in range(eng._parts):
-                    eng._copy_blocks(S, "Rv" if rows_part else "Rb", j * part, part, cs, rows_part)
-            e1.record(B); torch.cuda.synchronize()
-            if rank == 0: print(f"    {name}: {e0.elapsed_time(e1)/5:.3f} ms per exchange ({rows*n*cs*(world-1)/world/1e6/(e0.elapsed_time(e1)/5)*1e-3*1e3:.0f} GB/s to the peers)")
-        # the passes alone (engine stream), then passes + copies together
-        Tx = eng._peer_view("Tx", (world, rows, rows), np.uint8)
-        state = eng._mem_upload(np.array([1.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0])); partial = eng._mem_empty((rows, 4), np.float64)
-        Y = eng._peer_view("Y", eng.shape, np.complex64)
-        torch.cuda.synchronize(); dist.barrier()
-        e0.record()
-        for _ in range(5):
-            for j in range(eng._parts):
-                eng._check(eng._lib.slm_rows_gs_row_pass_part(eng._ctx, eng._mem_ptr(X), eng._mem_ptr(Y), 0, j * part, part))
-            for j in range(eng._parts):
-                eng._fourier(Rv, S, Tx, state, partial, None, j * part, part)
-        e1.record(); torch.cuda.synchronize()
-        if rank == 0: print(f"    the two passes alone: {e0.elapsed_time(e1)/5:.3f} ms per iteration")
-        torch.cuda.synchronize(); dist.barrier()
-        e0.record()
-        for _ in range(5):
-            for j in range(eng._parts):
-                eng._check(eng._lib.slm_rows_gs_row_pass_part(eng._ctx, eng._mem_ptr(X), eng._mem_ptr(Y), 0, j * part, part))
-                eng._copy_blocks(S, "Rv", j * part, part, cs, True)
-            for j in range(eng._parts):
-                eng._fourier(Rv, S, Tx, state, partial, None, j * part, part)
-                eng._copy_blocks(S, "Rb", j * part, part, cs, False)
-        e1.record(); eng._after(eng._stream, B); e1.record(); torch.cuda.synchronize()
-        if rank == 0: print(f"    passes + unordered copies on the second stream: {e0.elapsed_time(e1)/5:.3f} ms per iteration")
     if peer:
         e0.record()
         for _ in range(20): eng._peer_barrier()

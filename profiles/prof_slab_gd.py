@@ -10,10 +10,7 @@ from spatial_light_modulator_module_b200 import host_logic as hl
 from spatial_light_modulator_module_b200.slab import SlabEngine
 n = int(sys.argv[1]) if len(sys.argv) > 1 else 16384
 for mode in ("peer", "coll"):
-    os.environ.pop("SLM_SLAB_NO_PEER", None)
-    if mode == "coll":
-        os.environ["SLM_SLAB_NO_PEER"] = "1"
-    eng = SlabEngine(n, world, rank, "fp32")
+    eng = SlabEngine(n, world, rank, "fp32", peer=None if mode == "peer" else False)
     rows = n // world
     slab = eng._mem_upload((np.random.default_rng(100 + rank).random((rows, n)) * 255).astype(np.uint8))
     u = eng._mem_upload(np.random.default_rng(200 + rank).random((rows, n)))

@@ -41,18 +41,14 @@ SIGNATURES = {
     "slm_rows_create": (_i, [C.POINTER(_vp), _i, _i, _i, _i, _vp]),
     "slm_rows_fft": (_i, [_vp, _vp, _vp, _dp, _vp, _i, _i, _i]),
     "slm_rows_gs_row_pass": (_i, [_vp, _vp, _vp, _vp, _i, _i, _vp]),
-    "slm_rows_gs_fourier_pass": (_i, [_vp, _vp, _vp, _i, _vp, _dp, _d, _vp, _vp]),
-    "slm_rows_gs_fourier_pass_dev": (_i, [_vp, _vp, _vp, _i, _vp, _dp, _vp, _vp, _vp, _i, _i]),
-    "slm_rows_gs_row_pass_part": (_i, [_vp, _vp, _vp, _i, _i, _i]),
+    "slm_rows_gs_fourier_pass": (_i, [_vp, _vp, _vp, _i, _vp, _dp, _vp, _vp, _vp]),
     "slm_rows_reduce": (_i, [_vp, _vp, _i, _vp, _vp, _i, _i]),
     "slm_rows_close": (_i, [_vp, _vp, _i, _d, _d, _i, _d, _vp, _vp]),
     "slm_rows_reset": (_i, [_vp]),
     "slm_rows_gd_row_pass": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _vp]),
     "slm_rows_gd_fourier_pass": (_i, [_vp, _vp, _vp, _i, _vp, _dp, _d, _vp, _vp, _vp, _i]),
     "slm_transpose_blocks": (_i, [_vp, _vp, _vp, _i, _i, _i, _i]),
-    "slm_copy2d_async": (_i, [_vp, _vp, C.c_size_t, _vp, C.c_size_t, C.c_size_t, C.c_size_t]),
-    "slm_copy2d_multi": (_i, [_vp, _i, _vp, _vp, C.c_size_t, C.c_size_t, C.c_size_t, C.c_size_t]),
-    "slm_transpose_blocks_peer": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i]),
+    "slm_transpose_blocks_peer": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i, _i]),
     "slm_read_curves": (_i, [_vp, _i, _i, _dp, _ip]),
     "slm_expected_outcome": (_i, [_vp, _i, _vp, _dp, _vp]),
     "slm_deflect_phase": (_i, [_vp, _i, _i, _d, _d, _d, _vp]),

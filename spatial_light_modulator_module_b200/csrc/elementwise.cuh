@@ -244,7 +244,7 @@ SLM_GLOBAL void transpose_blocks_kernel(const T* in, T* out, int h, int W, int f
 // The stores ARE the all-to-all: the blocks cross the links while the tiles are being transposed.
 struct PeerPtrs { void* p[16]; };
 template <typename T>
-SLM_GLOBAL void transpose_blocks_peer_kernel(const T* in, PeerPtrs peers, int h, int W, int from_exchange, int self, int i0, int c0, int n_x) {
+SLM_GLOBAL void transpose_blocks_peer_kernel(const T* in, PeerPtrs peers, int h, int W, int from_exchange, int self, int n_x) {
     SLM_STATIC_SMEM T tile[32][33];
     // Destinations vary FASTEST over the grid and start behind this rank: at any moment a rank's CTAs write to all
     // peers at once, and no two ranks begin with the same one.  (With the peer as the slowest index every rank stored
@@ -252,7 +252,7 @@ SLM_GLOBAL void transpose_blocks_peer_kernel(const T* in, PeerPtrs peers, int h,
     // on 8 GPUs at 16384^2: 1.2 ms per exchange of 117 MB per rank, the time of 940 MB through ONE port.)
     const int np = gridDim.x / n_x;
     const int q = (blockIdx.x % np + self + 1) % np;
-    const int tc = c0 + blockIdx.y * 32, ti = i0 + (blockIdx.x / np) * 32;              // (i0, c0: the part of every block this launch moves)
+    const int tc = blockIdx.y * 32, ti = (blockIdx.x / np) * 32;
     const int tx = threadIdx.x % 32, ty = threadIdx.x / 32;
     T* out = static_cast<T*>(peers.p[q]);
     if (!from_exchange) {

@@ -390,7 +390,7 @@ template <class F> static int replay_iterations(slm_ctx* c, int batch, int times
 }
 
 extern "C" const char* slm_last_error(void) { return g_err.c_str(); }
-extern "C" int slm_version(void) { return 100; }
+extern "C" int slm_version(void) { return 101; }
 extern "C" int slm_supported_lengths(int* out, int cap) { return supported_lengths(out, cap); }
 
 extern "C" void slm_ctx_destroy(slm_ctx* c) {
@@ -885,49 +885,15 @@ extern "C" int slm_rows_gs_row_pass(slm_ctx* c, const void* in, void* out, const
     return 0;
 }
 
-extern "C" int slm_rows_gs_row_pass_part(slm_ctx* c, const void* in, void* out, int in_is_field, int row0, int nrows) {
-    if (!c || !in || !out) return fail(SLM_ERR_ARG, "slm_rows_gs_row_pass_part: bad argument");
-    if (row0 < 0 || nrows < 1 || row0 + nrows > c->H || row0 % c->row->rows_per_cta || nrows % c->row->rows_per_cta)
-        return fail(SLM_ERR_ARG, "slm_rows_gs_row_pass_part: bad row range");
-    SLM_CUDA(cudaSetDevice(c->device));
-    const size_t cs = 2 * real_size(c->prec), off = (size_t)row0 * c->W;
-    const size_t cs_in = in_is_field == 2 ? 2 * sizeof(float) : cs;
-    const char* src = static_cast<const char*>(in) + off * cs_in;
-    RowArgs ra{};
-    ra.B = 1; ra.H = nrows; ra.Y = src; ra.field = src; ra.A32 = src; ra.X = static_cast<char*>(out) + off * cs; ra.stats = c->stats;
-    ra.inv_hw = 1.0; ra.tw = c->tw_row;
-    ra.source = in_is_field == 2 ? ROW_FROM_A32 : (in_is_field ? ROW_FROM_A : ROW_FROM_Y);
-    SLM_TIMED(K_ROW_PASS, c->row->row_pass(ALG_GS, ra, c->stream));
-    return 0;
-}
-
 extern "C" int slm_rows_gs_fourier_pass(slm_ctx* c, const void* in, void* out, int block_w, const uint8_t* target_u8,
-                                        const double* amp_lut, double scale_prev, double* partial, double* intensity) {
-    if (!c || !in || !out || !target_u8 || !amp_lut || !partial) return fail(SLM_ERR_ARG, "slm_rows_gs_fourier_pass: bad argument");
+                                        const double* amp_lut, const double* scale_prev_dev, double* partial, double* intensity) {
+    if (!c || !in || !out || !target_u8 || !amp_lut || !partial || !scale_prev_dev) return fail(SLM_ERR_ARG, "slm_rows_gs_fourier_pass: bad argument");
     if (!block_width_ok(c, block_w))
         return fail(SLM_ERR_SHAPE, "slm_rows_gs_fourier_pass: the exchange block width must be a power-of-two multiple of the line's thread count");
     SLM_CUDA(cudaSetDevice(c->device));
     SLM_TRY(upload_lut(c, amp_lut));
     RowFourierArgs fa{};
-    fa.rows = c->H; fa.block_w = block_w; fa.in = in; fa.out = out; fa.T8 = target_u8; fa.lut = c->lut; fa.s0 = scale_prev;
-    fa.partial = partial; fa.intensity = intensity; fa.tw = c->tw_row;
-    SLM_TIMED(K_COL_PASS, c->row->row_fourier(fa, c->stream));
-    return 0;
-}
-
-extern "C" int slm_rows_gs_fourier_pass_dev(slm_ctx* c, const void* in, void* out, int block_w, const uint8_t* target_u8,
-                                            const double* amp_lut, const double* scale_prev_dev, double* partial, double* intensity,
-                                            int line0, int nlines) {
-    if (!c || !in || !out || !target_u8 || !amp_lut || !partial || !scale_prev_dev) return fail(SLM_ERR_ARG, "slm_rows_gs_fourier_pass_dev: bad argument");
-    if (line0 < 0 || nlines < 0 || line0 + nlines > c->H || line0 % c->row->rows_per_cta || nlines % c->row->rows_per_cta)
-        return fail(SLM_ERR_ARG, "slm_rows_gs_fourier_pass_dev: bad line range");
-    if (!block_width_ok(c, block_w))
-        return fail(SLM_ERR_SHAPE, "slm_rows_gs_fourier_pass_dev: the exchange block width must be a power-of-two multiple of the line's thread count");
-    SLM_CUDA(cudaSetDevice(c->device));
-    SLM_TRY(upload_lut(c, amp_lut));
-    RowFourierArgs fa{};
-    fa.rows = c->H; fa.block_w = block_w; fa.in = in; fa.out = out; fa.T8 = target_u8; fa.lut = c->lut; fa.s0 = 0.0; fa.s0_dev = scale_prev_dev;
-    fa.row0 = line0; fa.nrows = nlines;
+    fa.rows = c->H; fa.block_w = block_w; fa.in = in; fa.out = out; fa.T8 = target_u8; fa.lut = c->lut; fa.s0_dev = scale_prev_dev;
     fa.partial = partial; fa.intensity = intensity; fa.tw = c->tw_row;
     SLM_TIMED(K_COL_PASS, c->row->row_fourier(fa, c->stream));
     return 0;
@@ -996,51 +962,22 @@ extern "C" int slm_rows_gd_fourier_pass(slm_ctx* c, const void* in, void* out, i
 }
 
 extern "C" int slm_transpose_blocks_peer(slm_ctx* c, const void* in, const void* const* peers, int n_peers, int self, int rows, int W,
-                                         int elem_bytes, int from_exchange, int first, int count) {
+                                         int elem_bytes, int from_exchange) {
     if (!c || !in || n_peers < 1 || self < 0 || self >= n_peers) return fail(SLM_ERR_ARG, "slm_transpose_blocks_peer: bad argument");
     if (rows < 32 || rows % 32 || W != rows * n_peers) return fail(SLM_ERR_SHAPE, "slm_transpose_blocks_peer: W must be rows * peers, rows a multiple of 32");
-    if (count == 0) { first = 0; count = rows; }
-    if (first < 0 || count < 32 || first % 32 || count % 32 || first + count > rows) return fail(SLM_ERR_ARG, "slm_transpose_blocks_peer: bad part");
     SLM_CUDA(cudaSetDevice(c->device));
     PeerPtrs pp;
     SLM_TRY(peer_ptrs(peers, n_peers, &pp, "slm_transpose_blocks_peer"));
-    // a part: rows [first, first + count) of the slab on the way out, lines [first, first + count) on the way back
-    const int i0 = from_exchange ? 0 : first, c0 = from_exchange ? first : 0;
-    const int n_x = (from_exchange ? rows : count) / 32;
-    const dim3 grid(n_x * (W / rows), (from_exchange ? count : rows) / 32, 1), block(256);             // x: (tile, destination), destination fastest
+    const int n_x = rows / 32;
+    const dim3 grid(n_x * n_peers, rows / 32, 1), block(256);             // x: (tile, destination), destination fastest
     {
         LaunchTimer t_(c, K_ELEMENTWISE);
-        if (elem_bytes == 16) SLM_LAUNCH((transpose_blocks_peer_kernel<cpx<double>>), grid, block, 0, c->stream, static_cast<const cpx<double>*>(in), pp, rows, W, from_exchange, self, i0, c0, n_x);
-        else if (elem_bytes == 8) SLM_LAUNCH((transpose_blocks_peer_kernel<double>), grid, block, 0, c->stream, static_cast<const double*>(in), pp, rows, W, from_exchange, self, i0, c0, n_x);
-        else if (elem_bytes == 1) SLM_LAUNCH((transpose_blocks_peer_kernel<unsigned char>), grid, block, 0, c->stream, static_cast<const unsigned char*>(in), pp, rows, W, from_exchange, self, i0, c0, n_x);
+        if (elem_bytes == 16) SLM_LAUNCH((transpose_blocks_peer_kernel<cpx<double>>), grid, block, 0, c->stream, static_cast<const cpx<double>*>(in), pp, rows, W, from_exchange, self, n_x);
+        else if (elem_bytes == 8) SLM_LAUNCH((transpose_blocks_peer_kernel<double>), grid, block, 0, c->stream, static_cast<const double*>(in), pp, rows, W, from_exchange, self, n_x);
+        else if (elem_bytes == 1) SLM_LAUNCH((transpose_blocks_peer_kernel<unsigned char>), grid, block, 0, c->stream, static_cast<const unsigned char*>(in), pp, rows, W, from_exchange, self, n_x);
         else return fail(SLM_ERR_ARG, "slm_transpose_blocks_peer: elem_bytes must be 1, 8 or 16");
     }
     SLM_CUDA(cudaGetLastError());
-    return 0;
-}
-
-extern "C" int slm_copy2d_async(slm_ctx* c, void* dst, size_t dst_pitch, const void* src, size_t src_pitch, size_t width_bytes, size_t rows) {
-    if (!c || !dst || !src || !width_bytes || !rows || dst_pitch < width_bytes || src_pitch < width_bytes)
-        return fail(SLM_ERR_ARG, "slm_copy2d_async: bad argument");
-    SLM_CUDA(cudaSetDevice(c->device));
-#ifdef SLM_EMULATE
-    for (size_t r = 0; r < rows; ++r) memcpy(static_cast<char*>(dst) + r * dst_pitch, static_cast<const char*>(src) + r * src_pitch, width_bytes);
-#else
-    // device to device, possibly to ANOTHER device's memory mapped into this process: the copy engines carry it
-    // (over NVLink) while the SMs run the passes
-    if (dst_pitch == width_bytes && src_pitch == width_bytes)
-        SLM_CUDA(cudaMemcpyAsync(dst, src, width_bytes * rows, cudaMemcpyDeviceToDevice, c->stream));
-    else
-        SLM_CUDA(cudaMemcpy2DAsync(dst, dst_pitch, src, src_pitch, width_bytes, rows, cudaMemcpyDeviceToDevice, c->stream));
-#endif
-    c->launches++;
-    return 0;
-}
-
-extern "C" int slm_copy2d_multi(slm_ctx* c, int n, void* const* dst, const void* const* src, size_t dst_pitch, size_t src_pitch,
-                                size_t width_bytes, size_t rows) {
-    if (!c || n < 0 || (n && (!dst || !src))) return fail(SLM_ERR_ARG, "slm_copy2d_multi: bad argument");
-    for (int i = 0; i < n; ++i) SLM_TRY(slm_copy2d_async(c, dst[i], dst_pitch, src[i], src_pitch, width_bytes, rows));
     return 0;
 }
 

@@ -150,9 +150,7 @@ struct RowFourierArgs {
     void* out;               // complex<R>: lines ready for the return exchange
     const uint8_t* T8;       // target, same layout as `in`
     const void* lut;         // R[256] amplitude by grey level
-    double s0;               // scale of the previous iteration (algorithms.py:37) ...
-    const double* s0_dev;    // ... or, when not null, where it lies in device memory (loop state kept on the device)
-    int row0, nrows;         // the lines [row0, row0 + nrows) only (nrows == 0: all) -- chunks that overlap the exchange
+    const double* s0_dev;    // RF_GS: scale of the previous iteration (algorithms.py:37), in device memory (loop state)
     int mode;                // RowFourierMode
     double norm;             // RF_GD_POST: amax(T) (algorithms.py:74)
     const double* state;     // RF_GD_POST: device loop state {norm/max, error, iterations, ended, max} (slm_rows_close)

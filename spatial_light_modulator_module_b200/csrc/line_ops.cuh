@@ -124,7 +124,7 @@ template <typename R, int L> struct RowLaunch {
         return check();
     }
     static int row_fourier(const RowFourierArgs& a, cudaStream_t s) {
-        const dim3 grid((unsigned)((a.nrows ? a.nrows : a.rows) / RG::NR)), block(RG::THREADS);
+        const dim3 grid((unsigned)(a.rows / RG::NR)), block(RG::THREADS);
         if (a.mode == RF_GD_MAX) SLM_LAUNCH((row_fourier_kernel<R, L, RF_GD_MAX>), grid, block, RG::SMEM, s, a);
         else if (a.mode == RF_GD_POST) SLM_LAUNCH((row_fourier_kernel<R, L, RF_GD_POST>), grid, block, RG::SMEM, s, a);
         else SLM_LAUNCH((row_fourier_kernel<R, L, RF_GS>), grid, block, RG::SMEM, s, a);

@@ -553,7 +553,7 @@ SLM_GLOBAL void SLM_LAUNCH_BOUNDS((RowGeom<R, W>::THREADS), (RowGeom<R, W>::MIN_
     constexpr bool HAS_T = MODE != RF_GD_MAX;                 // needs the target's grey levels and a table
     SLM_DYN_SMEM(raw);
     const int t = threadIdx.x, rr = t / M, j = t % M;
-    const long long row = (long long)a.row0 + (long long)blockIdx.x * G::NR + rr;
+    const long long row = (long long)blockIdx.x * G::NR + rr;
     cpx<R>* line = reinterpret_cast<cpx<R>*>(raw) + (size_t)rr * P::NP;
     const typename G::Sync sync{1 + rr / G::LPG};
     const cpx<R>* tw = static_cast<const cpx<R>*>(a.tw);
@@ -564,7 +564,7 @@ SLM_GLOBAL void SLM_LAUNCH_BOUNDS((RowGeom<R, W>::THREADS), (RowGeom<R, W>::MIN_
     // (one CTA per SM and nothing to hide a global load behind)
     SLM_STATIC_SMEM R lut_s[256];
     if (HAS_T) for (int i = t; i < 256; i += G::THREADS) lut_s[i] = ld_ro(lut + i);
-    const R s0r = MODE == RF_GS ? (R)(a.s0_dev ? ld_cg(a.s0_dev) : a.s0) : (R)0;
+    const R s0r = MODE == RF_GS ? (R)ld_cg(a.s0_dev) : (R)0;
     const double gd_scale = MODE == RF_GD_POST ? ld_cg(a.state) : 0.0, gd_max = MODE == RF_GD_POST ? ld_cg(a.state + 4) : 0.0;
     sync_cta();
     cpx<R> v[E];

@@ -28,8 +28,8 @@ Two ways of moving the blocks:
 from __future__ import annotations
 
 import ctypes as C
-import os
 import time
+from types import SimpleNamespace
 
 import numpy as np
 
@@ -68,8 +68,6 @@ class SlabEngine(Engine):
     def _peer_setup(self, required: bool):
         """One symmetric allocation per rank holding its two row slabs, its receive buffer and the gathered reduction
         numbers; every rank learns the others' base pointers (torch's symmetric memory does the mapping)."""
-        if os.environ.get("SLM_SLAB_NO_PEER"):
-            return
         try:
             torch = self._torch
             import torch.distributed as dist
@@ -78,7 +76,7 @@ class SlabEngine(Engine):
             plane = self.rows * self.n * cs
             align = lambda v: (v + 1023) // 1024 * 1024       # noqa: E731
             offs, total = {}, 0
-            for name, size in (("X", plane), ("Y", plane), ("Rv", plane), ("Rb", plane), ("Tx", self.rows * self.n),
+            for name, size in (("X", plane), ("Y", plane), ("Rv", plane), ("Tx", self.rows * self.n),
                                ("gathered", 2 * self.world * 32)):
                 offs[name] = total
                 total += align(size)
@@ -89,38 +87,8 @@ class SlabEngine(Engine):
             ptrs = [int(p) for p in hdl.buffer_ptrs]
             if len(ptrs) != self.world:
                 raise RuntimeError("symmetric memory handle does not cover the group")
-            # a second stream (and a library context bound to it) carries the transposing stores, so that the blocks of
-            # the rows / lines already done cross the links while the pass works on the next ones
-            comm_stream = torch.cuda.Stream(self._dev)
-            comm_ctx = C.c_void_p()
-            _ffi.check(self._lib, self._lib.slm_rows_create(C.byref(comm_ctx), self._device_index, self.rows, self.n,
-                                                            _PREC[self.precision], C.c_void_p(comm_stream.cuda_stream)))
-            # optional further streams (and contexts) so that the copies to different peers run on different copy engines at
-            # once: measured at 4 GPUs it does not raise the bandwidth (460-510 GB/s to the peers either way) and costs the
-            # passes more (32.1 instead of 28.4 ms per 10 iterations), so one lane is the default
-            lanes = []
-            for _ in range(min(self.world - 1, int(os.environ.get("SLM_SLAB_COPY_LANES", "1"))) - 1):
-                st = torch.cuda.Stream(self._dev)
-                cx = C.c_void_p()
-                _ffi.check(self._lib, self._lib.slm_rows_create(C.byref(cx), self._device_index, self.rows, self.n,
-                                                                _PREC[self.precision], C.c_void_p(st.cuda_stream)))
-                lanes.append((st, cx))
-            self._peer = {"buf": buf, "hdl": hdl, "ptrs": ptrs, "offs": offs, "comm_stream": comm_stream, "comm_ctx": comm_ctx,
-                          "lanes": lanes}
-            # A pass can be cut in parts whose blocks travel (second stream) while the next part is computed.  Measured at
-            # 16384^2 with the stores of the exchange spread over all peers (elementwise.cuh): one part -- pass, then ONE
-            # storing kernel, then the barrier -- is as fast or faster at every size of the group (2 GPUs 227 = 227, 4 GPUs
-            # 414 against 400, 8 GPUs 736 against 732 (stores in parts) / 575 (copy engines) iterations/s): what the overlap
-            # hides it takes back as memory contention, events and small kernels.  So one part is the default.
-            parts = int(os.environ.get("SLM_SLAB_PARTS", "1"))
-            self._parts = parts if parts > 1 and self.rows % (32 * parts) == 0 else 1
-            # how the blocks travel when a pass is split in parts: "copy" -- packed by a local transposing kernel, then moved
-            # by the COPY ENGINES into the peers' memory while the SMs go on with the next part (the passes hold the whole
-            # register file, so a storing kernel cannot run beside them); "store" -- the transposing kernel stores straight
-            # into the peers' memory (between the parts)
-            self._how = os.environ.get("SLM_SLAB_EXCHANGE", "copy") if self._parts > 1 else "store"
-            self.peer_status = (f"peer memory (torch symmetric memory over NVLink; {self._parts} part(s) per pass, "
-                                f"{'copy engines beside the passes' if self._how == 'copy' else 'transposing stores'})")
+            self._peer = {"buf": buf, "hdl": hdl, "ptrs": ptrs, "offs": offs}
+            self.peer_status = "peer memory (torch symmetric memory over NVLink; transposing stores)"
         except Exception as exc:                  # no symmetric memory on this system: keep the collectives
             self._peer = None
             self.peer_status = f"collectives (peer memory unavailable: {type(exc).__name__}: {exc})"
@@ -209,7 +177,7 @@ class SlabEngine(Engine):
             return
         if self._peer is not None and peer_name is not None:
             self._check(self._lib.slm_transpose_blocks_peer(self._ctx, self._mem_ptr(slab), self._peer_array(peer_name), self.world,
-                                                            self.rank, self.rows, self.n, elem_bytes, 0, 0, 0))
+                                                            self.rank, self.rows, self.n, elem_bytes, 0))
             self._peer_barrier()                 # every block of `recv` has landed (and every rank is done with `slab`)
             return
         self._transpose(slab, send, elem_bytes, False)
@@ -222,120 +190,98 @@ class SlabEngine(Engine):
             return
         if self._peer is not None and peer_name is not None:
             self._check(self._lib.slm_transpose_blocks_peer(self._ctx, self._mem_ptr(lines), self._peer_array(peer_name), self.world,
-                                                            self.rank, self.rows, self.n, elem_bytes, 1, 0, 0))
+                                                            self.rank, self.rows, self.n, elem_bytes, 1))
             self._peer_barrier()
             return
         self._all_to_all(lines, recv)
         self._transpose(recv, slab, elem_bytes, True)
 
-    # ---- one GS iteration with the exchange overlapped (peer memory, several parts per pass) ------------------------
-    def _after(self, waiter, stream):
-        """`waiter` (a stream) waits for what `stream` has been given so far"""
-        ev = self._torch.cuda.Event()
-        ev.record(stream)
-        waiter.wait_event(ev)
-
-    def _row_pass_and_push(self, src, cur, field, cs):
-        """SLM-plane pass over the slab in parts; the blocks of a finished part are stored into the peers' receive buffers
-        (comm stream) while the pass works on the next part.  Returns with the engine's stream waiting for the barrier."""
-        A, B, part = self._stream, self._peer["comm_stream"], self.rows // self._parts
-        peers = self._peer_array("Rv")
-        for j in range(self._parts):
-            self._check(self._lib.slm_rows_gs_row_pass_part(self._ctx, self._mem_ptr(src), self._mem_ptr(cur), int(field), j * part, part))
-            self._after(B, A)
-            self._check(self._lib.slm_transpose_blocks_peer(self._peer["comm_ctx"], self._mem_ptr(cur), peers, self.world, self.rank,
-                                                            self.rows, self.n, cs, 0, j * part, part))
-        with self._torch.cuda.stream(B):
-            self._peer["hdl"].barrier(channel=0)          # every rank's blocks have landed
-        self._after(A, B)
-
-    def _fourier_and_push_back(self, Rv, S, Tx, state, partial, inten, cur_name, cs, mine, slot):
-        """Fourier-plane pass over this rank's lines in parts; finished lines go back into the peers' row slabs meanwhile.
-        Ends with this rank's four sums stored on every rank and all ranks past the barrier."""
-        A, B, part = self._stream, self._peer["comm_stream"], self.rows // self._parts
-        peers = self._peer_array(cur_name)
-        for j in range(self._parts):
-            self._fourier(Rv, S, Tx, state, partial, inten, j * part, part)
-            self._after(B, A)
-            self._check(self._lib.slm_transpose_blocks_peer(self._peer["comm_ctx"], self._mem_ptr(S), peers, self.world, self.rank,
-                                                            self.rows, self.n, cs, 1, j * part, part))
-        self._check(self._lib.slm_rows_reduce(self._ctx, self._mem_ptr(partial), self.rows, self._mem_ptr(mine),
-                                              self._peer_array("gathered", slot * self.world * 32), self.world, self.rank))
-        self._after(B, A)
-        with self._torch.cuda.stream(B):
-            self._peer["hdl"].barrier(channel=0)          # the lines are back in the slabs, the sums on every rank
-        self._after(A, B)
-
-    # ---- the same with the COPY ENGINES moving the blocks while the SMs compute ------------------------------------------
-    def _copy_blocks(self, src_buf, dst_name, first, count, cs, rows_part):
-        """comm stream: my blocks for every peer -> the peer's buffer `dst_name`, block `self.rank`.  rows_part: the part is
-        a range of slab rows i (way out: [q][c][i in part] -- h runs of `count` elements); else a range of lines c (way
-        back: [q][c in part][i] -- one contiguous run)."""
-        h = self.rows
-        B = self._peer["comm_stream"]
-        lanes = [(B, self._peer["comm_ctx"])] + self._peer["lanes"]     # (optionally copies to different peers on different streams)
-        for st, _ in lanes[1:]:
-            self._after(st, B)
-        base = self._mem_ptr(src_buf).value
-        dst_off = self._peer["offs"][dst_name]
-        off = (first if rows_part else first * h)
-        per_lane = [([], []) for _ in lanes]
-        for d in range(1, self.world + 1):                         # start with the neighbour: the ranks do not all hit rank 0 first
-            q = (self.rank + d) % self.world
-            dsts, srcs = per_lane[d % len(lanes)]
-            srcs.append(base + (q * h * h + off) * cs)
-            dsts.append(self._peer["ptrs"][q] + dst_off + (self.rank * h * h + off) * cs)
-        for (_, ctx), (dsts, srcs) in zip(lanes, per_lane):
-            if not dsts:
-                continue
-            n = len(dsts)
-            da, sa = (C.c_void_p * n)(*dsts), (C.c_void_p * n)(*srcs)
-            if rows_part:
-                self._check(self._lib.slm_copy2d_multi(ctx, n, da, sa, h * cs, h * cs, count * cs, h))
-            else:
-                self._check(self._lib.slm_copy2d_multi(ctx, n, da, sa, count * h * cs, count * h * cs, count * h * cs, 1))
-        for st, _ in lanes[1:]:
-            self._after(B, st)
-
-    def _pack_ptrs(self, S):
-        """peer-pointer table that makes slm_transpose_blocks_peer write block q of the LOCAL buffer S (it writes block
-        `self.rank` of table entry q)"""
-        cs = np.dtype(self.complex_dtype).itemsize
-        base = self._mem_ptr(S).value
-        return (C.c_void_p * self.world)(*[base + (q - self.rank) * self.rows * self.rows * cs for q in range(self.world)])
-
-    def _row_pass_and_copy(self, src, cur, field, S, cs):
-        A, B, part = self._stream, self._peer["comm_stream"], self.rows // self._parts
-        pack = self._pack_ptrs(S)
-        for j in range(self._parts):
-            self._check(self._lib.slm_rows_gs_row_pass_part(self._ctx, self._mem_ptr(src), self._mem_ptr(cur), int(field), j * part, part))
-            self._check(self._lib.slm_transpose_blocks_peer(self._ctx, self._mem_ptr(cur), pack, self.world, self.rank, self.rows, self.n,
-                                                            cs, 0, j * part, part))          # pack: [q][c][i in part] of S
-            self._after(B, A)
-            self._copy_blocks(S, "Rv", j * part, part, cs, True)
-        with self._torch.cuda.stream(B):
-            self._peer["hdl"].barrier(channel=0)
-        self._after(A, B)
-
-    def _fourier_and_copy_back(self, Rv, S, Rb, Tx, state, partial, inten, cur, cs, mine, slot):
-        A, B, part = self._stream, self._peer["comm_stream"], self.rows // self._parts
-        self._after(B, A)                                          # (the comm stream's copies out of S are over: ordered by the barrier)
-        for j in range(self._parts):
-            self._fourier(Rv, S, Tx, state, partial, inten, j * part, part)
-            self._after(B, A)
-            self._copy_blocks(S, "Rb", j * part, part, cs, False)
-        self._check(self._lib.slm_rows_reduce(self._ctx, self._mem_ptr(partial), self.rows, self._mem_ptr(mine),
-                                              self._peer_array("gathered", slot * self.world * 32), self.world, self.rank))
-        self._after(B, A)
-        with self._torch.cuda.stream(B):
-            self._peer["hdl"].barrier(channel=0)
-        self._after(A, B)
-        self._transpose(Rb, cur, cs, True)                         # unpack: the lines of every rank -> my rows
-
     def _rows_fft(self, src, dst, inverse, block_in=0, block_out=0, u8=None):
         lut = self._dp(self._amp_lut) if u8 is not None else None
         self._check(self._lib.slm_rows_fft(self._ctx, self._mem_ptr(src), self._mem_ptr(u8), lut, self._mem_ptr(dst),
                                            int(inverse), int(block_in), int(block_out)))
+
+    # ---- what a GS and a GD run share ---------------------------------------------------------------------------------
+    def _begin(self, target_slab, max_loops: int, want_expected: bool) -> SimpleNamespace:
+        """Check this rank's uint8 target rows (host array or device buffer), take the plane's max over the ranks, exchange
+        the target once into the column layout, allocate the run's buffers and loop state and reset the context's."""
+        if self._mem_is_device(target_slab):
+            T = target_slab
+            if tuple(T.shape) != self.shape or self._mem_np_dtype(T) != np.uint8:
+                raise ValueError(f"target slab must be uint8 {self.shape}")
+            local_max = float(self.to_host(T.max() if hasattr(T, "is_cuda") else np.asarray(T).max()))
+        else:
+            t = np.ascontiguousarray(target_slab)
+            if t.dtype != np.uint8 or t.shape != self.shape:
+                raise ValueError(f"target slab must be uint8 {self.shape}")
+            T, local_max = self._mem_upload(t), float(t.max())
+        norm = float(self._all_reduce(np.array([local_max]), "max")[0])
+        peer = self._peer is not None
+        blocks = (self.world, self.rows, self.rows)
+
+        def buf(name, shape, dtype):                                      # the peers store into the symmetric ones
+            return self._peer_view(name, shape, dtype) if peer else self._mem_empty(shape, dtype)
+
+        r = SimpleNamespace(T=T, blocks=blocks, norm=norm, hw=float(self.n) * float(self.n), Tx=buf("Tx", blocks, np.uint8))
+        self._exchange(T, None if peer else self._mem_empty(blocks, np.uint8), r.Tx, 1, "Tx")      # target columns, once
+        r.X, r.Y = buf("X", self.shape, self.complex_dtype), buf("Y", self.shape, self.complex_dtype)   # row slabs
+        r.S = self._mem_empty(blocks, self.complex_dtype)                 # exchange layout: lines (and the send side of the collectives)
+        r.Rv = buf("Rv", blocks, self.complex_dtype)                      # receive side
+        r.partial = self._mem_empty((self.rows, 4), np.float64)
+        # loop state on the device: {scale, last error, iterations done, loop ended, max}, the error curve, the ranks' sums
+        r.state = self._mem_upload(np.array([1.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0]))
+        r.curve = self._mem_empty((max_loops,), np.float64)
+        r.mine = self._mem_empty((4,), np.float64)
+        # (two slots used in turn: a rank may run one closing step ahead of a peer that is still reading the previous one)
+        r.gathered = buf("gathered", (2, self.world, 4), np.float64)
+        r.inten = self._mem_empty(blocks, np.float64) if want_expected else None
+        self._slot = 0
+        self._check(self._lib.slm_rows_reset(self._ctx))                 # (a finished run's flags would stop the row passes)
+        return r
+
+    def _close(self, r, form: int, tolerance: float):
+        """this rank's sums -> every rank -> scale / error / loop condition in ``r.state`` (all on the device); ``form``: that
+        of slm_rows_close (0: GS iteration, 1: scale and max only, 2: GD iteration)"""
+        peer = self._peer is not None
+        slot, self._slot = self._slot, self._slot ^ 1
+        self._check(self._lib.slm_rows_reduce(self._ctx, self._mem_ptr(r.partial), self.rows, self._mem_ptr(r.mine),
+                                              self._peer_array("gathered", slot * self.world * 32) if peer else None,
+                                              self.world if peer else 0, self.rank))
+        if peer:
+            self._peer_barrier()
+        else:
+            self._all_gather4(r.mine, r.gathered[slot])
+        self._check(self._lib.slm_rows_close(self._ctx, self._mem_ptr(r.gathered[slot]), self.world, r.norm, r.hw, form,
+                                             float(tolerance), self._mem_ptr(r.state), self._mem_ptr(r.curve)))
+
+    def _curve(self, r, done_iters: int, tolerance: float):
+        """(error curve, loop state), read back; the curve cut where the reference stops (tolerance <= 0: the loop ran on)"""
+        errors = [np.float64(e) for e in self.to_host(r.curve)[:done_iters]]
+        for i, e in enumerate(errors):
+            if not (e > tolerance):
+                errors = errors[:i + 1]
+                break
+        return errors, self.to_host(r.state)
+
+    def _expected(self, r, on_device: bool, scale: float, divisor: float = None):
+        """the intensity the run kept, back in rows, times ``scale`` and then over ``divisor`` (GD: times norm, over the max,
+        rounded as algorithms.py:86 rounds it); None if the run kept none"""
+        if r.inten is None:
+            return None
+        exp_slab = self._mem_empty(self.shape, np.float64)
+        if self.world == 1:
+            self._transpose(r.inten, exp_slab, 8, True)
+        else:
+            recv_i = self._mem_empty(r.blocks, np.float64)
+            self._all_to_all(r.inten, recv_i)
+            self._transpose(recv_i, exp_slab, 8, True)
+        if not on_device:
+            exp_slab = self.to_host(exp_slab) * scale
+            return exp_slab if divisor is None else exp_slab / divisor
+        exp_slab *= scale
+        if divisor is not None:
+            exp_slab /= divisor
+        return exp_slab
 
     # ---- Gerchberg-Saxton on the distributed plane --------------------------------------------------------------
     def gs(self, target_slab, max_loops: int, tolerance: float = 0.0, want_expected: bool = True, on_device: bool = False,
@@ -346,130 +292,47 @@ class SlabEngine(Engine):
         curve is identical on every rank.  ``on_device`` leaves hologram / expected in device memory."""
         if max_loops < 1:
             raise UnboundLocalError("cannot access local variable 'expected_outcome' where it is not associated with a value")
-        if self._mem_is_device(target_slab):
-            T, t = target_slab, None
-            if tuple(T.shape) != self.shape or self._mem_np_dtype(T) != np.uint8:
-                raise ValueError(f"target slab must be uint8 {self.shape}")
-            local_max = float(self.to_host(T.max() if hasattr(T, "is_cuda") else np.asarray(T).max()))
-        else:
-            t = np.ascontiguousarray(target_slab)
-            if t.dtype != np.uint8 or t.shape != self.shape:
-                raise ValueError(f"target slab must be uint8 {self.shape}")
-            T, local_max = self._mem_upload(t), float(t.max())
-        h, n, cs = self.rows, self.n, np.dtype(self.complex_dtype).itemsize
         inc = self._as_device(inc_amp_slab, self.real_dtype, "inc_amp_slab")
         if inc is not None and tuple(inc.shape) != self.shape:
             raise ValueError(f"inc_amp_slab must have shape {self.shape}")
-        norm = float(self._all_reduce(np.array([local_max]), "max")[0])
-        peer = self._peer is not None
-        blocks = (self.world, h, h)
-        Tx_send = None if peer else self._mem_empty(blocks, np.uint8)
-        Tx = self._peer_view("Tx", blocks, np.uint8) if peer else self._mem_empty(blocks, np.uint8)
-        self._exchange(T, Tx_send, Tx, 1, "Tx")                              # target columns, once
-        X = self._peer_view("X", self.shape, self.complex_dtype) if peer else self._mem_empty(self.shape, self.complex_dtype)   # row slabs
-        Y = self._peer_view("Y", self.shape, self.complex_dtype) if peer else self._mem_empty(self.shape, self.complex_dtype)
-        S = self._mem_empty(blocks, self.complex_dtype)                      # exchange layout: lines (and the send side of the collectives)
-        Rv = self._peer_view("Rv", blocks, self.complex_dtype) if peer else self._mem_empty(blocks, self.complex_dtype)  # receive side
-        Rb = self._peer_view("Rb", blocks, self.complex_dtype) if peer else None                                            # ... of the way back (copies)
-        partial = self._mem_empty((h, 4), np.float64)
+        r = self._begin(target_slab, max_loops, want_expected)
+        cs = np.dtype(self.complex_dtype).itemsize
         # A = ifft2(sqrt(T))  (algorithms.py:27), unnormalised: only its phase is used.  For 8-bit targets the
         # reference computes it (and the first phasor) in complex64, so an fp64 plane borrows an fp32 engine.
         if self.precision == "fp32":
-            self._setup_field(T, X, S, Rv, "Rv", "X")
-            A0, field_kind = X, 1
+            self._setup_field(r.T, r.X, r.S, r.Rv, "Rv", "X")
+            A0, field_kind = r.X, 1
         else:
             helper = type(self)(self.n, self.world, self.rank, "fp32", self._device_index, None, self.group, peer=False)
             A0 = helper._mem_empty(self.shape, np.complex64)
-            helper._setup_field(T, A0, helper._mem_empty(blocks, np.complex64), helper._mem_empty(blocks, np.complex64))
+            helper._setup_field(r.T, A0, helper._mem_empty(r.blocks, np.complex64), helper._mem_empty(r.blocks, np.complex64))
             helper._sync()
             helper.close()
             field_kind = 2
-        hw = float(n) * float(n)
-        # loop state on the device: {scale, last error, iterations done, loop ended}, the error curve, the ranks' sums
-        state = self._mem_upload(np.array([1.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0]))
-        curve = self._mem_empty((max_loops,), np.float64)
-        mine = self._mem_empty((4,), np.float64)
-        # (two slots used in turn: a rank may run one closing step ahead of a peer that is still reading the previous one)
-        gathered = self._peer_view("gathered", (2, self.world, 4), np.float64) if peer else self._mem_empty((2, self.world, 4), np.float64)
-        self._slot = 0
-        inten = None
-        if want_expected:
-            inten = self._mem_empty(blocks, np.float64)
         check_every = tolerance > 0                                           # the host must see every error to stop the loop
         src, field, done_iters = A0, field_kind, 0
         t_loop = time.perf_counter()
         for k in range(max_loops):
-            cur = X if src is Y else Y                                        # receives the row-transformed B
-            overlap = peer and getattr(self, "_parts", 1) > 1 and inc is None   # (the passes in parts take no illumination plane)
-            by_copy = overlap and self._how == "copy"
-            if by_copy:
-                self._row_pass_and_copy(src, cur, field, S, cs)
-            elif overlap:
-                self._row_pass_and_push(src, cur, field, cs)
-            else:
-                self._check(self._lib.slm_rows_gs_row_pass(self._ctx, self._mem_ptr(src), self._mem_ptr(cur), self._mem_ptr(inc), int(field), 0, None))
-                self._exchange(cur, S, Rv, cs, "Rv")
+            cur = r.X if src is r.Y else r.Y                                  # receives the row-transformed B
+            self._check(self._lib.slm_rows_gs_row_pass(self._ctx, self._mem_ptr(src), self._mem_ptr(cur), self._mem_ptr(inc), int(field), 0, None))
+            self._exchange(cur, r.S, r.Rv, cs, "Rv")
             if k == 0:                                                        # exact scale of iteration 0: max pre-pass
-                self._fourier(Rv, S, Tx, state, partial, None)
-                self._close(partial, mine, gathered, norm, hw, True, tolerance, state, curve)
+                self._fourier(r, None)
+                self._close(r, 1, tolerance)
             last = k == max_loops - 1
-            want_i = inten if (want_expected and (last or check_every or k == 0)) else None
-            if overlap:
-                slot, self._slot = self._slot, self._slot ^ 1
-                if by_copy:
-                    self._fourier_and_copy_back(Rv, S, Rb, Tx, state, partial, want_i, cur, cs, mine, slot)
-                else:
-                    self._fourier_and_push_back(Rv, S, Tx, state, partial, want_i, "X" if cur is X else "Y", cs, mine, slot)
-                self._check(self._lib.slm_rows_close(self._ctx, self._mem_ptr(gathered[slot]), self.world, float(norm), float(hw), 0,
-                                                     float(tolerance), self._mem_ptr(state), self._mem_ptr(curve)))
-            else:
-                self._fourier(Rv, S, Tx, state, partial, want_i)
-                self._close(partial, mine, gathered, norm, hw, False, tolerance, state, curve)
-                self._exchange_back(S, Rv, cur, cs, "X" if cur is X else "Y") # D with the columns inverse-transformed
+            self._fourier(r, r.inten if (last or check_every or k == 0) else None)
+            self._close(r, 0, tolerance)
+            self._exchange_back(r.S, r.Rv, cur, cs, "X" if cur is r.X else "Y")   # D with the columns inverse-transformed
             src, field, done_iters = cur, 0, k + 1
-            if check_every or (k == 0 and not norm > 0):                      # (an all-zero target ends the loop at once: 0/0, algorithms.py:29,37)
-                st = self.to_host(state)
-                if st[3] != 0.0:
+            if check_every or (k == 0 and not r.norm > 0):                    # (an all-zero target ends the loop at once: 0/0, algorithms.py:29,37)
+                if self.to_host(r.state)[3] != 0.0:
                     break
         self.enqueue_s = time.perf_counter() - t_loop                        # host time to issue the loop (measurements: is the host the bound?)
-        errors = [np.float64(e) for e in self.to_host(curve)[:done_iters]]
-        for i, e in enumerate(errors):                                        # tolerance <= 0: the loop ran on; cut where the reference stops
-            if not (e > tolerance):
-                errors = errors[:i + 1]
-                break
-        s_last = float(self.to_host(state)[0])
+        errors, st = self._curve(r, done_iters, tolerance)
         holo = self._mem_empty(self.shape, np.float64)
         self._check(self._lib.slm_rows_gs_row_pass(self._ctx, self._mem_ptr(src), None, None, 0, 1, self._mem_ptr(holo)))
-        expected = None
-        if want_expected:
-            exp_slab = self._mem_empty(self.shape, np.float64)
-            if self.world == 1:
-                self._transpose(inten, exp_slab, 8, True)
-            else:
-                recv_i = self._mem_empty(blocks, np.float64)
-                self._all_to_all(inten, recv_i)
-                self._transpose(recv_i, exp_slab, 8, True)
-            if on_device:
-                exp_slab *= s_last                                            # expected_outcome *= norm / max, :37
-                expected = exp_slab
-            else:
-                expected = self.to_host(exp_slab) * s_last
+        expected = self._expected(r, on_device, float(st[0]))                # expected_outcome *= norm / max, :37
         return (holo if on_device else self.to_host(holo)), expected, errors
-
-    def _close(self, partial, mine, gathered, norm, hw, prepass, tolerance, state, curve):
-        """this rank's sums -> every rank -> scale / error / loop condition in `state` (all on the device); ``prepass``:
-        the form of slm_rows_close (False / 0: GS iteration, True / 1: scale and max only, 2: GD iteration)"""
-        peer = self._peer is not None
-        slot, self._slot = self._slot, self._slot ^ 1
-        self._check(self._lib.slm_rows_reduce(self._ctx, self._mem_ptr(partial), self.rows, self._mem_ptr(mine),
-                                              self._peer_array("gathered", slot * self.world * 32) if peer else None,
-                                              self.world if peer else 0, self.rank))
-        if peer:
-            self._peer_barrier()
-        else:
-            self._all_gather4(mine, gathered[slot])
-        self._check(self._lib.slm_rows_close(self._ctx, self._mem_ptr(gathered[slot]), self.world, float(norm), float(hw), int(prepass),
-                                             float(tolerance), self._mem_ptr(state), self._mem_ptr(curve)))
 
     # ---- gradient descent on the distributed plane (algorithms.py:60-112) ------------------------------------------------
     def gd(self, target_slab, x0_slab, lr_schedule, max_loops: int, tolerance: float = 0.0, white_attention=1,
@@ -481,16 +344,6 @@ class SlabEngine(Engine):
         (algorithms.py:86), and here it lives on several devices."""
         if max_loops < 1:
             raise UnboundLocalError("cannot access local variable 'output' where it is not associated with a value")
-        if self._mem_is_device(target_slab):
-            T = target_slab
-            if tuple(T.shape) != self.shape or self._mem_np_dtype(T) != np.uint8:
-                raise ValueError(f"target slab must be uint8 {self.shape}")
-            local_max = float(self.to_host(T.max() if hasattr(T, "is_cuda") else np.asarray(T).max()))
-        else:
-            t = np.ascontiguousarray(target_slab)
-            if t.dtype != np.uint8 or t.shape != self.shape:
-                raise ValueError(f"target slab must be uint8 {self.shape}")
-            T, local_max = self._mem_upload(t), float(t.max())
         x_on_device = self._mem_is_device(x0_slab)
         x0 = x0_slab if x_on_device else np.asarray(x0_slab)
         if tuple(x0.shape) != self.shape or (x_on_device and not str(x0.dtype).endswith(np.dtype(self.complex_dtype).name)):
@@ -498,17 +351,8 @@ class SlabEngine(Engine):
         lr = np.ascontiguousarray(lr_schedule, dtype=np.float64)
         if lr.shape != (max_loops,):
             raise ValueError("lr_schedule must have max_loops entries")
-        h, n, cs = self.rows, self.n, np.dtype(self.complex_dtype).itemsize
-        norm = float(self._all_reduce(np.array([local_max]), "max")[0])
-        peer = self._peer is not None
-        blocks = (self.world, h, h)
-        Tx_send = None if peer else self._mem_empty(blocks, np.uint8)
-        Tx = self._peer_view("Tx", blocks, np.uint8) if peer else self._mem_empty(blocks, np.uint8)
-        self._exchange(T, Tx_send, Tx, 1, "Tx")
-        X = self._peer_view("X", self.shape, self.complex_dtype) if peer else self._mem_empty(self.shape, self.complex_dtype)
-        Y = self._peer_view("Y", self.shape, self.complex_dtype) if peer else self._mem_empty(self.shape, self.complex_dtype)
-        S = self._mem_empty(blocks, self.complex_dtype)
-        Rv = self._peer_view("Rv", blocks, self.complex_dtype) if peer else self._mem_empty(blocks, self.complex_dtype)
+        r = self._begin(target_slab, max_loops, want_expected)
+        h, cs = self.rows, np.dtype(self.complex_dtype).itemsize
         if x_on_device:                                                   # (the row pass updates x in place: work on a copy)
             x = self._mem_empty(self.shape, self.complex_dtype)
             self._copy(x0, x)
@@ -516,60 +360,33 @@ class SlabEngine(Engine):
             x = self._mem_upload(x0.astype(self.complex_dtype))
         lr_dev = self._mem_upload(lr)
         mask_lut = hl.gd_mask_lut(white_attention)
-        partial = self._mem_empty((h, 4), np.float64)
-        state = self._mem_upload(np.array([1.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0]))
-        curve = self._mem_empty((max_loops,), np.float64)
-        mine = self._mem_empty((4,), np.float64)
-        gathered = self._peer_view("gathered", (2, self.world, 4), np.float64) if peer else self._mem_empty((2, self.world, 4), np.float64)
-        self._slot = 0
-        inten = self._mem_empty(blocks, np.float64) if want_expected else None
-        hw = float(n) * float(n)
         check_every = tolerance > 0
-        self._check(self._lib.slm_rows_reset(self._ctx))
         done_iters = 0
         for k in range(max_loops):
             # SLM-plane pass: the update of the previous iteration (none yet at k = 0), x/|x|, rows of fft2
-            self._check(self._lib.slm_rows_gd_row_pass(self._ctx, self._mem_ptr(Y), self._mem_ptr(x), self._mem_ptr(X), self._mem_ptr(lr_dev),
+            self._check(self._lib.slm_rows_gd_row_pass(self._ctx, self._mem_ptr(r.Y), self._mem_ptr(x), self._mem_ptr(r.X), self._mem_ptr(lr_dev),
                                                        int(k == 0), 0, None))
-            self._exchange(X, S, Rv, cs, "Rv")
+            self._exchange(r.X, r.S, r.Rv, cs, "Rv")
             # the plane's max (the transform is kept in S), then the gradient step on it
-            self._check(self._lib.slm_rows_gd_fourier_pass(self._ctx, self._mem_ptr(Rv), self._mem_ptr(S), h, None, None, norm, None,
-                                                           self._mem_ptr(partial), None, 0))
-            self._close(partial, mine, gathered, norm, hw, 1, tolerance, state, curve)
+            self._check(self._lib.slm_rows_gd_fourier_pass(self._ctx, self._mem_ptr(r.Rv), self._mem_ptr(r.S), h, None, None, r.norm, None,
+                                                           self._mem_ptr(r.partial), None, 0))
+            self._close(r, 1, tolerance)
             last = k == max_loops - 1
-            want_i = inten if (want_expected and (last or check_every or k == 0)) else None
-            self._check(self._lib.slm_rows_gd_fourier_pass(self._ctx, self._mem_ptr(S), self._mem_ptr(S), h, self._mem_ptr(Tx), self._dp(mask_lut),
-                                                           norm, self._mem_ptr(state), self._mem_ptr(partial), self._mem_ptr(want_i), 1))
-            self._close(partial, mine, gathered, norm, hw, 2, tolerance, state, curve)
-            self._exchange_back(S, Rv, Y, cs, "Y")
+            want_i = r.inten if (last or check_every or k == 0) else None
+            self._check(self._lib.slm_rows_gd_fourier_pass(self._ctx, self._mem_ptr(r.S), self._mem_ptr(r.S), h, self._mem_ptr(r.Tx),
+                                                           self._dp(mask_lut), r.norm, self._mem_ptr(r.state), self._mem_ptr(r.partial),
+                                                           self._mem_ptr(want_i), 1))
+            self._close(r, 2, tolerance)
+            self._exchange_back(r.S, r.Rv, r.Y, cs, "Y")
             done_iters = k + 1
-            if check_every or (k == 0 and not norm > 0):
-                if self.to_host(state)[3] != 0.0:
+            if check_every or (k == 0 and not r.norm > 0):
+                if self.to_host(r.state)[3] != 0.0:
                     break
-        errors = [np.float64(e) for e in self.to_host(curve)[:done_iters]]
-        for i, e in enumerate(errors):
-            if not (e > tolerance):
-                errors = errors[:i + 1]
-                break
-        st = self.to_host(state)
+        errors, st = self._curve(r, done_iters, tolerance)
         holo = self._mem_empty(self.shape, np.float64)
-        self._check(self._lib.slm_rows_gd_row_pass(self._ctx, self._mem_ptr(Y), self._mem_ptr(x), None, self._mem_ptr(lr_dev), 0, 1,
+        self._check(self._lib.slm_rows_gd_row_pass(self._ctx, self._mem_ptr(r.Y), self._mem_ptr(x), None, self._mem_ptr(lr_dev), 0, 1,
                                                    self._mem_ptr(holo)))
-        expected = None
-        if want_expected:
-            exp_slab = self._mem_empty(self.shape, np.float64)
-            if self.world == 1:
-                self._transpose(inten, exp_slab, 8, True)
-            else:
-                recv_i = self._mem_empty(blocks, np.float64)
-                self._all_to_all(inten, recv_i)
-                self._transpose(recv_i, exp_slab, 8, True)
-            if on_device:
-                exp_slab *= norm                                              # output_unnormed * norm / amax, algorithms.py:86
-                exp_slab /= float(st[4])
-                expected = exp_slab
-            else:
-                expected = self.to_host(exp_slab) * norm / float(st[4])
+        expected = self._expected(r, on_device, r.norm, float(st[4]))      # output_unnormed * norm / amax, algorithms.py:86
         return (holo if on_device else self.to_host(holo)), expected, errors
 
     def _setup_field(self, T, X, S, Rv, peer_recv=None, peer_slab=None):
@@ -580,18 +397,23 @@ class SlabEngine(Engine):
         self._rows_fft(Rv, S, True, block_in=h, block_out=h)
         self._exchange_back(S, Rv, X, cs, peer_slab)
 
-    def _fourier(self, lines_in, lines_out, Tx, state, partial, inten, line0=0, nlines=0):
-        self._check(self._lib.slm_rows_gs_fourier_pass_dev(self._ctx, self._mem_ptr(lines_in), self._mem_ptr(lines_out), self.rows,
-                                                           self._mem_ptr(Tx), self._dp(self._amp_lut), self._mem_ptr(state),
-                                                           self._mem_ptr(partial), self._mem_ptr(inten), int(line0), int(nlines)))
+    def _fourier(self, r, inten):
+        self._check(self._lib.slm_rows_gs_fourier_pass(self._ctx, self._mem_ptr(r.Rv), self._mem_ptr(r.S), self.rows, self._mem_ptr(r.Tx),
+                                                       self._dp(self._amp_lut), self._mem_ptr(r.state), self._mem_ptr(r.partial),
+                                                       self._mem_ptr(inten)))
 
     def close(self):
-        if self._peer is not None and self._peer.get("comm_ctx") is not None and getattr(self, "_ctx", None):
-            self._lib.slm_ctx_destroy(self._peer["comm_ctx"])
-            for _, cx in self._peer.get("lanes", []):
-                self._lib.slm_ctx_destroy(cx)
-        self._peer = None
+        self._peer = None                     # (releases this rank's symmetric allocation)
         super().close()
+
+
+def _world_rank():
+    """(world size, rank) of the default process group; (1, 0) without one."""
+    try:
+        import torch.distributed as dist
+        return (dist.get_world_size(), dist.get_rank()) if dist.is_available() and dist.is_initialized() else (1, 0)
+    except Exception:
+        return 1, 0
 
 
 def gerchberg_saxton_slab(target, max_loops: int, tolerance: float = 0.0, precision: str = "fp32", want_expected: bool = True,
@@ -599,11 +421,7 @@ def gerchberg_saxton_slab(target, max_loops: int, tolerance: float = 0.0, precis
     """GS hologram of one large square uint8 ``target`` (every rank passes the same array, or only its
     own rows via ``target[lo:hi]`` semantics handled here) on all ranks of the default process group.
     Returns this rank's row slab of (hologram, expected) and the error curve."""
-    try:
-        import torch.distributed as dist
-        world, rank = (dist.get_world_size(), dist.get_rank()) if dist.is_available() and dist.is_initialized() else (1, 0)
-    except Exception:
-        world, rank = 1, 0
+    world, rank = _world_rank()
     target = np.asarray(target)
     n = target.shape[1]
     lo, hi = rank * (n // world), (rank + 1) * (n // world)
@@ -623,11 +441,7 @@ def gradient_descent_slab(target, max_loops: int, learning_rate: float = 0.005, 
     (algorithms.py:115-153; the MT19937 stream is drawn row-major for the whole plane, every rank keeps its own rows) --
     "fourier" is not offered here.  Returns this rank's row slab of (hologram, expected), the error curve and the learning rate the
     reference would leave in ``args.learning_rate``."""
-    try:
-        import torch.distributed as dist
-        world, rank = (dist.get_world_size(), dist.get_rank()) if dist.is_available() and dist.is_initialized() else (1, 0)
-    except Exception:
-        world, rank = 1, 0
+    world, rank = _world_rank()
     target = np.asarray(target)
     n = target.shape[1]
     lo, hi = rank * (n // world), (rank + 1) * (n // world)

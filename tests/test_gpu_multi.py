@@ -58,12 +58,8 @@ def _slab_worker(rank, world, port, n, loops, out_dir):
                             device_id=torch.device("cuda", rank))
     try:
         t = synthetic.noise_target((n, n), seed=6)
-        for tag, env in (("peer", {"SLM_SLAB_PARTS": "4"}), ("peer_store", {"SLM_SLAB_PARTS": "4", "SLM_SLAB_EXCHANGE": "store"}), ("peer1", {}),
-                         ("coll", {"SLM_SLAB_NO_PEER": "1"})):
-            for k in ("SLM_SLAB_NO_PEER", "SLM_SLAB_PARTS", "SLM_SLAB_EXCHANGE"):
-                os.environ.pop(k, None)
-            os.environ.update(env)
-            eng = slab.SlabEngine(n, world, rank, "fp32")
+        for tag, peer in (("peer", None), ("coll", False)):
+            eng = slab.SlabEngine(n, world, rank, "fp32", peer=peer)
             h, e, errs = eng.gs(t[rank * (n // world):(rank + 1) * (n // world)], loops)
             np.savez(os.path.join(out_dir, f"slab_{tag}{rank}.npz"), h=h, e=e, errs=np.array(errs), status=np.array(eng.peer_status))
             eng.close()
@@ -84,9 +80,8 @@ def test_two_gpu_slab_gs_matches_single_gpu(tmp_path):
     eng = SlabEngine(n, 1, 0, "fp32")
     h, e, errs = eng.gs(synthetic.noise_target((n, n), seed=6), loops)
     statuses = {}
-    # copy engines beside the passes / transposing stores into the peer's memory (in parts, in one go) / NCCL all-to-all:
-    # the same bits
-    for tag in ("peer", "peer_store", "peer1", "coll"):
+    # transposing stores into the peer's memory / NCCL all-to-all: the same bits
+    for tag in ("peer", "coll"):
         r0, r1 = np.load(tmp_path / f"slab_{tag}0.npz"), np.load(tmp_path / f"slab_{tag}1.npz")
         statuses[tag] = str(r0["status"])
         np.testing.assert_array_equal(np.concatenate([r0["h"], r1["h"]]), h)
@@ -111,10 +106,8 @@ def _slab_gd_worker(rank, world, port, n, loops, out_dir):
         x0 = hl.host_initial_guess("random", (n, n), 11)
         during, _ = hl.learning_rate_schedule(0.005, 1, loops)
         lo, hi = rank * (n // world), (rank + 1) * (n // world)
-        for tag, env in (("peer", {}), ("coll", {"SLM_SLAB_NO_PEER": "1"})):
-            os.environ.pop("SLM_SLAB_NO_PEER", None)
-            os.environ.update(env)
-            eng = slab.SlabEngine(n, world, rank, "fp32")
+        for tag, peer in (("peer", None), ("coll", False)):
+            eng = slab.SlabEngine(n, world, rank, "fp32", peer=peer)
             h, e, errs = eng.gd(t[lo:hi], x0[lo:hi], during, loops, white_attention=2.0)
             np.savez(os.path.join(out_dir, f"slabgd_{tag}{rank}.npz"), h=h, e=e, errs=np.array(errs))
             eng.close()
