@@ -67,8 +67,12 @@ template <typename R, int H> struct ColGroupGeom {
     static constexpr size_t TW_BYTES = (size_t)H * sizeof(cpx<R>);
     static constexpr bool TW_SHARED = OFF_TW + TW_BYTES <= 232448; // 227 KB of shared memory per CTA
     static constexpr size_t SMEM = OFF_TW + (TW_SHARED ? TW_BYTES : 0);
+    // P::ONE_STAGE: the radix-5 and composite middle stages (1152, 1280, 1920) hold up to QMAX x radix points per thread
+    // beside the tile's grey levels and sums; under this kernel's register cap (128 at 448 threads, 96 at 608) they
+    // spilled 200-700 bytes per thread, so those lengths take the spill-free one-CTA-per-tile kernel instead.
     static constexpr bool OK = (ROWB == 64 || ROWB == 32) && COMPUTE % 32 == 0 && TC % LPG == 0 && GROUPS <= 14 &&
-                               H % 32 == 0 && NW <= 32 && OFF_TW <= 232448;    // (two tile buffers + exchange must fit)
+                               H % 32 == 0 && NW <= 32 && OFF_TW <= 232448 &&   // (two tile buffers + exchange must fit)
+                               P::ONE_STAGE;
     using Sync = GroupSync<GROUP_THREADS>;
 };
 

@@ -130,11 +130,18 @@ static int make_twiddles(slm_ctx* c, int N, int prec, void** out) {
 }
 
 // Describe a field plane stack ([rows][W complex columns]) to the TMA unit: 2-D tensor of real
-// elements, box = TC complex columns x up to 256 rows, 32B/64B-swizzled shared-memory image.
+// elements, box = TC complex columns x up to 256 rows, 32B/64B-swizzled shared-memory image.  A tile is
+// H / box_rows whole boxes, so box_rows divides H (a box that ran past the tile would land in the next buffer
+// and overshoot the barrier's byte count); 256 for every length the column-group kernel serves now.
+static int tile_box_rows(int H) {
+    int b = H < 256 ? H : 256;
+    while (H % b != 0) --b;
+    return b;
+}
 static int make_tile_map(slm_ctx* c, void* base, long long rows, TileMap* out) {
     const size_t cs = 2 * real_size(c->prec);
     const int row_bytes = c->col->group_row_bytes;
-    const int box_rows = c->H < 256 ? c->H : 256;
+    const int box_rows = tile_box_rows(c->H);
 #ifdef SLM_EMULATE
     (void)rows;
     out->base = static_cast<unsigned char*>(base);
@@ -390,7 +397,7 @@ template <class F> static int replay_iterations(slm_ctx* c, int batch, int times
 }
 
 extern "C" const char* slm_last_error(void) { return g_err.c_str(); }
-extern "C" int slm_version(void) { return 101; }
+extern "C" int slm_version(void) { return 102; }
 extern "C" int slm_supported_lengths(int* out, int cap) { return supported_lengths(out, cap); }
 
 extern "C" void slm_ctx_destroy(slm_ctx* c) {
@@ -412,8 +419,15 @@ extern "C" int slm_ctx_create(slm_ctx** out, int device, int H, int W, int max_b
     const LineTable* col = find_line_table(H, precision);
     if (!row || !col) {
         char buf[160];
-        snprintf(buf, sizeof buf, "unsupported plane shape %dx%d: rows and columns must be one of the built line lengths", H, W);
-        return fail(SLM_ERR_SHAPE, buf);
+        snprintf(buf, sizeof buf, "unsupported plane shape %dx%d: rows and columns must be one of the built line lengths (", H, W);
+        std::string both, rows;
+        int lens[64];
+        const int n = supported_lengths(lens, 64);
+        for (int i = 0; i < n && i < 64; ++i) {
+            std::string& s = find_line_table(lens[i], precision)->rows_only ? rows : both;
+            s += (s.empty() ? "" : ", ") + std::to_string(lens[i]);
+        }
+        return fail(SLM_ERR_SHAPE, buf + both + (rows.empty() ? "" : "; row length only: " + rows) + ")");
     }
     if (H % row->rows_per_cta != 0 || W % col->cols_per_cta != 0) return fail(SLM_ERR_SHAPE, "plane shape not divisible by the CTA tile");
     SLM_CUDA(cudaSetDevice(device));
@@ -832,6 +846,11 @@ extern "C" int slm_rows_create(slm_ctx** out, int device, int rows, int W, int p
     if (!out || rows < 1 || (precision != PREC_F32 && precision != PREC_F64)) return fail(SLM_ERR_ARG, "slm_rows_create: bad argument");
     const LineTable* row = find_line_table(W, precision);
     if (!row) return fail(SLM_ERR_SHAPE, "unsupported line length " + std::to_string(W));
+    // the slab Fourier-plane kernel sums a line's partials per warp: a line is either within one warp or whole warps
+    const int m = row->row_threads / row->rows_per_cta;
+    if (m > 32 && m % 32 != 0)
+        return fail(SLM_ERR_SHAPE, "line length " + std::to_string(W) + " is not supported on the slab path (" + std::to_string(m) +
+                                       " threads per line: neither within one warp nor whole warps)");
     if (rows % row->rows_per_cta != 0 || rows % 32 != 0) return fail(SLM_ERR_SHAPE, "slab rows must be a multiple of 32 and of the CTA row tile");
     SLM_CUDA(cudaSetDevice(device));
     slm_ctx* c = new slm_ctx;

@@ -3,7 +3,8 @@
 // A "line" is one row or one column of an H x W plane.  Each thread owns E points of a line
 // in registers; a line of N = E * m * E points is transformed by
 //   stage 1 : radix-E butterflies on register data            -> shared memory
-//   middle  : one radix-m stage, shared -> registers -> shared (m in {1,2,3,4,8,16})
+//   middle  : one radix-m stage, shared -> registers -> shared (m in {1,2,3,4,8,16}), or for any other
+//             5-smooth m one such stage per radix of m (radices 2..16, 3, 5: mid_stages)
 //   last    : radix-E butterflies, shared -> registers
 // (Stockham autosort, so results come out in natural order and thread j again owns the
 // points j + r*N/E, r = 0..E-1: exactly the mapping stage 1 consumes.  A fused
@@ -205,9 +206,22 @@ template <int DIR, typename R> SLM_DEV void dft32(cpx<R>* v) {
     dft16<DIR>(o);
     Dft32Combine<DIR, 0, R>::run(v, e, o);
 }
+template <int DIR, typename R> SLM_DEV void dft5(cpx<R>* v) {
+    const R c1 = (R)0.30901699437494742410, c2 = (R)-0.80901699437494742410;     // cos(2pi/5), cos(4pi/5)
+    const R s1 = (R)0.95105651629515357212, s2 = (R)0.58778525229247312917;      // sin(2pi/5), sin(4pi/5)
+    const cpx<R> t1 = cadd(v[1], v[4]), t2 = cadd(v[2], v[3]), t3 = csub(v[1], v[4]), t4 = csub(v[2], v[3]);
+    const cpx<R> a1 = pk_fma(mk<R>(c2, c2), t2, pk_fma(mk<R>(c1, c1), t1, v[0]));
+    const cpx<R> a2 = pk_fma(mk<R>(c1, c1), t2, pk_fma(mk<R>(c2, c2), t1, v[0]));
+    const cpx<R> b1 = rot90<DIR>(pk_fma(mk<R>(s2, s2), t4, cscale(t3, s1)));    // DIR * i * (s1 t3 + s2 t4)
+    const cpx<R> b2 = rot90<DIR>(pk_fma(mk<R>(-s1, -s1), t4, cscale(t3, s2)));  // DIR * i * (s2 t3 - s1 t4)
+    v[0] = cadd(v[0], cadd(t1, t2));
+    v[1] = cadd(a1, b1); v[4] = csub(a1, b1);
+    v[2] = cadd(a2, b2); v[3] = csub(a2, b2);
+}
 template <int RAD, int DIR, typename R> SLM_DEV void dft_small(cpx<R>* v) {
     if constexpr (RAD == 2) dft2<DIR>(v[0], v[1]);
     else if constexpr (RAD == 3) dft3<DIR>(v[0], v[1], v[2]);
+    else if constexpr (RAD == 5) dft5<DIR>(v);
     else if constexpr (RAD == 4) dft4<DIR>(v[0], v[1], v[2], v[3]);
     else if constexpr (RAD == 8) dft8<DIR>(v);
     else if constexpr (RAD == 16) dft16<DIR>(v);
@@ -234,7 +248,23 @@ template <int RAD, typename R> SLM_DEV void twiddle_powers(cpx<R>* w, cpx<R> w1)
 #ifndef SLM_E32_LEN
 #define SLM_E32_LEN 0          // tuning builds: one more line length transformed with 32 points per thread
 #endif
-SLM_HOSTDEV constexpr int default_points(int N) { return (N >= 8192 || N == SLM_E32_LEN) ? 32 : (N >= 256) ? 16 : 8; }
+// The middle of a plan is a list of Stockham stages, one per radix: the power-of-two part of m as one radix (at most 16),
+// then the 3s, then the 5s.  E.g. 1152 = 8 * (2*3*3) * 8, 1920 = 8 * (2*3*5) * 8, 1280 = 16 * 5 * 16.
+struct MidRadices { int n; int r[8]; };
+SLM_HOSTDEV constexpr MidRadices mid_radices(int m) {
+    MidRadices s{0, {0, 0, 0, 0, 0, 0, 0, 0}};
+    int p2 = 1;
+    while (m > 0 && m % 2 == 0) { p2 *= 2; m /= 2; }
+    if (p2 > 1) s.r[s.n++] = p2;
+    while (m > 0 && m % 3 == 0 && s.n < 8) { s.r[s.n++] = 3; m /= 3; }
+    while (m > 0 && m % 5 == 0 && s.n < 8) { s.r[s.n++] = 5; m /= 5; }
+    if (m != 1 || p2 > 16) s.n = -1;               // a prime factor above 5, or a power-of-two part above 16
+    return s;
+}
+SLM_HOSTDEV constexpr bool valid_middle(int m) { return m >= 1 && mid_radices(m).n >= 0; }
+SLM_HOSTDEV constexpr int default_points(int N) {
+    return (N >= 8192 || N == SLM_E32_LEN) ? 32 : (N % 256 == 0 && valid_middle(N / 256)) ? 16 : 8;
+}
 // Column transforms of 4096 points keep 32 points per thread: 128 threads per column let a CTA hold FOUR columns
 // (32-byte row segments, whole sectors) instead of two; measured 0.48 -> 0.36 ms per Fourier-plane pass (2 x 4096^2).
 // The row kernels stay at 16 (the GD row pass holds x beside the field and would spill).
@@ -247,9 +277,13 @@ template <int N, int EP = default_points(N)> struct FftPlan {
     static constexpr int M = N / E;                    // threads per line
     static constexpr int MID = N / (E * E);            // middle radix (1 = none)
     static constexpr int NP = N + N / E;               // padded line length in shared memory
+    // ONE_STAGE: the middle radices with their own stage code (one butterfly set per thread, or radix 3 predicated);
+    // every other middle runs as the Stockham stages of mid_radices(MID)
+    static constexpr bool ONE_STAGE = MID == 1 || MID == 2 || MID == 3 || MID == 4 || MID == 8 || MID == 16;
     static_assert(E * E * MID == N, "line length must be E*E*m");
-    static_assert(MID == 1 || MID == 2 || MID == 3 || MID == 4 || MID == 8 || MID == 16, "unsupported line length");
-    static_assert(MID <= E || MID == 3, "middle radix must fit the per-thread register tile");
+    static_assert(valid_middle(MID), "unsupported line length: the middle must be 5-smooth with a power-of-two part <= 16");
+    static_assert(M % 8 == 0, "threads per line must be a multiple of 8");
+    static_assert(!ONE_STAGE || MID <= E || MID == 3, "middle radix must fit the per-thread register tile");
     SLM_HOSTDEV static constexpr int pad(int i) { return i + i / E; }
 };
 template <int N> using ColPlan = FftPlan<N, column_points(N)>;
@@ -273,6 +307,45 @@ template <int THREADS> struct GroupSync {          // THREADS == 0: whole CTA
     SLM_DEV void operator()() const { if (THREADS == 0) sync_cta(); else if (THREADS == 32) sync_warp(); else sync_named(id, THREADS); }
 };
 
+// Middle stages S, S+1, ... of a composite plan (FftPlan::ONE_STAGE false), shared -> registers -> shared.  Stage S
+// has radix RS = mid_radices(MID).r[S] and Ns = E * (earlier middle radices): butterfly b < N/RS (k = b mod Ns) reads
+// points b + p*N/RS, multiplies them by tw[k*p*N/(Ns*RS)] and writes its outputs to (b/Ns)*Ns*RS + k + p*Ns.  Thread j
+// takes the butterflies b = j + q*M (q < QMAX, the last ones predicated).  Ns divides M = E*MID, so k = j mod Ns for
+// every q, and every offset below is a multiple of E: pad() keeps (per-thread base) + (compile-time offset).
+template <typename R, int N, int E, int DIR, int STRIDE, bool TW_SHARED, int S, int NS, class Sync>
+SLM_DEV void mid_stages(cpx<R>* line, int j, const cpx<R>* SLM_RESTRICT tw, Sync sync) {
+    constexpr MidRadices MR = mid_radices(N / (E * E));
+    constexpr int RS = MR.r[S], M = N / E, EP = E + 1;
+    constexpr int NB = N / RS, QMAX = (NB + M - 1) / M;
+    const int k = j % NS, o = (j / NS) * NS * RS + k;
+    cpx<R>* const ldp = line + (j + j / E) * STRIDE;
+    cpx<R>* const stp = line + (o + o / E) * STRIDE;
+    cpx<R> w[RS];
+#pragma unroll
+    for (int p = 1; p < RS; ++p) w[p] = tw_load<DIR, TW_SHARED>(tw, k * p * (N / (NS * RS)));
+    cpx<R> a[QMAX][RS];
+#pragma unroll
+    for (int q = 0; q < QMAX; ++q) {
+        if (QMAX * M == NB || j + q * M < NB) {
+#pragma unroll
+            for (int p = 0; p < RS; ++p) a[q][p] = ldp[((q * M + p * NB) / E) * EP * STRIDE];
+        }
+    }
+    sync();
+#pragma unroll
+    for (int q = 0; q < QMAX; ++q) {
+        if (QMAX * M == NB || j + q * M < NB) {
+#pragma unroll
+            for (int p = 1; p < RS; ++p) a[q][p] = cmul(a[q][p], w[p]);
+            dft_small<RS, DIR>(a[q]);
+#pragma unroll
+            for (int p = 0; p < RS; ++p) stp[((q * M * RS + p * NS) / E) * EP * STRIDE] = a[q][p];
+        }
+    }
+    sync();
+    if constexpr (S + 1 < MR.n) mid_stages<R, N, E, DIR, STRIDE, TW_SHARED, S + 1, NS * RS>(line, j, tw, sync);
+}
+
 template <typename R, int N, int DIR, int STRIDE, class Sync = CtaSync, bool TW_SHARED = false, int POINTS = default_points(N)>
 SLM_DEV void line_fft(cpx<R>* v, cpx<R>* line, int j, const cpx<R>* SLM_RESTRICT tw, Sync sync = Sync()) {
     using P = FftPlan<N, POINTS>;
@@ -287,7 +360,9 @@ SLM_DEV void line_fft(cpx<R>* v, cpx<R>* line, int j, const cpx<R>* SLM_RESTRICT
     for (int r = 0; r < E; ++r) st1[r * STRIDE] = v[r];
     sync();
 
-    if constexpr (MID > 1) {
+    if constexpr (!P::ONE_STAGE) {
+        mid_stages<R, N, E, DIR, STRIDE, TW_SHARED, 0, E>(line, j, tw, sync);
+    } else if constexpr (MID > 1) {
         const int jh = j / E, jl = j % E;
         cpx<R>* const stm = line + (jh * BLK + jl) * STRIDE;
         cpx<R> w[MID];

@@ -138,6 +138,7 @@ template <int NT, int FIELDS> SLM_DEV bool publish_and_collect(Partial mine, int
 
 // ---- geometry --------------------------------------------------------------------------------------
 constexpr int floor_pow2(int v) { int p = 1; while (2 * p <= v) p *= 2; return p; }
+constexpr int whole_warp_columns(int tc, int m) { while ((tc * m) % 32 != 0) tc *= 2; return tc; }
 template <typename R, int L> struct RowGeom {
     using P = FftPlan<L>;
     static constexpr int M = P::M;
@@ -169,7 +170,9 @@ template <typename R, int L> struct ColGeom {
     static constexpr int TMAX = sizeof(R) == 4 ? 512 : 256;
     static constexpr int TCMAX = sizeof(R) == 4 ? SLM_TCMAX_F32 : SLM_TCMAX_F64;
     static constexpr int TCRAW = (TMAX / M) < TCMAX ? (TMAX / M) : TCMAX;
-    static constexpr int TC = TCRAW >= 8 ? 8 : TCRAW >= 4 ? 4 : TCRAW >= 2 ? 2 : 1;            // columns per CTA
+    static constexpr int TC0 = TCRAW >= 8 ? 8 : TCRAW >= 4 ? 4 : TCRAW >= 2 ? 2 : 1;
+    // columns per CTA: doubled until the CTA is whole warps (M = 144 or 240 points in fp64: 2 columns)
+    static constexpr int TC = whole_warp_columns(TC0, M);
     static constexpr int THREADS = TC * M;
     static constexpr size_t SMEM = (size_t)TC * P::NP * sizeof(cpx<R>);
     static_assert(THREADS % 32 == 0, "column CTA must be whole warps");
