@@ -76,6 +76,21 @@ int slm_gs_run(slm_ctx* ctx, int batch, const uint8_t* target_u8, const void* ta
                const double* amp_lut, const double* norm, const void* inc_amp, const void* phasor0, int setup_c64,
                int max_loops, double tolerance, double* hologram_out, double* expected_out);
 
+/* Weighted Gerchberg-Saxton (GSW; Di Leonardo, Ianni & Ruocco, Opt. Express 15, 1913 (2007)): GS with per-pixel
+ * weights w on the target amplitude, so that the reconstructed intensity follows the target's levels (uniform trap
+ * arrays).  Per iteration k, on the signal set {T > 0} where I_k = |C_k|^2 > 0:
+ *     w_k = clamp(w_{k-1} * amp / sqrt(sigma_k * I_k), 1/weight_limit, weight_limit),   D_k = (amp * w_k) * C_k / |C_k|
+ * with sigma_k = target_sum / P_{k-1}, P = sum of I over the signal set (P_0 for k = 0); elsewhere w_k = w_{k-1}.
+ * Scale, error curve, tolerance stop, expected outcome and hologram are GS's; weight_limit = 1 gives GS's bits.
+ * Arguments as slm_gs_run, plus
+ *   target_sum     host double[batch]: sum(T) per plane
+ *   weights        device real<R> [batch][H][W]: initial weights in (ones for plain GSW), final weights out
+ *   weight_limit   c >= 1 (else SLM_ERR_ARG) */
+int slm_gsw_run(slm_ctx* ctx, int batch, const uint8_t* target_u8, const void* target_real, const void* amp_real,
+                const double* amp_lut, const double* norm, const void* inc_amp, const void* phasor0, int setup_c64,
+                int max_loops, double tolerance, double* hologram_out, double* expected_out,
+                const double* target_sum, void* weights, double weight_limit);
+
 /* gradient_descent(demanded_output, args) -- algorithms.py:60-112 (+ dEdX_complex :179-185).
  *   x              device complex<R> [batch][H][W]: the initial guess (algorithms.py:75), updated in place
  *   mask_lut       host double[256]: 1 + white_attention*g/255 for g = 0..255 as numpy computes it

@@ -31,6 +31,7 @@ SIGNATURES = {
     "slm_ctx_profile_read": (_i, [_vp, _dp, C.POINTER(_ll)]),
     "slm_fft2": (_i, [_vp, _i, _vp, _vp, _i]),
     "slm_gs_run": (_i, [_vp, _i, _vp, _vp, _vp, _dp, _dp, _vp, _vp, _i, _i, _d, _vp, _vp]),
+    "slm_gsw_run": (_i, [_vp, _i, _vp, _vp, _vp, _dp, _dp, _vp, _vp, _i, _i, _d, _vp, _vp, _dp, _vp, _d]),
     "slm_gd_run": (_i, [_vp, _i, _vp, _vp, _vp, _dp, _dp, _vp, _vp, _dp, _i, _d, _vp, _vp]),
     "slm_fourier_guess": (_i, [_vp, _i, _vp, _vp, _dp, _vp, _i, _vp]),
     "slm_random_phasor": (_i, [_vp, _vp, _vp, _ll, _d]),

@@ -23,7 +23,7 @@ import numpy as np
 from . import host_logic as hl
 from .engine import Engine, get_engine
 
-__all__ = ["gerchberg_saxton", "gradient_descent", "make_initial_guess", "error_f", "printout",
+__all__ = ["gerchberg_saxton", "weighted_gerchberg_saxton", "gradient_descent", "make_initial_guess", "error_f", "printout",
            "complex_to_real_phase", "dEdX_complex", "add_gif_image"]
 
 
@@ -68,6 +68,32 @@ def gerchberg_saxton(demanded_output, args):
         res = eng.gs(target, int(args.max_loops), float(args.tolerance), inc_amp=inc)
         errors = [np.float64(e) for e in res.errors[0]]
         hologram, expected = (a[0] for a in eng.to_host_many([res.hologram, res.expected]))
+    _progress(len(errors), args.max_loops)
+    if args.print_info:
+        print()
+        printout(errors[-1], len(errors), errors, args.plot_error)
+    return hologram, expected, errors
+
+
+def weighted_gerchberg_saxton(demanded_output, args):
+    """Weighted Gerchberg-Saxton (Di Leonardo, Ianni & Ruocco, Opt. Express 15, 1913 (2007)): GS whose target
+    amplitude carries per-pixel weights, fed back each iteration so that the reconstructed intensity follows the
+    target's levels -- plain GS leaves trap arrays with a spread of intensities.  The contract of
+    :func:`gerchberg_saxton` (error curve and expected outcome are computed the same way, so the curves compare
+    directly), plus the optional ``args.weight_limit`` (default 10): the weights stay within [1/limit, limit].
+    ``args.gif`` snapshots are not offered (ValueError)."""
+    if getattr(args, "gif", False):
+        raise ValueError("weighted_gerchberg_saxton does not offer GIF snapshots (args.gif)")
+    target = np.asarray(demanded_output)
+    inc = _illumination(args, target.shape)
+    if args.max_loops < 1 or not (args.tolerance + 1 > args.tolerance):
+        print()
+        raise UnboundLocalError("cannot access local variable 'expected_outcome' where it is not associated with a value")
+    eng = _engine(target.shape, args)
+    res, _w = eng.gsw(target, int(args.max_loops), float(args.tolerance), inc_amp=inc,
+                      weight_limit=float(getattr(args, "weight_limit", 10.0)))
+    errors = [np.float64(e) for e in res.errors[0]]
+    hologram, expected = (a[0] for a in eng.to_host_many([res.hologram, res.expected]))
     _progress(len(errors), args.max_loops)
     if args.print_info:
         print()

@@ -48,6 +48,8 @@ struct slm_ctx {
     int fused_ctas = 0;                                   // grid of the fused GD column pass (0: two passes)
     bool pipe_ok = false;                                 // CGM_GD_PIPE may be used (warp-per-column kernel, a plane's tiles fit the CTAs' buffers)
     double *err_curve = nullptr, *lr = nullptr, *norm = nullptr;
+    // weighted GS, allocated by the first slm_gsw_run: [max_batch] S_T, [max_batch] P, [max_batch][tiles] partials of P
+    double *target_sum = nullptr, *signal_sum = nullptr, *signal_partial = nullptr;
     void* lut = nullptr;
     float* lut32 = nullptr;
     double lut_host[256];                                 // the table the device copies hold (upload_lut)
@@ -397,7 +399,7 @@ template <class F> static int replay_iterations(slm_ctx* c, int batch, int times
 }
 
 extern "C" const char* slm_last_error(void) { return g_err.c_str(); }
-extern "C" int slm_version(void) { return 102; }
+extern "C" int slm_version(void) { return 103; }
 extern "C" int slm_supported_lengths(int* out, int cap) { return supported_lengths(out, cap); }
 
 extern "C" void slm_ctx_destroy(slm_ctx* c) {
@@ -666,6 +668,65 @@ extern "C" int slm_gs_run(slm_ctx* c, int batch, const uint8_t* T8, const void* 
         }
         SLM_TIMED(K_COL_PLAIN, c->col->col_plain(ia, c->stream));
     }
+    return 0;
+}
+
+// Weighted GS: the launches of slm_gs_run's one-CTA-per-tile branch ("gs/plain") at every batch size, with the GSW
+// forms of the max pre-pass and of the column pass (col_pass_tile<ALG_GSW>).  The persistent column kernels have no
+// room for a weight tile (col_warp.cuh: three 64 KB tile buffers), so the context's batch does not choose a kernel here.
+extern "C" int slm_gsw_run(slm_ctx* c, int batch, const uint8_t* T8, const void* Treal, const void* amp_real,
+                           const double* amp_lut, const double* norm, const void* inc_amp, const void* phasor0,
+                           int setup_c64, int max_loops, double tolerance, double* hologram_out, double* expected_out,
+                           const double* target_sum, void* weights, double weight_limit) {
+    SLM_TRY(check_batch(c, batch, "slm_gsw_run"));
+    if (max_loops < 1) return fail(SLM_ERR_ARG, "slm_gsw_run: max_loops must be >= 1");
+    if (!norm || !hologram_out || !target_sum || !weights) return fail(SLM_ERR_ARG, "slm_gsw_run: norm, target_sum, weights and hologram_out are required");
+    if (T8 ? !amp_lut : !(Treal && amp_real)) return fail(SLM_ERR_ARG, "slm_gsw_run: give target_u8 + amp_lut, or target_real + amp_real");
+    if (!(weight_limit >= 1.0)) return fail(SLM_ERR_ARG, "slm_gsw_run: weight_limit must be >= 1");
+    if (!c->target_sum) {
+        SLM_TRY(dev_alloc(c, (void**)&c->target_sum, (size_t)c->max_batch * sizeof(double)));
+        SLM_TRY(dev_alloc(c, (void**)&c->signal_sum, (size_t)c->max_batch * sizeof(double)));
+        SLM_TRY(dev_alloc(c, (void**)&c->signal_partial, (size_t)c->max_batch * c->tiles * sizeof(double)));
+    }
+    SLM_TRY(begin_run(c, batch, norm, max_loops));
+    SLM_CUDA(cudaMemcpyAsync(c->target_sum, target_sum, (size_t)batch * sizeof(double), cudaMemcpyHostToDevice, c->stream));
+    if (T8) SLM_TRY(upload_lut(c, amp_lut));
+
+    RowArgs ra{};
+    ra.B = batch; ra.H = c->H; ra.Y = c->Y; ra.X = c->X; ra.inc = inc_amp; ra.stats = c->stats;
+    ra.inv_hw = 1.0 / ((double)c->H * c->W); ra.hologram = hologram_out; ra.tw = c->tw_row;
+    if (phasor0) { ra.source = ROW_FROM_FIELD; ra.field = phasor0; }
+    else {
+        int src = 0;
+        SLM_TRY(setup_field(c, batch, T8, amp_real, setup_c64, &src));
+        ra.source = src; ra.A32 = c->Y; ra.field = c->Y;
+    }
+    SLM_TIMED(K_ROW_PASS, c->row->row_pass(ALG_GS, ra, c->stream));
+
+    ColArgs ca{};
+    ca.B = batch; ca.W = c->W; ca.X = c->X; ca.Y = c->Y; ca.T8 = T8; ca.Treal = Treal; ca.plane2 = amp_real;
+    ca.lut = c->lut; ca.norm = c->norm; ca.stats = c->stats; ca.partial = c->partial; ca.counter = c->counter;
+    ca.err_curve = c->err_curve; ca.max_loops = max_loops; ca.tolerance = tolerance;
+    ca.inv_hw = ra.inv_hw; ca.tw = c->tw_col;
+    ca.weights = weights; ca.target_sum = c->target_sum; ca.signal_sum = c->signal_sum; ca.signal_partial = c->signal_partial;
+    ca.weight_limit = weight_limit;
+    // exact scale of iteration 0 (as GS takes it) and P_0 for sigma_0
+    SLM_TIMED(K_COL_STATS, c->col->col_pass(ALG_GSW_STATS, ca, c->stream));
+    ra.source = ROW_FROM_Y;
+    std::string key("gsw/plain");                                   // every argument the loop's launches are made of
+    RowArgs ra_key = ra;
+    ra_key.hologram = nullptr;
+    key.append(reinterpret_cast<const char*>(&ra_key), sizeof ra_key).append(reinterpret_cast<const char*>(&ca), sizeof ca);
+    key.append(reinterpret_cast<const char*>(&batch), sizeof batch);
+    SLM_TRY(replay_iterations(c, batch, max_loops - 1, key, [&]() -> int {
+        SLM_TIMED(K_COL_PASS, c->col->col_pass(ALG_GSW, ca, c->stream));
+        SLM_TIMED(K_ROW_PASS, c->row->row_pass(ALG_GS, ra, c->stream));
+        return 0;
+    }));
+    SLM_TIMED(K_COL_PASS, c->col->col_pass(ALG_GSW, ca, c->stream));
+    ra.final_pass = 1;
+    SLM_TIMED(K_ROW_PASS, c->row->row_pass(ALG_GS, ra, c->stream));
+    if (expected_out) SLM_TIMED(K_COL_PLAIN, c->col->col_plain(stats_args(c, batch, OUT_INTENSITY_GS, expected_out), c->stream));
     return 0;
 }
 

@@ -6,7 +6,9 @@
 namespace slm {
 
 enum Precision { PREC_F32 = 0, PREC_F64 = 1 };
-enum Algorithm { ALG_GS = 0, ALG_GD = 1 };
+// ALG_GSW: weighted GS (per-pixel amplitude feedback, DESIGN.md); ALG_GSW_STATS selects its iteration-0 pre-pass
+// (col_gsw_stats_kernel) in LineTable::col_pass
+enum Algorithm { ALG_GS = 0, ALG_GD = 1, ALG_GSW = 2, ALG_GSW_STATS = 3 };
 
 // ---- per-plane loop state, device resident --------------------------------------------------
 // Written only by the last column tile of a plane to finish a Fourier-plane pass.
@@ -68,6 +70,12 @@ struct ColArgs {
     unsigned* fused_max;     // one-pass GD forms: [max_planes] pairs {bit pattern of the plane's running max |F|^2, tiles that have
                              // contributed} (8-byte aligned, 0 between launches) + the time-out flag behind them (col_warp.cuh)
     int max_planes;
+    // weighted GS (ALG_GSW, ALG_GSW_STATS); appended so that the offsets the other kernels read stay where they were
+    void* weights;           // real<R> [B][H][W]: w_{k-1} in, w_k out
+    const double* target_sum;   // [B] sum(T), the signal energy S_T
+    double* signal_sum;      // [B] P = sum of |C|^2 over {T > 0} of the latest Fourier-plane pass (written by the last tile)
+    double* signal_partial;  // [B][W / TC] per-tile partial sums of P
+    double weight_limit;     // c >= 1: weights are clamped to [1/c, c]
 };
 
 // ---- warp-specialised persistent column kernel (col_groups.cuh) ---------------------------------------

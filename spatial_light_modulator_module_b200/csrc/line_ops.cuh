@@ -140,12 +140,16 @@ template <typename R, int L> struct ColLaunch {
     static void prepare() {
         cudaFuncSetAttribute(col_pass_kernel<R, L, ALG_GS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CG::SMEM);
         cudaFuncSetAttribute(col_pass_kernel<R, L, ALG_GD>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CG::SMEM);
+        cudaFuncSetAttribute(col_pass_kernel<R, L, ALG_GSW>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CG::SMEM);
+        cudaFuncSetAttribute(col_gsw_stats_kernel<R, L>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CG::SMEM);
         cudaFuncSetAttribute(col_plain_kernel<R, L>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CG::SMEM);
         GroupLaunch<R, L>::prepare();
     }
     static int col_pass(int alg, const ColArgs& a, cudaStream_t s) {
         const dim3 grid((unsigned)((long long)a.B * (a.W / CG::TC))), block(CG::THREADS);
         if (alg == ALG_GS) SLM_LAUNCH((col_pass_kernel<R, L, ALG_GS>), grid, block, CG::SMEM, s, a);
+        else if (alg == ALG_GSW) SLM_LAUNCH((col_pass_kernel<R, L, ALG_GSW>), grid, block, CG::SMEM, s, a);
+        else if (alg == ALG_GSW_STATS) SLM_LAUNCH((col_gsw_stats_kernel<R, L>), grid, block, CG::SMEM, s, a);
         else SLM_LAUNCH((col_pass_kernel<R, L, ALG_GD>), grid, block, CG::SMEM, s, a);
         return check();
     }

@@ -79,8 +79,11 @@ template <int FIELDS> SLM_DEV Partial warp_reduce(Partial p) {
     }
     return p;
 }
-// Result valid in thread 0.  NT = threads per CTA (multiple of 32).
-template <int NT, int FIELDS> SLM_DEV Partial block_reduce(Partial p, int t) {
+// Result valid in thread 0.  NT = threads per CTA (multiple of 32).  OWNER: calls with different values use separate
+// `red` arrays.  The weighted-GS kernels pass 1, so that they share no array with the other kernels: an array that one
+// kernel alone uses is allocated with it, one that several use is a module variable, and that alone changed the
+// registers the GS column kernel got.
+template <int NT, int FIELDS, int OWNER = 0> SLM_DEV Partial block_reduce(Partial p, int t) {
     static_assert(NT % 32 == 0 && NT <= 1024, "CTA size");
     SLM_STATIC_SMEM Partial red[32];
     p = warp_reduce<FIELDS>(p);
@@ -112,6 +115,14 @@ template <int FIELDS> SLM_DEV bool collect_if_last(unsigned ticket, int t, const
     for (int i = t; i < tiles; i += 32) q = combine<FIELDS>(q, ld_partial(plane_partials + i));
     total = warp_reduce<FIELDS>(q);
     return true;
+}
+// warp 0 of a plane's last tile, after collect_if_last: the plane total of one more per-tile sum, in every lane
+SLM_DEV double collect_sum(int t, const double* plane_partials, int tiles) {
+    double q = 0;
+    for (int i = t; i < tiles; i += 32) q += ld_cg(plane_partials + i);
+#pragma unroll
+    for (int m = 16; m >= 1; m >>= 1) q += shfl_xor(q, m);
+    return q;
 }
 // Publish this tile's partial; returns (to every thread) whether this CTA is the last of its plane,
 // in which case thread 0 of it receives the plane total in `total`.
@@ -283,12 +294,19 @@ SLM_GLOBAL void SLM_LAUNCH_BOUNDS((RowGeom<R, W>::THREADS), (RowGeom<R, W>::MIN_
 // Ordering is chosen so no warp waits on a dependent global access: the grey levels are requested
 // before the forward transform and only looked up (in shared memory) after it; the tile's partial
 // sums are published before the inverse transform, whose work covers the atomic's round trip.
+//
+// ALG_GSW is GS with per-pixel weights w on the amplitude (weighted GS, Di Leonardo, Ianni & Ruocco, Opt. Express 15,
+// 1913 (2007)): on the signal set {T > 0} where |C|^2 > 0, w_k = clamp(w_{k-1} amp / sqrt(sigma |C|^2), 1/c, c) with
+// sigma = S_T / P_{k-1} (P: the signal set's sum of |C|^2 of the previous pass -- of this one at iteration 0, from the
+// pre-pass), and D = (amp w) C/|C|.  Scale, error and loop condition are GS's.  amp * w is formed first, so with c = 1
+// (w == 1.0 exactly) the arithmetic is GS's, bit for bit.
 template <typename R, int H, int ALG>
 SLM_DEV void col_pass_tile(const ColArgs& a, int b, int tile, int tiles, cpx<R>* v, cpx<R>* line, const R* lut_s,
                            int t, int c, int j) {
     using G = ColGeom<R, H>;
     using P = ColPlan<H>;
     constexpr int E = P::E, M = P::M, TC = G::TC;
+    constexpr bool GSW = ALG == ALG_GSW;
     PlaneStats* st = a.stats + b;
     const size_t W = a.W;
     const size_t off = (size_t)b * H * W + (size_t)j * W + tile * TC + c;
@@ -314,18 +332,34 @@ SLM_DEV void col_pass_tile(const ColArgs& a, int b, int tile, int tiles, cpx<R>*
 
     // per-thread sums in R (E terms), widened to double before they meet other threads
     R mx = 0, sa = 0, sb = 0, sc = 0;
+    R sp = 0;                                                   // GSW: P, the signal set's sum of |C|^2
     const R s0r = (R)s0;                                        // GS: scale of the previous iteration
     const R gdk = sizeof(R) == 8 ? (R)0 : (R)(norm / imax);    // GD fp32: output = |F|^2 * (norm/max)
+    const R sig = GSW ? (R)(ld_ro(a.target_sum + b) / ld_cg(a.signal_sum + b)) : (R)0;   // sigma_k = S_T / P_{k-1}
+    const R wlo = GSW ? (R)(1.0 / a.weight_limit) : (R)0, whi = GSW ? (R)a.weight_limit : (R)0;
 #pragma unroll
     for (int r = 0; r < E; ++r) {
         const R m2 = cnorm2(v[r]);                              // |C|^2, algorithms.py:36 / :85
-        if (ALG == ALG_GS) {
+        if (ALG == ALG_GS || GSW) {
             // error of this iteration against the scale s0 of the previous one; the exact scale
             // s = norm/max is folded in by the last tile (see finish below).
             const R u = s0r * m2, d = u - tv[r];
             mx = fmax(mx, m2); sa += d * d; sb += d * u; sc += u * u;
+            R amp = aux[r];
+            if (GSW) {
+                // the weights are read here, after the forward transform, not before it like the target: held through
+                // the transform they would not fit in registers at the long lines
+                R* const wp = static_cast<R*>(a.weights) + off + (size_t)r * M * W;
+                R w = ld_cg(wp);
+                if (tv[r] > (R)0) {
+                    sp += m2;
+                    if (m2 > (R)0) w = fmin(fmax(w * aux[r] * rsqrt_fast(sig * m2), wlo), whi);
+                }
+                st_cg(wp, w);
+                amp = aux[r] * w;
+            }
             // D = |amp| * exp(1j*angle(C)), algorithms.py:33
-            v[r] = (m2 == (R)0) ? mk<R>(copysign(aux[r], v[r].x), (R)0) : cscale(v[r], aux[r] * rsqrt_fast(m2));
+            v[r] = (m2 == (R)0) ? mk<R>(copysign(amp, v[r].x), (R)0) : cscale(v[r], amp * rsqrt_fast(m2));
         } else {
             R I;                                                 // output, algorithms.py:86
             if (sizeof(R) == 8) I = (R)(((double)m2 * norm) / imax);
@@ -335,9 +369,15 @@ SLM_DEV void col_pass_tile(const ColArgs& a, int b, int tile, int tiles, cpx<R>*
             v[r] = cscale(cscale(v[r], aux[r]), d);              // mask * med_output * (output - T), :88
         }
     }
-    constexpr int FIELDS = ALG == ALG_GS ? F_ALL : F_A;
+    constexpr int FIELDS = ALG == ALG_GD ? F_A : F_ALL;
     Partial p; p.mx = (double)mx; p.a = (double)sa; p.b = (double)sb; p.c = (double)sc;
-    p = block_reduce<G::THREADS, FIELDS>(p, t);
+    p = block_reduce<G::THREADS, FIELDS, GSW ? 1 : 0>(p, t);
+    double* sig_partials = GSW ? a.signal_partial + (size_t)b * tiles : nullptr;
+    if (GSW) {
+        Partial q; q.mx = 0; q.a = 0; q.b = (double)sp; q.c = 0;
+        q = block_reduce<G::THREADS, F_B, 1>(q, t);           // (F_B: shared memory of its own, apart from the reduce above)
+        if (t == 0) sig_partials[tile] = q.b;                   // published by the fence in publish_partial
+    }
     Partial* plane_partials = a.partial + (size_t)b * tiles;
     unsigned ticket = 0;
     if (t == 0) ticket = publish_partial(p, plane_partials, tile, tiles, a.counter + b);
@@ -350,10 +390,14 @@ SLM_DEV void col_pass_tile(const ColArgs& a, int b, int tile, int tiles, cpx<R>*
     if (t >= 32) return;
     Partial tot;
     if (!collect_if_last<FIELDS>(ticket, t, plane_partials, tiles, tot)) return;
+    if (GSW) {
+        const double psum = collect_sum(t, sig_partials, tiles);
+        if (t == 0) a.signal_sum[b] = psum;
+    }
     if (t == 0) {
         const double hw = (double)H * (double)W;
         double err;
-        if (ALG == ALG_GS) {
+        if (ALG != ALG_GD) {
             const double s = norm / tot.mx;                      // algorithms.py:37
             const double s0u = (double)s0r;                      // the scale the tiles actually used
             const double dl = (s0u != 0.0) ? s / s0u - 1.0 : 0.0;
@@ -455,6 +499,59 @@ SLM_GLOBAL void SLM_LAUNCH_BOUNDS((ColGeom<R, H>::THREADS), 1) col_pass_kernel(C
         [&](int b) { return ld_cg(&a.stats[b].done) != 0; },
         [&](int b, int tile, int tiles, cpx<R>* v, cpx<R>* line, int t, int c, int j) {
             col_pass_tile<R, H, ALG>(a, b, tile, tiles, v, line, lut_s, t, c, j);
+        });
+}
+
+// Weighted GS, iteration 0: the forward transform's max |C|^2 -> stats (as col_plain_tile's OUT_STATS takes it, so the
+// scale is GS's) and the signal set's sum P_0 of |C|^2 -> signal_sum, for sigma_0 = S_T / P_0 of the first ALG_GSW pass.
+template <typename R, int H>
+SLM_GLOBAL void SLM_LAUNCH_BOUNDS((ColGeom<R, H>::THREADS), 1) col_gsw_stats_kernel(ColArgs a) {
+    SLM_DYN_SMEM(raw);
+    col_tiles<R, H>(a.X, a.W, raw,
+        [&](int b) { return ld_cg(&a.stats[b].done) != 0; },
+        [&](int b, int tile, int tiles, cpx<R>* v, cpx<R>* line, int t, int c, int j) {
+            using G = ColGeom<R, H>;
+            using P = ColPlan<H>;
+            constexpr int E = P::E, M = P::M, TC = G::TC;
+            const size_t W = a.W;
+            const size_t off = (size_t)b * H * W + (size_t)j * W + tile * TC + c;
+            bool sig[E];                                                // the point lies in the signal set {T > 0}
+            if (a.T8) {
+#pragma unroll
+                for (int r = 0; r < E; ++r) sig[r] = ld_ro(a.T8 + off + (size_t)r * M * W) != 0;
+            } else {
+                const R* T = static_cast<const R*>(a.Treal) + off;
+#pragma unroll
+                for (int r = 0; r < E; ++r) sig[r] = ld_ro(T + (size_t)r * M * W) > (R)0;
+            }
+            line_fft<R, H, -1, TC, CtaSync, false, column_points(H)>(v, line, j, static_cast<const cpx<R>*>(a.tw));
+            R mx = 0, sp = 0;
+#pragma unroll
+            for (int r = 0; r < E; ++r) {
+                const R m2 = cnorm2(v[r]);
+                mx = fmax(mx, m2);
+                if (sig[r]) sp += m2;
+            }
+            Partial p; p.mx = (double)mx; p.a = 0; p.b = 0; p.c = 0;
+            p = block_reduce<G::THREADS, F_MX, 1>(p, t);
+            Partial q; q.mx = 0; q.a = 0; q.b = (double)sp; q.c = 0;
+            q = block_reduce<G::THREADS, F_B, 1>(q, t);
+            if (t >= 32) return;
+            Partial* plane_partials = a.partial + (size_t)b * tiles;
+            double* sig_partials = a.signal_partial + (size_t)b * tiles;
+            unsigned ticket = 0;
+            if (t == 0) {
+                sig_partials[tile] = q.b;
+                ticket = publish_partial(p, plane_partials, tile, tiles, a.counter + b);
+            }
+            Partial tot;
+            if (!collect_if_last<F_MX>(ticket, t, plane_partials, tiles, tot)) return;
+            const double psum = collect_sum(t, sig_partials, tiles);
+            if (t == 0) {
+                PlaneStats* st = a.stats + b;
+                st->imax = tot.mx; st->scale = ld_ro(a.norm + b) / tot.mx;
+                a.signal_sum[b] = psum;
+            }
         });
 }
 

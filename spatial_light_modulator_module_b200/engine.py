@@ -124,8 +124,18 @@ class Engine:
         """max over each plane of a uint8 device stack [B,H,W] -> float64 [B] on the host."""
         return np.ascontiguousarray(dev.reshape(dev.shape[0], -1).amax(dim=1).double().cpu().numpy(), dtype=np.float64)
 
+    def _mem_plane_sum(self, dev) -> np.ndarray:
+        """sum over each plane of a uint8 device stack [B,H,W] -> float64 [B] on the host (exact: integer sums)."""
+        return np.ascontiguousarray(dev.reshape(dev.shape[0], -1).sum(dim=1, dtype=self._torch.float64).cpu().numpy(),
+                                    dtype=np.float64)
+
     def _mem_contiguous(self, dev):
         return dev.contiguous()
+
+    def _mem_fill(self, buf, value) -> None:
+        """set every element of a device buffer, in order on the engine's stream"""
+        with self._torch.cuda.stream(self._stream):
+            buf.fill_(value)
 
     def _mem_repeat(self, plane, n: int):
         """[1,H,W] device plane -> [n,H,W] copies (every target of a batch starts from the same guess)"""
@@ -246,6 +256,45 @@ class Engine:
             self._dp(self._amp_lut), self._dp(norms), self._mem_ptr(inc_dev), self._mem_ptr(ph_dev), int(c64),
             int(max_loops), float(tolerance), self._mem_ptr(holo), self._mem_ptr(exp)))
         return self._collect(batch, max_loops, holo, exp)
+
+    def gsw(self, targets, max_loops: int, tolerance: float = 0.0, inc_amp=None, phasor0=None, weight_limit: float = 10.0,
+            weights=None, want_expected: bool = True, norms=None):
+        """Weighted GS (include/slm_holo.h slm_gsw_run): GS whose target amplitude carries per-pixel weights, which
+        even out the intensities of trap arrays.  ``weights``: initial weights [B,H,W] (host or device; a device tensor
+        of the engine's real dtype is updated in place), None = ones.  ``weight_limit`` >= 1 bounds them to
+        [1/weight_limit, weight_limit]; 1 gives GS's results bit for bit.  Scale, error curve, tolerance stop and
+        expected outcome are GS's.  Returns (LoopResult, weights_device)."""
+        if max_loops < 1:
+            raise UnboundLocalError("cannot access local variable 'expected_outcome' where it is not associated with a value")
+        if not float(weight_limit) >= 1.0:
+            raise ValueError(f"weight_limit must be >= 1, not {weight_limit!r}")
+        batch, t8, treal, amp, norms, c64 = self._targets(targets, norms)
+        if t8 is not None and self._mem_is_device(targets):
+            sums = self._mem_plane_sum(t8)
+        else:
+            sums = np.asarray(targets).reshape(batch, -1).sum(axis=1, dtype=np.float64)      # S_T, like the norms
+        sums = np.ascontiguousarray(sums, dtype=np.float64)
+        shape = (batch,) + self.shape
+        if weights is None:
+            w = self._mem_empty(shape, self.real_dtype)
+            self._mem_fill(w, 1.0)
+        else:
+            w = self._as_device(weights, self.real_dtype, "weights")
+            if tuple(w.shape) == self.shape and batch == 1:
+                w = w[None]
+            if tuple(w.shape) != shape:
+                raise ValueError(f"weights must have shape {shape}, not {tuple(w.shape)}")
+        amp_dev = self._mem_upload(amp.astype(self.real_dtype)) if amp is not None else None
+        inc_dev = self._as_device(inc_amp, self.real_dtype, "inc_amp")
+        ph_dev = self._as_device(phasor0, self.complex_dtype, "phasor0")
+        holo = self._mem_empty(shape, np.float64)
+        exp = self._mem_empty(shape, np.float64) if want_expected else None
+        self._check(self._lib.slm_gsw_run(
+            self._ctx, batch, self._mem_ptr(t8), self._mem_ptr(treal), self._mem_ptr(amp_dev),
+            self._dp(self._amp_lut), self._dp(norms), self._mem_ptr(inc_dev), self._mem_ptr(ph_dev), int(c64),
+            int(max_loops), float(tolerance), self._mem_ptr(holo), self._mem_ptr(exp),
+            self._dp(sums), self._mem_ptr(w), float(weight_limit)))
+        return self._collect(batch, max_loops, holo, exp), w
 
     # ---- gradient descent (algorithms.py:60-112) --------------------------------------------------------
     def gd(self, targets, x0, lr_schedule, max_loops: int, tolerance: float = 0.0, white_attention=1,

@@ -11,8 +11,12 @@ from PIL import Image as im
 
 from . import constants as c
 from . import wavefront_correction as wfc
-from .algorithms import gerchberg_saxton, gradient_descent
+from .algorithms import gerchberg_saxton, gradient_descent, weighted_gerchberg_saxton
 from .engine import get_engine
+
+# -alg choices -> hologram functions (the reference sends every choice but GS to gradient descent)
+ALGORITHMS = {"gerchberg_saxton": gerchberg_saxton, "gradient_descent": gradient_descent,
+              "weighted_gerchberg_saxton": weighted_gerchberg_saxton}
 
 
 def main(args):
@@ -62,7 +66,7 @@ def pad_to_square(img):
 
 def make_hologram(args):
     """reference: generate_hologram.py:70-79."""
-    algorithm = gerchberg_saxton if args.algorithm == "gerchberg_saxton" else gradient_descent
+    algorithm = ALGORITHMS.get(args.algorithm, gradient_descent)
     target = prepare_target(args.img_name, args)
     if getattr(args, "gif", False):
         add_gif_dirs(args)
@@ -215,7 +219,7 @@ def build_parser():
     p.add_argument("-dest_dir", "--destination_directory", type=str, default="holograms", help="where the hologram is saved")
     p.add_argument("-q", "--quarterize", action="store_true", help="shrink the target into one quadrant of a black image")
     p.add_argument("-i", "--invert", action="store_true", help="invert the target image")
-    p.add_argument("-alg", "--algorithm", default="gerchberg_saxton", choices=["gerchberg_saxton", "gradient_descent"])
+    p.add_argument("-alg", "--algorithm", default="gerchberg_saxton", choices=list(ALGORITHMS))
     p.add_argument("-tol", "--tolerance", default=0, metavar="FLOAT", type=float, help="stop when the error falls to this value")
     p.add_argument("-l", "--max_loops", default=42, metavar="INTEGER", type=int, help="upper bound on the number of iterations")
     p.add_argument("-lr", "--learning_rate", default=0.005, type=float, help="gradient descent step")
@@ -230,6 +234,8 @@ def build_parser():
                    help="add a deflection hologram (units: a quarter of the first diffraction maximum)")
     p.add_argument("-lens", default=None, type=float, metavar="FOCAL_LENGTH", help="add a lens of this focal length [m]")
     p.add_argument("--precision", default=None, choices=["fp32", "fp64"], help="engine arithmetic (default fp32)")
+    p.add_argument("--weight_limit", default=10.0, type=float, metavar="FLOAT",
+                   help="weighted_gerchberg_saxton: the weights stay within [1/limit, limit] (>= 1)")
     return p
 
 

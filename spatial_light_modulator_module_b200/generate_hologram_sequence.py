@@ -29,9 +29,13 @@ def _dist():
 def sequence_holograms(frames, max_loops: int, tolerance: float = 0.0, precision: str = "fp32",
                        batch: Optional[int] = None, want_expected: bool = False, engine_factory: Optional[Callable] = None,
                        gather: bool = True, inc_amp=None, warm_start: bool = False, output: str = "float64",
-                       mask=None, ct2pi=256, trap_dots=None, on_batch: Optional[Callable] = None):
+                       mask=None, ct2pi=256, trap_dots=None, on_batch: Optional[Callable] = None,
+                       weighted: bool = False, weight_limit: float = 10.0):
     """GS holograms of ``frames`` (uint8 [F,H,W], a host array or a device tensor); ``inc_amp``: illumination amplitude
     plane [H,W] shared by all frames (algorithms.py:14-19), None = uniform.
+
+    ``weighted``: weighted GS (Engine.gsw, weights bounded by ``weight_limit``) instead of GS, for trap intensities
+    that follow the frames' grey levels.  Every frame's weights start at 1 (``warm_start`` carries only the phase).
 
     ``output``: "float64" -- the holograms as the reference saves them (generate_hologram_sequence.py:26, 8 bytes per
     pixel); "uint8" -- the frames the SLM is shown: wavefront-correction ``mask`` added (None: no mask) and quantised
@@ -111,6 +115,12 @@ def sequence_holograms(frames, max_loops: int, tolerance: float = 0.0, precision
     errors: List[np.ndarray] = []
     writer = _Writer(on_batch)
 
+    def run(targets, phasor0=None):
+        if weighted:
+            return eng.gsw(targets, max_loops, tolerance, inc_amp=inc_amp, phasor0=phasor0, weight_limit=weight_limit,
+                           want_expected=want_expected)[0]
+        return eng.gs(targets, max_loops, tolerance, inc_amp=inc_amp, phasor0=phasor0, want_expected=want_expected)
+
     def finish(res):
         """device results of one batch in the requested output format"""
         if output == "float64":
@@ -134,7 +144,7 @@ def sequence_holograms(frames, max_loops: int, tolerance: float = 0.0, precision
             raise ValueError("warm_start chains the frames of a block: gather=False only")
         phasor = None
         for s in range(n_local):
-            res = eng.gs(targets_of(s, s + 1), max_loops, tolerance, inc_amp=inc_amp, phasor0=phasor, want_expected=want_expected)
+            res = run(targets_of(s, s + 1), phasor0=phasor)
             holos[s] = eng.to_host(finish(res))[0]
             if want_expected:
                 exps[s] = eng.to_host(res.expected)[0]
@@ -150,7 +160,7 @@ def sequence_holograms(frames, max_loops: int, tolerance: float = 0.0, precision
         res, cur = None, ahead
         ahead = targets_of(s + batch, min(s + 2 * batch, n_local))        # the next batch's frames travel beside this batch's iterations
         if e > s:
-            res = eng.gs(cur, max_loops, tolerance, inc_amp=inc_amp, want_expected=want_expected, norms=None)
+            res = run(cur)
             errors.extend(res.errors)
         for jobs, a, b in pending:
             writer.put(jobs, a, b, holos[a - base:b - base], exps[a - base:b - base] if want_expected else None)
@@ -287,7 +297,8 @@ def generate_hologram_sequence(args):
     _, _, errors, _ = sequence_holograms(
         frames, int(args.max_loops), float(args.tolerance), getattr(args, "precision", None) or
         os.environ.get("SLM_PRECISION", "fp32"), getattr(args, "batch", None), bool(args.preview), gather=False,
-        inc_amp=inc, on_batch=write)
+        inc_amp=inc, on_batch=write, weighted=bool(getattr(args, "weighted", False)),
+        weight_limit=float(getattr(args, "weight_limit", 10.0)))
     plot_error_evolution([list(e) for e in errors])
     return errors
 
@@ -320,6 +331,9 @@ def build_parser():
     p.add_argument("-p", "--preview", action="store_true", help="also write the expected images of the holograms")
     p.add_argument("--batch", type=int, default=None, help="frames per device batch (default: chosen from the number of frames)")
     p.add_argument("--precision", default=None, choices=["fp32", "fp64"], help="engine arithmetic (default fp32)")
+    p.add_argument("--weighted", action="store_true", help="weighted Gerchberg-Saxton: even trap intensities")
+    p.add_argument("--weight_limit", default=10.0, type=float, metavar="FLOAT",
+                   help="weighted GS: the weights stay within [1/limit, limit] (>= 1)")
     return p
 
 
