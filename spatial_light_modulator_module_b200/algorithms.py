@@ -52,9 +52,23 @@ def _progress(i, max_loops):
     print()
 
 
-def gerchberg_saxton(demanded_output, args):
-    """classical Gerchberg-Saxton algorithm for generating phase holograms in far field regime
-    (reference: algorithms.py:10-49)."""
+def _report(args, hologram, expected, errors):
+    """The drop-ins' epilogue: progress line, then the reference's printout with ``args.print_info``."""
+    _progress(len(errors), args.max_loops)
+    if args.print_info:
+        print()
+        printout(errors[-1], len(errors), errors, args.plot_error)
+    return hologram, expected, errors
+
+
+def _to_host(eng, res):
+    """One plane's LoopResult -> (hologram, expected, errors) on the host."""
+    hologram, expected = (a[0] for a in eng.to_host_many([res.hologram, res.expected]))
+    return hologram, expected, [np.float64(e) for e in res.errors[0]]
+
+
+def _gs_family(demanded_output, args, run):
+    """gerchberg_saxton and weighted_gerchberg_saxton: ``run(eng, target, max_loops, inc, phasor0)`` -> LoopResult."""
     target = np.asarray(demanded_output)
     inc = _illumination(args, target.shape)
     if args.max_loops < 1 or not (args.tolerance + 1 > args.tolerance):
@@ -62,17 +76,23 @@ def gerchberg_saxton(demanded_output, args):
         print()
         raise UnboundLocalError("cannot access local variable 'expected_outcome' where it is not associated with a value")
     eng = _engine(target.shape, args)
-    if getattr(args, "gif", False):
-        hologram, expected, errors = _gs_with_snapshots(eng, target, inc, args)
-    else:
-        res = eng.gs(target, int(args.max_loops), float(args.tolerance), inc_amp=inc)
-        errors = [np.float64(e) for e in res.errors[0]]
-        hologram, expected = (a[0] for a in eng.to_host_many([res.hologram, res.expected]))
-    _progress(len(errors), args.max_loops)
-    if args.print_info:
-        print()
-        printout(errors[-1], len(errors), errors, args.plot_error)
-    return hologram, expected, errors
+    if not getattr(args, "gif", False):
+        return _report(args, *_to_host(eng, run(eng, target, int(args.max_loops), inc, None)))
+    phasor = None
+
+    def restart(res):
+        # the next chunk starts from B = inc*exp(1j*angle(A)) (algorithms.py:30), which is what the next iteration of
+        # an uninterrupted run computes
+        nonlocal phasor
+        phasor = eng.phase_phasor(res.hologram, inc)
+    return _report(args, *_with_snapshots(eng, args, lambda n, done: run(eng, target, n, inc, phasor), restart))
+
+
+def gerchberg_saxton(demanded_output, args):
+    """classical Gerchberg-Saxton algorithm for generating phase holograms in far field regime
+    (reference: algorithms.py:10-49)."""
+    return _gs_family(demanded_output, args, lambda eng, target, n, inc, phasor0:
+                      eng.gs(target, n, float(args.tolerance), inc_amp=inc, phasor0=phasor0))
 
 
 def weighted_gerchberg_saxton(demanded_output, args):
@@ -84,21 +104,9 @@ def weighted_gerchberg_saxton(demanded_output, args):
     ``args.gif`` snapshots are not offered (ValueError)."""
     if getattr(args, "gif", False):
         raise ValueError("weighted_gerchberg_saxton does not offer GIF snapshots (args.gif)")
-    target = np.asarray(demanded_output)
-    inc = _illumination(args, target.shape)
-    if args.max_loops < 1 or not (args.tolerance + 1 > args.tolerance):
-        print()
-        raise UnboundLocalError("cannot access local variable 'expected_outcome' where it is not associated with a value")
-    eng = _engine(target.shape, args)
-    res, _w = eng.gsw(target, int(args.max_loops), float(args.tolerance), inc_amp=inc,
-                      weight_limit=float(getattr(args, "weight_limit", 10.0)))
-    errors = [np.float64(e) for e in res.errors[0]]
-    hologram, expected = (a[0] for a in eng.to_host_many([res.hologram, res.expected]))
-    _progress(len(errors), args.max_loops)
-    if args.print_info:
-        print()
-        printout(errors[-1], len(errors), errors, args.plot_error)
-    return hologram, expected, errors
+    return _gs_family(demanded_output, args, lambda eng, target, n, inc, phasor0:
+                      eng.gsw(target, n, float(args.tolerance), inc_amp=inc, phasor0=phasor0,
+                              weight_limit=float(getattr(args, "weight_limit", 10.0)))[0])
 
 
 def gradient_descent(demanded_output, args):
@@ -108,26 +116,25 @@ def gradient_descent(demanded_output, args):
     inc = _illumination(args, target.shape)
     eng = _engine(target.shape, args)
     inc_amp = np.float64(1.0) if inc is None else inc        # (uniform illumination: make_initial_guess takes a scalar too)
-    x0 = make_initial_guess(args.initial_guess, inc_amp, target, args.random_seed, _engine_hint=eng, _device=True)
+    x = make_initial_guess(args.initial_guess, inc_amp, target, args.random_seed, _engine_hint=eng, _device=True)
     if args.print_info:
         print("computing hologram")
     if args.max_loops < 1 or not (args.tolerance + 1 > args.tolerance):
         print()
         raise UnboundLocalError("cannot access local variable 'output' where it is not associated with a value")
     during, after = hl.learning_rate_schedule(args.learning_rate, args.unsettle, int(args.max_loops))
+
+    def chunk(n, done):
+        nonlocal x
+        res, x = eng.gd(target, x, during[done:done + n], n, float(args.tolerance),
+                        white_attention=args.white_attention, inc_amp=inc)
+        return res
     if getattr(args, "gif", False):
-        hologram, expected, errors = _gd_with_snapshots(eng, target, x0, during, inc, args)
+        hologram, expected, errors = _with_snapshots(eng, args, chunk)
     else:
-        res, _x = eng.gd(target, x0, during, int(args.max_loops), float(args.tolerance),
-                         white_attention=args.white_attention, inc_amp=inc)
-        errors = [np.float64(e) for e in res.errors[0]]
-        hologram, expected = (a[0] for a in eng.to_host_many([res.hologram, res.expected]))
+        hologram, expected, errors = _to_host(eng, chunk(int(args.max_loops), 0))
     args.learning_rate = after[len(errors)]
-    _progress(len(errors), args.max_loops)
-    if args.print_info:
-        print()
-        printout(errors[-1], len(errors), errors, args.plot_error)
-    return hologram, expected, errors
+    return _report(args, hologram, expected, errors)
 
 
 def make_initial_guess(initial_guess_type, incomming_amplitude, demanded_output, seed, _engine_hint=None, _device=False):
@@ -203,36 +210,22 @@ def _save_snapshot(args, expected, hologram, i):
     img.convert("L").save(f"{args.gif_source_dir}/{i // args.gif_skip}.png")
 
 
-def _gs_with_snapshots(eng, target, inc, args):
-    """GS in chunks ending at the snapshot iterations; each chunk restarts from B = inc*exp(1j*angle(A))
-    (algorithms.py:30), which is what the next iteration of an uninterrupted run computes."""
-    errors, done, phasor, hologram, expected = [], 0, None, None, None
+def _with_snapshots(eng, args, chunk, restart=None):
+    """The loop in chunks that end at the iterations the reference snapshots; ``chunk(n, done)`` runs the next ``n``
+    iterations after ``done`` and returns their LoopResult; ``restart(result)`` follows every chunk that does not end
+    the run."""
+    errors, done, hologram, expected = [], 0, None, None
     for n in hl.snapshot_chunks(int(args.max_loops), int(args.gif_skip)):
-        res = eng.gs(target, n, float(args.tolerance), inc_amp=inc, phasor0=phasor)
+        res = chunk(n, done)
         errors += [np.float64(e) for e in res.errors[0]]
         hologram, expected = eng.to_host(res.hologram)[0], eng.to_host(res.expected)[0]
         last = done + len(res.errors[0]) - 1
         if last % args.gif_skip == 0:
             _save_snapshot(args, expected, hologram, last)
         done += n
-        # the loop condition (algorithms.py:29) holds across chunk borders: a chunk's last error ends the run too
+        # the loop condition (algorithms.py:29,83) holds across chunk borders: a chunk's last error ends the run too
         if len(res.errors[0]) < n or not (errors[-1] > float(args.tolerance)):
             break
-        phasor = eng.phase_phasor(res.hologram, inc)
-    return hologram, expected, errors
-
-
-def _gd_with_snapshots(eng, target, x0, during, inc, args):
-    errors, done, x, hologram, expected = [], 0, x0, None, None
-    for n in hl.snapshot_chunks(int(args.max_loops), int(args.gif_skip)):
-        res, x = eng.gd(target, x, during[done:done + n], n, float(args.tolerance),
-                        white_attention=args.white_attention, inc_amp=inc)
-        errors += [np.float64(e) for e in res.errors[0]]
-        hologram, expected = eng.to_host(res.hologram)[0], eng.to_host(res.expected)[0]
-        last = done + len(res.errors[0]) - 1
-        if last % args.gif_skip == 0:
-            _save_snapshot(args, expected, hologram, last)
-        done += n
-        if len(res.errors[0]) < n or not (errors[-1] > float(args.tolerance)):     # algorithms.py:83
-            break
+        if restart:
+            restart(res)
     return hologram, expected, errors

@@ -602,19 +602,62 @@ extern "C" int slm_fft2(slm_ctx* c, int batch, const void* in, void* out, int in
     return 0;
 }
 
-extern "C" int slm_gs_run(slm_ctx* c, int batch, const uint8_t* T8, const void* Treal, const void* amp_real,
-                          const double* amp_lut, const double* norm, const void* inc_amp, const void* phasor0,
-                          int setup_c64, int max_loops, double tolerance, double* hologram_out, double* expected_out) {
-    SLM_TRY(check_batch(c, batch, "slm_gs_run"));
-    if (max_loops < 1) return fail(SLM_ERR_ARG, "slm_gs_run: max_loops must be >= 1 (the reference raises UnboundLocalError for 0)");
-    if (!norm || !hologram_out) return fail(SLM_ERR_ARG, "slm_gs_run: norm and hologram_out are required");
-    if (T8 ? !amp_lut : !(Treal && amp_real)) return fail(SLM_ERR_ARG, "slm_gs_run: give target_u8 + amp_lut, or target_real + amp_real");
+// The start of a loop run (GS, weighted GS, GD): the checks the three entry points share -- their messages carry the
+// entry point's name `who` -- the run's state, the table, and the fields of the row and column arguments that do not
+// depend on the algorithm.  `given`: the entry point's own required pointers, which `required` names; `refused`: why
+// the entry point refuses one of its own arguments, or null.
+static int begin_loop(slm_ctx* c, int batch, const char* who, const char* loops_msg, bool given, const char* required,
+                      const char* table_msg, const char* refused, const uint8_t* T8, const void* Treal, const void* plane2, const double* lut,
+                      const double* norm, const void* inc_amp, int max_loops, double tolerance, double* hologram_out,
+                      RowArgs* ra, ColArgs* ca) {
+    const std::string w(who);
+    SLM_TRY(check_batch(c, batch, who));
+    if (max_loops < 1) return fail(SLM_ERR_ARG, w + ": " + loops_msg);
+    if (!given) return fail(SLM_ERR_ARG, w + ": " + required + " are required");
+    if (T8 ? !lut : !(Treal && plane2)) return fail(SLM_ERR_ARG, w + ": " + table_msg);
+    if (refused) return fail(SLM_ERR_ARG, w + ": " + refused);
     SLM_TRY(begin_run(c, batch, norm, max_loops));
-    if (T8) SLM_TRY(upload_lut(c, amp_lut));
+    if (T8) SLM_TRY(upload_lut(c, lut));
 
-    RowArgs ra{};
-    ra.B = batch; ra.H = c->H; ra.Y = c->Y; ra.X = c->X; ra.inc = inc_amp; ra.stats = c->stats;
-    ra.inv_hw = 1.0 / ((double)c->H * c->W); ra.hologram = hologram_out; ra.tw = c->tw_row;
+    memset(ra, 0, sizeof *ra);                                      // zero padding too: the loop's graph key is made of these bytes
+    ra->B = batch; ra->H = c->H; ra->Y = c->Y; ra->X = c->X; ra->inc = inc_amp; ra->stats = c->stats;
+    ra->inv_hw = 1.0 / ((double)c->H * c->W); ra->hologram = hologram_out; ra->tw = c->tw_row;
+    memset(ca, 0, sizeof *ca);
+    ca->B = batch; ca->W = c->W; ca->X = c->X; ca->Y = c->Y; ca->T8 = T8; ca->Treal = Treal; ca->plane2 = plane2;
+    ca->lut = c->lut; ca->norm = c->norm; ca->stats = c->stats; ca->partial = c->partial; ca->counter = c->counter;
+    ca->err_curve = c->err_curve; ca->max_loops = max_loops; ca->tolerance = tolerance;
+    ca->inv_hw = ra->inv_hw; ca->tw = c->tw_col;
+    return 0;
+}
+
+// Iterations 0 .. max_loops-2 (Fourier-plane step + SLM-plane pass), replayed under a key of `family` (the kernel family)
+// and every argument the loop's launches are made of; then the last iteration, which ends with the final pass.
+template <class F> static int run_loop(slm_ctx* c, int batch, const char* family, int alg, RowArgs& ra, const ColArgs& ca,
+                                       F fourier_step) {
+    ra.source = ROW_FROM_Y;
+    std::string key(family);
+    double* const hologram = ra.hologram;
+    ra.hologram = nullptr;                                          // (only the final pass -- outside the loop -- writes the hologram)
+    key.append(reinterpret_cast<const char*>(&ra), sizeof ra).append(reinterpret_cast<const char*>(&ca), sizeof ca);
+    key.append(reinterpret_cast<const char*>(&batch), sizeof batch);
+    ra.hologram = hologram;
+    SLM_TRY(replay_iterations(c, batch, ca.max_loops - 1, key, [&]() -> int {
+        SLM_TRY(fourier_step());
+        SLM_TIMED(K_ROW_PASS, c->row->row_pass(alg, ra, c->stream));
+        return 0;
+    }));
+    SLM_TRY(fourier_step());
+    ra.final_pass = 1;
+    SLM_TIMED(K_ROW_PASS, c->row->row_pass(alg, ra, c->stream));
+    return 0;
+}
+
+// GS and weighted GS after begin_loop.  Weighted GS runs the launches of GS's one-CTA-per-tile branch ("gs/plain") at
+// every batch size, with the GSW forms of the max pre-pass and of the column pass (col_pass_tile<ALG_GSW>).  The
+// persistent column kernels have no room for a weight tile (col_warp.cuh: three 64 KB tile buffers), so the context's
+// batch does not choose a kernel for it.
+static int gs_loop(slm_ctx* c, int batch, bool weighted, RowArgs& ra, ColArgs& ca, const uint8_t* T8, const void* amp_real,
+                   const void* phasor0, int setup_c64, double* expected_out) {
     if (phasor0) { ra.source = ROW_FROM_FIELD; ra.field = phasor0; }
     else {
         int src = 0;
@@ -629,35 +672,19 @@ extern "C" int slm_gs_run(slm_ctx* c, int batch, const uint8_t* T8, const void* 
     // differently, and a plane's result must not depend on how many planes share its batch (the tail of a movie).  One
     // kernel family per run also because the expected outcome below takes its maximum with the arithmetic that made
     // the transform.  SLM_GS_GROUPS=1 keeps the pipeline (tests compare contexts of different sizes bit for bit).
-    const bool groups = c->use_groups && ((long long)c->max_batch * (c->W / c->col->cols_per_cta) > c->persist_ctas || getenv("SLM_GS_GROUPS"));
-    // exact scale of iteration 0 so the one-pass error of later iterations is well conditioned
-    if (groups) SLM_TRY(run_stats(c, batch));
+    const bool groups = !weighted && c->use_groups &&
+                        ((long long)c->max_batch * (c->W / c->col->cols_per_cta) > c->persist_ctas || getenv("SLM_GS_GROUPS"));
+    // exact scale of iteration 0 so the one-pass error of later iterations is well conditioned (weighted: and P_0 for sigma_0)
+    if (weighted) SLM_TIMED(K_COL_STATS, c->col->col_pass(ALG_GSW_STATS, ca, c->stream));
+    else if (groups) SLM_TRY(run_stats(c, batch));
     else SLM_TIMED(K_COL_STATS, c->col->col_plain(stats_args(c, batch, OUT_STATS, nullptr), c->stream));
 
-    ColArgs ca{};
-    ca.B = batch; ca.W = c->W; ca.X = c->X; ca.Y = c->Y; ca.T8 = T8; ca.Treal = Treal; ca.plane2 = amp_real;
-    ca.lut = c->lut; ca.norm = c->norm; ca.stats = c->stats; ca.partial = c->partial; ca.counter = c->counter;
-    ca.err_curve = c->err_curve; ca.max_loops = max_loops; ca.tolerance = tolerance;
-    ca.inv_hw = ra.inv_hw; ca.tw = c->tw_col;
-    ra.source = ROW_FROM_Y;
-    auto fourier_step = [&]() -> int {
+    const int col_alg = weighted ? ALG_GSW : ALG_GS;
+    SLM_TRY(run_loop(c, batch, weighted ? "gsw/plain" : (groups ? "gs/pipeline" : "gs/plain"), ALG_GS, ra, ca, [&]() -> int {
         if (groups) SLM_TRY(launch_group(c, CGM_GS, batch, &ca, &c->map_y, 0, 1.0));
-        else SLM_TIMED(K_COL_PASS, c->col->col_pass(ALG_GS, ca, c->stream));
-        return 0;
-    };
-    std::string key(groups ? "gs/pipeline" : "gs/plain");           // the kernel family and every argument the loop's launches are made of
-    RowArgs ra_key = ra;
-    ra_key.hologram = nullptr;                                      // (only the final pass -- outside the loop -- writes the hologram)
-    key.append(reinterpret_cast<const char*>(&ra_key), sizeof ra_key).append(reinterpret_cast<const char*>(&ca), sizeof ca);
-    key.append(reinterpret_cast<const char*>(&batch), sizeof batch);
-    SLM_TRY(replay_iterations(c, batch, max_loops - 1, key, [&]() -> int {     // iterations 0 .. max_loops-2: Fourier-plane pass + SLM-plane pass
-        SLM_TRY(fourier_step());
-        SLM_TIMED(K_ROW_PASS, c->row->row_pass(ALG_GS, ra, c->stream));
+        else SLM_TIMED(K_COL_PASS, c->col->col_pass(col_alg, ca, c->stream));
         return 0;
     }));
-    SLM_TRY(fourier_step());                                        // the last iteration ends with the final pass below
-    ra.final_pass = 1;
-    SLM_TIMED(K_ROW_PASS, c->row->row_pass(ALG_GS, ra, c->stream));
     if (expected_out) {
         PlainColArgs ia = stats_args(c, batch, OUT_INTENSITY_GS, expected_out);
         if (groups) {
@@ -671,89 +698,48 @@ extern "C" int slm_gs_run(slm_ctx* c, int batch, const uint8_t* T8, const void* 
     return 0;
 }
 
-// Weighted GS: the launches of slm_gs_run's one-CTA-per-tile branch ("gs/plain") at every batch size, with the GSW
-// forms of the max pre-pass and of the column pass (col_pass_tile<ALG_GSW>).  The persistent column kernels have no
-// room for a weight tile (col_warp.cuh: three 64 KB tile buffers), so the context's batch does not choose a kernel here.
+extern "C" int slm_gs_run(slm_ctx* c, int batch, const uint8_t* T8, const void* Treal, const void* amp_real,
+                          const double* amp_lut, const double* norm, const void* inc_amp, const void* phasor0,
+                          int setup_c64, int max_loops, double tolerance, double* hologram_out, double* expected_out) {
+    RowArgs ra; ColArgs ca;
+    SLM_TRY(begin_loop(c, batch, "slm_gs_run", "max_loops must be >= 1 (the reference raises UnboundLocalError for 0)",
+                       norm && hologram_out, "norm and hologram_out", "give target_u8 + amp_lut, or target_real + amp_real",
+                       nullptr, T8, Treal, amp_real, amp_lut, norm, inc_amp, max_loops, tolerance, hologram_out, &ra, &ca));
+    return gs_loop(c, batch, false, ra, ca, T8, amp_real, phasor0, setup_c64, expected_out);
+}
+
 extern "C" int slm_gsw_run(slm_ctx* c, int batch, const uint8_t* T8, const void* Treal, const void* amp_real,
                            const double* amp_lut, const double* norm, const void* inc_amp, const void* phasor0,
                            int setup_c64, int max_loops, double tolerance, double* hologram_out, double* expected_out,
                            const double* target_sum, void* weights, double weight_limit) {
-    SLM_TRY(check_batch(c, batch, "slm_gsw_run"));
-    if (max_loops < 1) return fail(SLM_ERR_ARG, "slm_gsw_run: max_loops must be >= 1");
-    if (!norm || !hologram_out || !target_sum || !weights) return fail(SLM_ERR_ARG, "slm_gsw_run: norm, target_sum, weights and hologram_out are required");
-    if (T8 ? !amp_lut : !(Treal && amp_real)) return fail(SLM_ERR_ARG, "slm_gsw_run: give target_u8 + amp_lut, or target_real + amp_real");
-    if (!(weight_limit >= 1.0)) return fail(SLM_ERR_ARG, "slm_gsw_run: weight_limit must be >= 1");
+    RowArgs ra; ColArgs ca;
+    SLM_TRY(begin_loop(c, batch, "slm_gsw_run", "max_loops must be >= 1", norm && hologram_out && target_sum && weights,
+                       "norm, target_sum, weights and hologram_out", "give target_u8 + amp_lut, or target_real + amp_real",
+                       weight_limit >= 1.0 ? nullptr : "weight_limit must be >= 1",
+                       T8, Treal, amp_real, amp_lut, norm, inc_amp, max_loops, tolerance, hologram_out, &ra, &ca));
     if (!c->target_sum) {
         SLM_TRY(dev_alloc(c, (void**)&c->target_sum, (size_t)c->max_batch * sizeof(double)));
         SLM_TRY(dev_alloc(c, (void**)&c->signal_sum, (size_t)c->max_batch * sizeof(double)));
         SLM_TRY(dev_alloc(c, (void**)&c->signal_partial, (size_t)c->max_batch * c->tiles * sizeof(double)));
     }
-    SLM_TRY(begin_run(c, batch, norm, max_loops));
     SLM_CUDA(cudaMemcpyAsync(c->target_sum, target_sum, (size_t)batch * sizeof(double), cudaMemcpyHostToDevice, c->stream));
-    if (T8) SLM_TRY(upload_lut(c, amp_lut));
-
-    RowArgs ra{};
-    ra.B = batch; ra.H = c->H; ra.Y = c->Y; ra.X = c->X; ra.inc = inc_amp; ra.stats = c->stats;
-    ra.inv_hw = 1.0 / ((double)c->H * c->W); ra.hologram = hologram_out; ra.tw = c->tw_row;
-    if (phasor0) { ra.source = ROW_FROM_FIELD; ra.field = phasor0; }
-    else {
-        int src = 0;
-        SLM_TRY(setup_field(c, batch, T8, amp_real, setup_c64, &src));
-        ra.source = src; ra.A32 = c->Y; ra.field = c->Y;
-    }
-    SLM_TIMED(K_ROW_PASS, c->row->row_pass(ALG_GS, ra, c->stream));
-
-    ColArgs ca{};
-    ca.B = batch; ca.W = c->W; ca.X = c->X; ca.Y = c->Y; ca.T8 = T8; ca.Treal = Treal; ca.plane2 = amp_real;
-    ca.lut = c->lut; ca.norm = c->norm; ca.stats = c->stats; ca.partial = c->partial; ca.counter = c->counter;
-    ca.err_curve = c->err_curve; ca.max_loops = max_loops; ca.tolerance = tolerance;
-    ca.inv_hw = ra.inv_hw; ca.tw = c->tw_col;
     ca.weights = weights; ca.target_sum = c->target_sum; ca.signal_sum = c->signal_sum; ca.signal_partial = c->signal_partial;
     ca.weight_limit = weight_limit;
-    // exact scale of iteration 0 (as GS takes it) and P_0 for sigma_0
-    SLM_TIMED(K_COL_STATS, c->col->col_pass(ALG_GSW_STATS, ca, c->stream));
-    ra.source = ROW_FROM_Y;
-    std::string key("gsw/plain");                                   // every argument the loop's launches are made of
-    RowArgs ra_key = ra;
-    ra_key.hologram = nullptr;
-    key.append(reinterpret_cast<const char*>(&ra_key), sizeof ra_key).append(reinterpret_cast<const char*>(&ca), sizeof ca);
-    key.append(reinterpret_cast<const char*>(&batch), sizeof batch);
-    SLM_TRY(replay_iterations(c, batch, max_loops - 1, key, [&]() -> int {
-        SLM_TIMED(K_COL_PASS, c->col->col_pass(ALG_GSW, ca, c->stream));
-        SLM_TIMED(K_ROW_PASS, c->row->row_pass(ALG_GS, ra, c->stream));
-        return 0;
-    }));
-    SLM_TIMED(K_COL_PASS, c->col->col_pass(ALG_GSW, ca, c->stream));
-    ra.final_pass = 1;
-    SLM_TIMED(K_ROW_PASS, c->row->row_pass(ALG_GS, ra, c->stream));
-    if (expected_out) SLM_TIMED(K_COL_PLAIN, c->col->col_plain(stats_args(c, batch, OUT_INTENSITY_GS, expected_out), c->stream));
-    return 0;
+    return gs_loop(c, batch, true, ra, ca, T8, amp_real, phasor0, setup_c64, expected_out);
 }
 
 extern "C" int slm_gd_run(slm_ctx* c, int batch, const uint8_t* T8, const void* Treal, const void* mask_real,
                           const double* mask_lut, const double* norm, const void* inc_amp, void* x,
                           const double* lr_schedule, int max_loops, double tolerance, double* hologram_out,
                           double* expected_out) {
-    SLM_TRY(check_batch(c, batch, "slm_gd_run"));
-    if (max_loops < 1) return fail(SLM_ERR_ARG, "slm_gd_run: max_loops must be >= 1 (the reference raises UnboundLocalError for 0)");
-    if (!norm || !hologram_out || !x || !lr_schedule) return fail(SLM_ERR_ARG, "slm_gd_run: norm, x, lr_schedule and hologram_out are required");
-    if (T8 ? !mask_lut : !(Treal && mask_real)) return fail(SLM_ERR_ARG, "slm_gd_run: give target_u8 + mask_lut, or target_real + mask_real");
-    SLM_TRY(begin_run(c, batch, norm, max_loops));
+    RowArgs ra; ColArgs ca;
+    SLM_TRY(begin_loop(c, batch, "slm_gd_run", "max_loops must be >= 1 (the reference raises UnboundLocalError for 0)",
+                       norm && hologram_out && x && lr_schedule, "norm, x, lr_schedule and hologram_out",
+                       "give target_u8 + mask_lut, or target_real + mask_real", nullptr,
+                       T8, Treal, mask_real, mask_lut, norm, inc_amp, max_loops, tolerance, hologram_out, &ra, &ca));
     SLM_CUDA(cudaMemcpyAsync(c->lr, lr_schedule, (size_t)max_loops * sizeof(double), cudaMemcpyHostToDevice, c->stream));
-    if (T8) SLM_TRY(upload_lut(c, mask_lut));
-
-    RowArgs ra{};
-    ra.B = batch; ra.H = c->H; ra.Y = c->Y; ra.X = c->X; ra.x = x; ra.inc = inc_amp; ra.stats = c->stats; ra.lr = c->lr;
-    ra.inv_hw = 1.0 / ((double)c->H * c->W); ra.hologram = hologram_out; ra.tw = c->tw_row;
-    ra.source = ROW_FROM_FIELD;
+    ra.x = x; ra.lr = c->lr; ra.source = ROW_FROM_FIELD;
     SLM_TIMED(K_ROW_PASS, c->row->row_pass(ALG_GD, ra, c->stream));
-
-    ColArgs ca{};
-    ca.B = batch; ca.W = c->W; ca.X = c->X; ca.Y = c->Y; ca.T8 = T8; ca.Treal = Treal; ca.plane2 = mask_real;
-    ca.lut = c->lut; ca.norm = c->norm; ca.stats = c->stats; ca.partial = c->partial; ca.counter = c->counter;
-    ca.err_curve = c->err_curve; ca.max_loops = max_loops; ca.tolerance = tolerance;
-    ca.inv_hw = ra.inv_hw; ca.tw = c->tw_col;
-    ra.source = ROW_FROM_Y;
     // The fused pass saves a launch and a trip of the field through L2/HBM per iteration, but its CTAs wait for each
     // other once per plane and it leaves the SMs beyond a whole number of planes idle: measured faster for a few
     // planes (latency bound: 2.9 vs 3.3 ms per 100-iteration hologram), slower for a large batch (47.9 vs 46.4 ms).
@@ -767,7 +753,9 @@ extern "C" int slm_gd_run(slm_ctx* c, int batch, const uint8_t* T8, const void* 
         fused = form[0] == 'f' && c->fused_ctas;
         pipe = form[0] == 'p' && c->pipe_ok;
     }
-    auto fourier_step = [&]() -> int {
+    // two-pass form without the column groups: the max pass keeps the transformed field in X (below)
+    if (!c->use_groups) ca.skip_forward = 1;
+    SLM_TRY(run_loop(c, batch, fused ? "gdf" : (pipe ? "gdp" : "gd2"), ALG_GD, ra, ca, [&]() -> int {
         if (fused) {
             // one Fourier-plane pass: the tiles of a plane agree on amax(output_unnormed) (algorithms.py:86) between
             // their forward transforms and the gradient step
@@ -781,28 +769,14 @@ extern "C" int slm_gd_run(slm_ctx* c, int batch, const uint8_t* T8, const void* 
             SLM_TRY(launch_group(c, CGM_GD_POST, batch, &ca, &c->map_y, 0, 1.0));
         } else {
             // amax(output_unnormed), algorithms.py:86; the transformed field is kept in X so the gradient pass need not
-            // transform again
+            // transform again (ca.skip_forward)
             PlainColArgs sa = stats_args(c, batch, OUT_STATS, c->X);
             sa.keep = 1;
             SLM_TIMED(K_COL_STATS, c->col->col_plain(sa, c->stream));
-            ca.skip_forward = 1;
             SLM_TIMED(K_COL_PASS, c->col->col_pass(ALG_GD, ca, c->stream));
         }
         return 0;
-    };
-    std::string key(fused ? "gdf" : (pipe ? "gdp" : "gd2"));
-    RowArgs ra_key = ra;
-    ra_key.hologram = nullptr;                                      // (only the final pass -- outside the loop -- writes the hologram)
-    key.append(reinterpret_cast<const char*>(&ra_key), sizeof ra_key).append(reinterpret_cast<const char*>(&ca), sizeof ca);
-    key.append(reinterpret_cast<const char*>(&batch), sizeof batch);
-    SLM_TRY(replay_iterations(c, batch, max_loops - 1, key, [&]() -> int {     // iterations 0 .. max_loops-2: Fourier-plane step + SLM-plane pass
-        SLM_TRY(fourier_step());
-        SLM_TIMED(K_ROW_PASS, c->row->row_pass(ALG_GD, ra, c->stream));
-        return 0;
     }));
-    SLM_TRY(fourier_step());
-    ra.final_pass = 1;
-    SLM_TIMED(K_ROW_PASS, c->row->row_pass(ALG_GD, ra, c->stream));
     if (expected_out) {
         PlainColArgs ia = stats_args(c, batch, OUT_INTENSITY_GD, expected_out);
         // two-pass form: X already holds med_output; one-pass forms: transform X once more (same kernel arithmetic), kept

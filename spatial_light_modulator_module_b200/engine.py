@@ -8,6 +8,7 @@ without the built library raises.
 from __future__ import annotations
 
 import ctypes as C
+from collections import namedtuple
 from dataclasses import dataclass
 from typing import List, Optional
 
@@ -241,21 +242,34 @@ class Engine:
         return out
 
     # ---- Gerchberg-Saxton (algorithms.py:10-49) -------------------------------------------------------
-    def gs(self, targets, max_loops: int, tolerance: float = 0.0, inc_amp=None, phasor0=None,
-           want_expected: bool = True, norms=None) -> LoopResult:
+    # what _begin hands a run: the targets (fields of _targets), the illumination and the result buffers
+    _Begun = namedtuple("_Begun", "batch t8 treal amp norms c64 inc hologram expected")
+
+    def _begin(self, targets, max_loops, unbound, inc_amp, norms, want_expected):
+        """What gs, gsw and gd do first.  ``unbound``: the reference's variable that a run without iterations
+        leaves unbound."""
         if max_loops < 1:
-            raise UnboundLocalError("cannot access local variable 'expected_outcome' where it is not associated with a value")
+            raise UnboundLocalError(f"cannot access local variable '{unbound}' where it is not associated with a value")
         batch, t8, treal, amp, norms, c64 = self._targets(targets, norms)
-        amp_dev = self._mem_upload(amp.astype(self.real_dtype)) if amp is not None else None
         inc_dev = self._as_device(inc_amp, self.real_dtype, "inc_amp")
-        ph_dev = self._as_device(phasor0, self.complex_dtype, "phasor0")
         holo = self._mem_empty((batch,) + self.shape, np.float64)
         exp = self._mem_empty((batch,) + self.shape, np.float64) if want_expected else None
-        self._check(self._lib.slm_gs_run(
-            self._ctx, batch, self._mem_ptr(t8), self._mem_ptr(treal), self._mem_ptr(amp_dev),
-            self._dp(self._amp_lut), self._dp(norms), self._mem_ptr(inc_dev), self._mem_ptr(ph_dev), int(c64),
-            int(max_loops), float(tolerance), self._mem_ptr(holo), self._mem_ptr(exp)))
-        return self._collect(batch, max_loops, holo, exp)
+        return self._Begun(batch, t8, treal, amp, norms, c64, inc_dev, holo, exp)
+
+    def _gs_run(self, entry, b, phasor0, max_loops, tolerance, *gsw_args) -> LoopResult:
+        """slm_gs_run, or slm_gsw_run with its three further arguments ``gsw_args``, after :meth:`_begin` (``b``)."""
+        amp_dev = self._mem_upload(b.amp.astype(self.real_dtype)) if b.amp is not None else None
+        ph_dev = self._as_device(phasor0, self.complex_dtype, "phasor0")
+        self._check(entry(
+            self._ctx, b.batch, self._mem_ptr(b.t8), self._mem_ptr(b.treal), self._mem_ptr(amp_dev),
+            self._dp(self._amp_lut), self._dp(b.norms), self._mem_ptr(b.inc), self._mem_ptr(ph_dev), int(b.c64),
+            int(max_loops), float(tolerance), self._mem_ptr(b.hologram), self._mem_ptr(b.expected), *gsw_args))
+        return self._collect(b.batch, max_loops, b.hologram, b.expected)
+
+    def gs(self, targets, max_loops: int, tolerance: float = 0.0, inc_amp=None, phasor0=None,
+           want_expected: bool = True, norms=None) -> LoopResult:
+        begun = self._begin(targets, max_loops, "expected_outcome", inc_amp, norms, want_expected)
+        return self._gs_run(self._lib.slm_gs_run, begun, phasor0, max_loops, tolerance)
 
     def gsw(self, targets, max_loops: int, tolerance: float = 0.0, inc_amp=None, phasor0=None, weight_limit: float = 10.0,
             weights=None, want_expected: bool = True, norms=None):
@@ -264,66 +278,51 @@ class Engine:
         of the engine's real dtype is updated in place), None = ones.  ``weight_limit`` >= 1 bounds them to
         [1/weight_limit, weight_limit]; 1 gives GS's results bit for bit.  Scale, error curve, tolerance stop and
         expected outcome are GS's.  Returns (LoopResult, weights_device)."""
-        if max_loops < 1:
-            raise UnboundLocalError("cannot access local variable 'expected_outcome' where it is not associated with a value")
-        if not float(weight_limit) >= 1.0:
+        if max_loops >= 1 and not float(weight_limit) >= 1.0:        # (max_loops < 1 raises first, in _begin)
             raise ValueError(f"weight_limit must be >= 1, not {weight_limit!r}")
-        batch, t8, treal, amp, norms, c64 = self._targets(targets, norms)
-        if t8 is not None and self._mem_is_device(targets):
-            sums = self._mem_plane_sum(t8)
+        b = self._begin(targets, max_loops, "expected_outcome", inc_amp, norms, want_expected)
+        if b.t8 is not None and self._mem_is_device(targets):
+            sums = self._mem_plane_sum(b.t8)
         else:
-            sums = np.asarray(targets).reshape(batch, -1).sum(axis=1, dtype=np.float64)      # S_T, like the norms
+            sums = np.asarray(targets).reshape(b.batch, -1).sum(axis=1, dtype=np.float64)    # S_T, like the norms
         sums = np.ascontiguousarray(sums, dtype=np.float64)
-        shape = (batch,) + self.shape
+        shape = (b.batch,) + self.shape
         if weights is None:
             w = self._mem_empty(shape, self.real_dtype)
             self._mem_fill(w, 1.0)
         else:
             w = self._as_device(weights, self.real_dtype, "weights")
-            if tuple(w.shape) == self.shape and batch == 1:
+            if tuple(w.shape) == self.shape and b.batch == 1:
                 w = w[None]
             if tuple(w.shape) != shape:
                 raise ValueError(f"weights must have shape {shape}, not {tuple(w.shape)}")
-        amp_dev = self._mem_upload(amp.astype(self.real_dtype)) if amp is not None else None
-        inc_dev = self._as_device(inc_amp, self.real_dtype, "inc_amp")
-        ph_dev = self._as_device(phasor0, self.complex_dtype, "phasor0")
-        holo = self._mem_empty(shape, np.float64)
-        exp = self._mem_empty(shape, np.float64) if want_expected else None
-        self._check(self._lib.slm_gsw_run(
-            self._ctx, batch, self._mem_ptr(t8), self._mem_ptr(treal), self._mem_ptr(amp_dev),
-            self._dp(self._amp_lut), self._dp(norms), self._mem_ptr(inc_dev), self._mem_ptr(ph_dev), int(c64),
-            int(max_loops), float(tolerance), self._mem_ptr(holo), self._mem_ptr(exp),
-            self._dp(sums), self._mem_ptr(w), float(weight_limit)))
-        return self._collect(batch, max_loops, holo, exp), w
+        res = self._gs_run(self._lib.slm_gsw_run, b, phasor0, max_loops, tolerance,
+                           self._dp(sums), self._mem_ptr(w), float(weight_limit))
+        return res, w
 
     # ---- gradient descent (algorithms.py:60-112) --------------------------------------------------------
     def gd(self, targets, x0, lr_schedule, max_loops: int, tolerance: float = 0.0, white_attention=1,
            inc_amp=None, want_expected: bool = True, norms=None):
         """``x0``: complex initial guess [B,H,W] (host or device; a device tensor is updated in place).
         Returns (LoopResult, x_device)."""
-        if max_loops < 1:
-            raise UnboundLocalError("cannot access local variable 'output' where it is not associated with a value")
-        batch, t8, treal, _amp, norms, _ = self._targets(targets, norms)
-        if t8 is not None:
+        b = self._begin(targets, max_loops, "output", inc_amp, norms, want_expected)
+        if b.t8 is not None:
             mask_lut, mask_dev = hl.gd_mask_lut(white_attention), None
         else:
             mask_lut = np.zeros(256)
-            mask_dev = self._mem_upload(np.asarray(1 + white_attention * np.asarray(targets).reshape((batch,) + self.shape) / 255,
+            mask_dev = self._mem_upload(np.asarray(1 + white_attention * np.asarray(targets).reshape((b.batch,) + self.shape) / 255,
                                                    dtype=self.real_dtype))
         x = self._as_device(x0, self.complex_dtype, "x0")
         if len(x.shape) == 2:
             x = x[None]
-        inc_dev = self._as_device(inc_amp, self.real_dtype, "inc_amp")
         lr = np.ascontiguousarray(lr_schedule, dtype=np.float64)
         if lr.shape != (max_loops,):
             raise ValueError("lr_schedule must have max_loops entries")
-        holo = self._mem_empty((batch,) + self.shape, np.float64)
-        exp = self._mem_empty((batch,) + self.shape, np.float64) if want_expected else None
         self._check(self._lib.slm_gd_run(
-            self._ctx, batch, self._mem_ptr(t8), self._mem_ptr(treal), self._mem_ptr(mask_dev), self._dp(mask_lut),
-            self._dp(norms), self._mem_ptr(inc_dev), self._mem_ptr(x), self._dp(lr), int(max_loops), float(tolerance),
-            self._mem_ptr(holo), self._mem_ptr(exp)))
-        return self._collect(batch, max_loops, holo, exp), x
+            self._ctx, b.batch, self._mem_ptr(b.t8), self._mem_ptr(b.treal), self._mem_ptr(mask_dev), self._dp(mask_lut),
+            self._dp(b.norms), self._mem_ptr(b.inc), self._mem_ptr(x), self._dp(lr), int(max_loops), float(tolerance),
+            self._mem_ptr(b.hologram), self._mem_ptr(b.expected)))
+        return self._collect(b.batch, max_loops, b.hologram, b.expected), x
 
     def random_phasor_guess(self, u, divide_by=1.0):
         """exp(1j*2*pi*u)/divide_by on the device from a host-drawn uniform stream ``u`` [B,H,W] or [H,W]

@@ -62,6 +62,13 @@ class EmuEngine(Engine):
         a = np.asarray(dev)
         return a.reshape(a.shape[0], -1).max(axis=1).astype(np.float64)
 
+    def _mem_plane_sum(self, dev):
+        a = np.asarray(dev)
+        return a.reshape(a.shape[0], -1).sum(axis=1, dtype=np.float64)
+
+    def _mem_fill(self, buf, value):
+        np.asarray(buf).fill(value)
+
     def _mem_contiguous(self, dev):
         return np.ascontiguousarray(dev).view(HostBuf)
 

@@ -11,17 +11,8 @@ from tests import gsw_checks as gc
 from tests.emu.emu_engine import EmuEngine
 
 
-class Engine(EmuEngine):
-    def _mem_plane_sum(self, dev):
-        a = np.asarray(dev)
-        return a.reshape(a.shape[0], -1).sum(axis=1, dtype=np.float64)
-
-    def _mem_fill(self, buf, value):
-        np.asarray(buf).fill(value)
-
-
 def make_engine(shape, precision, max_batch):
-    return Engine(shape, precision, max_batch)
+    return EmuEngine(shape, precision, max_batch)
 
 
 SHAPES = [(128, 128), (192, 256)]
