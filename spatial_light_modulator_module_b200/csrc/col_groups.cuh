@@ -102,16 +102,58 @@ template <int TC, int H, int NT, int CHMAX = 16> SLM_DEV void copy_grey_tile(con
     }
 }
 
+// ---- closing the planes of a persistent kernel's pass (column-group and warp-per-column kernels) ----------------
+// The one-pass GD forms' extra step (col_warp.cuh): the plane's max from the tiles' running max, re-armed.
+SLM_DEV void close_fused_max(const ColArgs& a, int b, double norm);
+// One thread closes plane b from the total of its tiles' sums.  s0 / norm: the plane's scale and norm as the tiles used them.
+template <typename R, int H, int MODE> SLM_DEV void close_group_plane(const ColArgs& a, int b, const Partial& tot, double s0, double norm) {
+    close_plane<R, cgm_close(MODE)>(a.stats + b, tot, s0, norm, (double)H * (double)a.W, a.err_curve + (size_t)b * a.max_loops,
+                                    a.tolerance);
+    if constexpr (MODE == CGM_GD_FUSED || MODE == CGM_GD_PIPE) close_fused_max(a, b, norm);
+}
+// The publisher warp's end of a finished tile (all 32 lanes; q: the tile's reduced sums, lane 0's are stored): keep the
+// sums for the closing kernel behind the launch (defer_close), or publish them and, in the plane's last tile, close it.
+template <typename R, int H, int MODE>
+SLM_DEV void publish_tile(const ColGroupArgs& ga, int b, int tile, int tiles, int lane, const Partial& q, double s0, double norm) {
+    const ColArgs& a = ga.c;
+    Partial* plane_partials = a.partial + (size_t)b * tiles;
+    if (ga.defer_close) {
+        if (lane == 0) plane_partials[tile] = q;
+        return;
+    }
+    unsigned ticket = 0;
+    if (lane == 0) ticket = publish_partial(q, plane_partials, tile, tiles, a.counter + b);
+    Partial tot;
+    if (collect_if_last<close_fields(cgm_close(MODE))>(ticket, lane, plane_partials, tiles, tot) && lane == 0)
+        close_group_plane<R, H, MODE>(a, b, tot, s0, norm);
+}
+// The planes' closing as a kernel of its own (ColGroupArgs::defer_close): one warp per plane sums the tiles'
+// partial sums in the order collect_if_last uses, so both forms give the same bits.
+template <typename R, int H, int MODE>
+SLM_GLOBAL void SLM_LAUNCH_BOUNDS(32, 1) close_planes_kernel(ColGroupArgs ga, int tiles) {
+    constexpr int FIELDS = close_fields(cgm_close(MODE));
+    const ColArgs& a = ga.c;
+    const int b = blockIdx.x, lane = threadIdx.x;
+    griddep_wait();
+    PlaneStats* st = a.stats + b;
+    if (!ga.all_planes && ld_cg(&st->done) != 0) return;         // the pass skipped this plane
+    const Partial* plane_partials = a.partial + (size_t)b * tiles;
+    Partial q; q.mx = 0; q.a = 0; q.b = 0; q.c = 0;
+    for (int i = lane; i < tiles; i += 32) q = combine<FIELDS>(q, ld_partial(plane_partials + i));
+    const Partial tot = warp_reduce<FIELDS>(q);
+    if (lane == 0) close_group_plane<R, H, MODE>(a, b, tot, ld_cg(&st->scale), ld_ro(a.norm + b));
+}
+
 template <typename R, int H, int MODE>
 SLM_GLOBAL void SLM_LAUNCH_BOUNDS((ColGroupGeom<R, H>::THREADS), 1)
 col_group_kernel(ColGroupArgs ga, const SLM_GRID_CONSTANT TileMap tm_in, const SLM_GRID_CONSTANT TileMap tm_out) {
     using G = ColGroupGeom<R, H>;
     using P = ColPlan<H>;
     constexpr int E = G::E, M = G::M, TC = G::TC, ROWB = G::ROWB, CS = (int)sizeof(cpx<R>);
-    constexpr bool HAS_T = MODE == CGM_GS || MODE == CGM_GD || MODE == CGM_GD_POST;
+    constexpr bool HAS_T = cgm_has_target(MODE);
     constexpr bool HAS_OUT = MODE != CGM_STATS;
-    constexpr bool IS_GD = MODE == CGM_GD || MODE == CGM_GD_POST;
-    constexpr bool IS_STATS = MODE == CGM_STATS || MODE == CGM_STATS_KEEP;
+    constexpr bool IS_GD = cgm_is_gd(MODE);
+    constexpr bool IS_STATS = cgm_is_stats(MODE);
     const ColArgs& a = ga.c;
     SLM_DYN_SMEM(raw);
     unsigned char* const tile0 = raw;
@@ -154,53 +196,23 @@ col_group_kernel(ColGroupArgs ga, const SLM_GRID_CONSTANT TileMap tm_in, const S
     auto rests = [&](int b) { return MODE != CGM_COMPLEX && !ga.all_planes && ld_cg(&a.stats[b].done) != 0; };
 
     constexpr bool HAS_STATS = MODE != CGM_COMPLEX;
-    constexpr int FIELDS = MODE == CGM_GS ? F_ALL : (IS_GD ? F_A : F_MX);
+    constexpr int FIELDS = close_fields(cgm_close(MODE));
     if (t >= G::COMPUTE + G::COPIERS) {
         // ================= publisher warp =================
         if (!HAS_STATS) return;
         const int lane = t - G::COMPUTE - G::COPIERS;
-        const double hw = (double)H * (double)a.W;
         unsigned k = 0;
         for (long long g = blockIdx.x; g < total; g += gridDim.x) {
             const int b = (int)(g / tiles), tile = (int)(g % tiles);
             if (rests(b)) continue;
             const int s = (int)(k & 1u);
-            PlaneStats* st = a.stats + b;
             // values the closing formulas need, read before this launch can change them
-            const double s0 = ld_cg(&st->scale), norm = ld_ro(a.norm + b);
+            const double s0 = ld_cg(&a.stats[b].scale), norm = ld_ro(a.norm + b);
             mbar_wait(done + s, (k >> 1) & 1u);              // every compute thread is through tile k (totals are in shared memory)
             Partial q = tile_total[s];
             shfl_idx(0u, 0);                                 // all lanes hold their copy before the slot is released
             if (lane == 0) mbar_arrive(pubfree + s);
-            Partial* plane_partials = a.partial + (size_t)b * tiles;
-            if (ga.defer_close) {                            // the closing kernel behind this launch sums the tiles (col_warp.cuh)
-                if (lane == 0) plane_partials[tile] = q;
-                ++k;
-                continue;
-            }
-            unsigned ticket = 0;
-            if (lane == 0) ticket = publish_partial(q, plane_partials, tile, tiles, a.counter + b);
-            Partial tot;
-            if (collect_if_last<FIELDS>(ticket, lane, plane_partials, tiles, tot) && lane == 0) {
-                if (IS_STATS) {
-                    st->imax = tot.mx; st->scale = norm / tot.mx;
-                } else {
-                    double err;
-                    if (MODE == CGM_GS) {
-                        const double sN = norm / tot.mx;                 // algorithms.py:37
-                        const double s0u = (double)(R)s0;                // the scale the tiles actually used
-                        const double dl = (s0u != 0.0) ? sN / s0u - 1.0 : 0.0;
-                        err = (tot.a + 2.0 * dl * tot.b + dl * dl * tot.c) / hw;   // == sum((s*I - T)^2)/HW, :38,:162
-                        st->imax = tot.mx; st->scale = sN;
-                    } else {
-                        err = tot.a / hw;                                // algorithms.py:92
-                    }
-                    const int it = st->iters;
-                    a.err_curve[(size_t)b * a.max_loops + it] = err;
-                    st->err = err; st->iters = it + 1;
-                    st->done = !(err > a.tolerance);                     // loop condition, algorithms.py:29,83
-                }
-            }
+            publish_tile<R, H, MODE>(ga, b, tile, tiles, lane, q, s0, norm);
             ++k;
         }
         return;

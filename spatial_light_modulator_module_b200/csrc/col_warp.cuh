@@ -198,54 +198,13 @@ SLM_DEV void warp_fft_inverse(cpx<R>* v, unsigned char* buf, unsigned lm, unsign
     dft_side_a<RA, +1>(v);                                       // over n1' = r: y[lane + 32 k1'], k1' = idx(p)
 }
 
-// Close a plane's Fourier-plane pass from the total of its tiles' sums (one thread): max and scale, error,
-// iteration count, loop condition.  s0 / norm: the plane's scale and norm as the tiles used them.
-template <typename R, int H, int MODE>
-SLM_DEV void close_plane(const ColArgs& a, int b, const Partial& tot, double s0, double norm) {
-    constexpr bool IS_STATS = MODE == CGM_STATS || MODE == CGM_STATS_KEEP;
+// Declared in col_groups.cuh: when a one-pass GD form closes a plane, every tile of the plane has used the plane's max --
+// record it and re-arm the plane's words for the next pass.
+SLM_DEV void close_fused_max(const ColArgs& a, int b, double norm) {
     PlaneStats* st = a.stats + b;
-    const double hw = (double)H * (double)a.W;
-    if (IS_STATS) {
-        st->imax = tot.mx; st->scale = norm / tot.mx;
-        return;
-    }
-    double err;
-    if (MODE == CGM_GS) {
-        const double sN = norm / tot.mx;                 // algorithms.py:37
-        const double s0u = (double)(R)s0;                // the scale the tiles actually used
-        const double dl = (s0u != 0.0) ? sN / s0u - 1.0 : 0.0;
-        err = (tot.a + 2.0 * dl * tot.b + dl * dl * tot.c) / hw;   // == sum((s*I - T)^2)/HW, :38,:162
-        st->imax = tot.mx; st->scale = sN;
-    } else {
-        err = tot.a / hw;                                // algorithms.py:92
-        if (MODE == CGM_GD_FUSED || MODE == CGM_GD_PIPE) {   // every tile of the plane has used the max: record and re-arm
-            const double pm = (double)__uint_as_float(ld_cg(plane_max_word(a, b)));
-            st->imax = pm; st->scale = norm / pm;
-            *plane_max_word(a, b) = 0u; *plane_count_word(a, b) = 0u;
-        }
-    }
-    const int it = st->iters;
-    a.err_curve[(size_t)b * a.max_loops + it] = err;
-    st->err = err; st->iters = it + 1;
-    st->done = !(err > a.tolerance);                     // loop condition, algorithms.py:29,83
-}
-
-// The planes' closing as a kernel of its own (ColGroupArgs::defer_close): one warp per plane sums the tiles'
-// partial sums in the order collect_if_last uses, so both forms give the same bits.
-template <typename R, int H, int MODE>
-SLM_GLOBAL void SLM_LAUNCH_BOUNDS(32, 1) close_planes_kernel(ColGroupArgs ga, int tiles) {
-    constexpr bool IS_GD = MODE == CGM_GD || MODE == CGM_GD_POST || MODE == CGM_GD_FUSED || MODE == CGM_GD_PIPE;
-    constexpr int FIELDS = MODE == CGM_GS ? F_ALL : (IS_GD ? F_A : F_MX);
-    const ColArgs& a = ga.c;
-    const int b = blockIdx.x, lane = threadIdx.x;
-    griddep_wait();
-    PlaneStats* st = a.stats + b;
-    if (!ga.all_planes && ld_cg(&st->done) != 0) return;         // the pass skipped this plane
-    const Partial* plane_partials = a.partial + (size_t)b * tiles;
-    Partial q; q.mx = 0; q.a = 0; q.b = 0; q.c = 0;
-    for (int i = lane; i < tiles; i += 32) q = combine<FIELDS>(q, ld_partial(plane_partials + i));
-    const Partial tot = warp_reduce<FIELDS>(q);
-    if (lane == 0) close_plane<R, H, MODE>(a, b, tot, ld_cg(&st->scale), ld_ro(a.norm + b));
+    const double pm = (double)__uint_as_float(ld_cg(plane_max_word(a, b)));
+    st->imax = pm; st->scale = norm / pm;
+    *plane_max_word(a, b) = 0u; *plane_count_word(a, b) = 0u;
 }
 
 template <typename R, int H, int MODE>
@@ -256,12 +215,12 @@ col_warp_kernel(ColGroupArgs ga, const SLM_GRID_CONSTANT TileMap tm_in, const SL
     constexpr bool FUSED = MODE == CGM_GD_FUSED;
     constexpr bool PIPE = MODE == CGM_GD_PIPE;                      // group 0 transforms forward, group 1 does the rest of the tile
     constexpr int STOPS = PIPE ? 1 : G::GROUPS;                     // stop markers that end the kernel (PIPE: both groups see every item)
-    constexpr bool HAS_T = MODE == CGM_GS || MODE == CGM_GD || MODE == CGM_GD_POST || FUSED || PIPE;
+    constexpr bool HAS_T = cgm_has_target(MODE);
     constexpr bool HAS_OUT = MODE != CGM_STATS;
-    constexpr bool IS_GD = MODE == CGM_GD || MODE == CGM_GD_POST || FUSED || PIPE;
-    constexpr bool IS_STATS = MODE == CGM_STATS || MODE == CGM_STATS_KEEP;
+    constexpr bool IS_GD = cgm_is_gd(MODE);
+    constexpr bool IS_STATS = cgm_is_stats(MODE);
     constexpr bool HAS_STATS = MODE != CGM_COMPLEX;
-    constexpr int FIELDS = MODE == CGM_GS ? F_ALL : (IS_GD ? F_A : F_MX);
+    constexpr int FIELDS = close_fields(cgm_close(MODE));
     const ColArgs& a = ga.c;
     SLM_DYN_SMEM(raw);
     R* const lut_s = reinterpret_cast<R*>(raw + G::OFF_LUT);
@@ -305,7 +264,6 @@ col_warp_kernel(ColGroupArgs ga, const SLM_GRID_CONSTANT TileMap tm_in, const SL
         // ================= publisher warp =================
         if (!HAS_STATS) return;
         const int lane = t - G::COMPUTE - 96;
-        const double hw = (double)H * (double)a.W;
         if constexpr (PIPE) {
             // Two duties, polled in turn so neither holds the other up: (i) a tile that group 0 has transformed hands its
             // max |F|^2 to its plane (atomic max, then the plane's arrival count) -- kept off the compute warps' path: a
@@ -363,16 +321,7 @@ col_warp_kernel(ColGroupArgs ga, const SLM_GRID_CONSTANT TileMap tm_in, const SL
                     if (lane < TC) q = red[s * TC + lane];
                     q = warp_reduce<FIELDS>(q);
                     if (lane == 0) mbar_arrive(bar(taken, s));
-                    Partial* plane_partials = a.partial + (size_t)b * tiles;
-                    if (ga.defer_close) {
-                        if (lane == 0) plane_partials[tile] = q;
-                    } else {
-                        unsigned ticket = 0;
-                        if (lane == 0) ticket = publish_partial(q, plane_partials, tile, tiles, a.counter + b);
-                        Partial tot;
-                        if (collect_if_last<FIELDS>(ticket, lane, plane_partials, tiles, tot) && lane == 0)
-                            close_plane<R, H, MODE>(a, b, tot, d.scale, d.norm);
-                    }
+                    publish_tile<R, H, MODE>(ga, b, tile, tiles, lane, q, d.scale, d.norm);
                     ++kd;
                 }
                 if (!(ev & (EV_FWD | EV_DONE | EV_FSTOP))) spin_pause();
@@ -391,16 +340,7 @@ col_warp_kernel(ColGroupArgs ga, const SLM_GRID_CONSTANT TileMap tm_in, const SL
             if (lane < TC) q = red[s * TC + lane];
             q = warp_reduce<FIELDS>(q);                      // (also: every lane holds its copy before the slot is released)
             if (lane == 0) mbar_arrive(bar(taken, s));
-            Partial* plane_partials = a.partial + (size_t)b * tiles;
-            if (ga.defer_close) {                            // the closing kernel behind this launch sums the tiles
-                if (lane == 0) plane_partials[tile] = q;
-                continue;
-            }
-            unsigned ticket = 0;
-            if (lane == 0) ticket = publish_partial(q, plane_partials, tile, tiles, a.counter + b);
-            Partial tot;
-            if (collect_if_last<FIELDS>(ticket, lane, plane_partials, tiles, tot) && lane == 0)
-                close_plane<R, H, MODE>(a, b, tot, d.scale, d.norm);
+            publish_tile<R, H, MODE>(ga, b, tile, tiles, lane, q, d.scale, d.norm);
         }
         return;
     }

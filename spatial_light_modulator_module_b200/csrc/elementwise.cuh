@@ -290,7 +290,7 @@ SLM_GLOBAL void rows_reduce_kernel(const double* partial, int rows, double* out,
     }
 }
 // gathered[world][4] -> the plane's max and sums (rank order: the same bits on every rank); closes the iteration like
-// close_plane<GS>: state[0] = scale (in: the one the pass used, out: norm / max), state[1] = error, state[2] = iterations
+// close_plane<CLOSE_GS>: state[0] = scale (in: the one the pass used, out: norm / max), state[1] = error, state[2] = iterations
 // done (as a double), state[3] = loop-ended flag.  prepass: only the scale (exact scale of iteration 0).
 // form: 0 GS iteration; 1 only the scale and the max (GS iteration 0's exact scale; the max pass of every GD iteration,
 // algorithms.py:86); 2 GD iteration: error = sum (output - T)^2 / HW (algorithms.py:92), scale and max stay.  `stats`
@@ -307,8 +307,7 @@ SLM_GLOBAL void rows_close_kernel(const double* gathered, int world, double norm
     if (form == 0) {
         const double s = norm / mx;                               // algorithms.py:37
         const double s0u = as_float ? (double)(float)state[0] : state[0];      // the scale the kernel used
-        const double dl = s0u != 0.0 ? s / s0u - 1.0 : 0.0;
-        err = (a + 2.0 * dl * b + dl * dl * c) / hw;              // algorithms.py:38,162
+        err = gs_error(a, b, c, s, s0u, hw);
         state[0] = s; state[4] = mx;
     } else {
         err = a / hw;                                             // algorithms.py:92

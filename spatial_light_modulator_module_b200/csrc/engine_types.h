@@ -23,6 +23,9 @@ struct PlaneStats {
 // Per-tile reduction record (deterministic two-stage reduce: tile -> plane).
 struct Partial { double mx, a, b, c; };
 
+// What the last tile of a plane closes (close_plane, passes.cuh): the max and the scale only, or a GS / GD iteration.
+enum PlaneClose { CLOSE_MAX = 0, CLOSE_GS = 1, CLOSE_GD = 2 };
+
 // ---- SLM-plane (row) pass ----------------------------------------------------------------------
 enum RowSource {
     ROW_FROM_Y = 0,      // rows of Y hold the column-inverse-transformed field: finish the ifft2
@@ -81,18 +84,21 @@ struct ColArgs {
 // ---- warp-specialised persistent column kernel (col_groups.cuh) ---------------------------------------
 enum ColGroupMode {
     CGM_GS = 0,       // Fourier-plane step of GS      (== col_pass_kernel<GS>)
-    CGM_GD = 1,       // Fourier-plane step of GD      (== col_pass_kernel<GD>)
     CGM_STATS = 2,    // forward transform, max |C|^2  (== col_plain_kernel OUT_STATS)
     CGM_COMPLEX = 3,  // plain transform, complex out  (== col_plain_kernel OUT_COMPLEX)
     CGM_STATS_KEEP = 4,  // CGM_STATS that also writes the transformed field back (GD: F = fft2(b) kept in X)
-    CGM_GD_POST = 5,     // CGM_GD on an already transformed field: no forward transform
-    CGM_GD_FUSED = 6,    // CGM_GD that takes the plane's max ITSELF: every tile of a plane is in flight at once (grid = a
+    CGM_GD_POST = 5,     // Fourier-plane step of GD on an already transformed field (== col_pass_kernel<GD> with skip_forward)
+    CGM_GD_FUSED = 6,    // the GD step that takes the plane's max ITSELF: every tile of a plane is in flight at once (grid = a
                          // multiple of the tiles per plane, all CTAs resident), tiles meet at a per-plane counter between
                          // the forward transform and the pointwise step (warp-per-column kernel only)
     CGM_GD_PIPE = 7,     // CGM_GD_FUSED for any batch, on every SM: the CTA's two compute groups split the tile's work -- one
                          // forward-transforms tile after tile (and feeds the planes' maxima), the other takes each tile on once
                          // its plane's maximum is complete -- so nobody idles while a plane's tiles meet.  Cooperative launch.
 };
+SLM_HOSTDEV constexpr bool cgm_is_gd(int m) { return m == CGM_GD_POST || m == CGM_GD_FUSED || m == CGM_GD_PIPE; }
+SLM_HOSTDEV constexpr bool cgm_is_stats(int m) { return m == CGM_STATS || m == CGM_STATS_KEEP; }
+SLM_HOSTDEV constexpr bool cgm_has_target(int m) { return m == CGM_GS || cgm_is_gd(m); }      // reads the target and its table
+SLM_HOSTDEV constexpr int cgm_close(int m) { return m == CGM_GS ? CLOSE_GS : (cgm_is_gd(m) ? CLOSE_GD : CLOSE_MAX); }
 struct ColGroupArgs {
     int mode_inverse;        // CGM_COMPLEX: transform direction
     int all_planes;          // 1: also planes whose loop has ended (the transform kept for the final intensity pass)

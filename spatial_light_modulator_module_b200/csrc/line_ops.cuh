@@ -39,8 +39,10 @@ template <typename R, int L> struct ColWarpLaunch<R, L, true> {
         static const bool coop = !(getenv("SLM_PIPE_COOP") && getenv("SLM_PIPE_COOP")[0] == '0');
         if (MODE == CGM_GD_PIPE && coop) SLM_LAUNCH_COOP((col_warp_kernel<R, L, MODE>), grid, block, WG::SMEM, s, ga, in, out);
         else SLM_LAUNCH_PDL((col_warp_kernel<R, L, MODE>), grid, block, WG::SMEM, s, ga, in, out);
-        if (MODE != CGM_COMPLEX && ga.defer_close)
-            SLM_LAUNCH((close_planes_kernel<R, L, MODE>), dim3((unsigned)ga.c.B), dim3(32), 0, s, ga, ga.c.W / WG::TC);
+        if constexpr (MODE != CGM_COMPLEX && MODE != CGM_GD_FUSED) {          // (the fused form closes its planes itself)
+            if (ga.defer_close)
+                SLM_LAUNCH((close_planes_kernel<R, L, MODE>), dim3((unsigned)ga.c.B), dim3(32), 0, s, ga, ga.c.W / WG::TC);
+        }
     }
     static bool launch(int mode, const ColGroupArgs& ga, const TileMap& in, const TileMap& out, int ctas, cudaStream_t s) {
         if (!enabled()) return false;
@@ -53,7 +55,6 @@ template <typename R, int L> struct ColWarpLaunch<R, L, true> {
         run<CGM_STATS_KEEP>(mode, ga, in, out, grid, block, s);
         run<CGM_GD_POST>(mode, ga, in, out, grid, block, s);
         run<CGM_COMPLEX>(mode, ga, in, out, grid, block, s);
-        if (mode == CGM_GD) return false;                    // (unused by the engine: the column-group kernel keeps it)
         return true;
     }
 };
@@ -63,7 +64,6 @@ template <typename R, int L> struct GroupLaunch<R, L, true> {
     static void prepare() {
         ColWarpLaunch<R, L>::prepare();
         cudaFuncSetAttribute(col_group_kernel<R, L, CGM_GS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GG::SMEM);
-        cudaFuncSetAttribute(col_group_kernel<R, L, CGM_GD>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GG::SMEM);
         cudaFuncSetAttribute(col_group_kernel<R, L, CGM_STATS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GG::SMEM);
         cudaFuncSetAttribute(col_group_kernel<R, L, CGM_COMPLEX>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GG::SMEM);
         cudaFuncSetAttribute(col_group_kernel<R, L, CGM_STATS_KEEP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GG::SMEM);
@@ -73,8 +73,10 @@ template <typename R, int L> struct GroupLaunch<R, L, true> {
                                         cudaStream_t s) {
         if (mode != MODE) return;
         SLM_LAUNCH_PDL((col_group_kernel<R, L, MODE>), grid, block, GG::SMEM, s, ga, in, out);
-        if (MODE != CGM_COMPLEX && ga.defer_close)
-            SLM_LAUNCH((close_planes_kernel<R, L, MODE>), dim3((unsigned)ga.c.B), dim3(32), 0, s, ga, ga.c.W / GG::TC);
+        if constexpr (MODE != CGM_COMPLEX) {
+            if (ga.defer_close)
+                SLM_LAUNCH((close_planes_kernel<R, L, MODE>), dim3((unsigned)ga.c.B), dim3(32), 0, s, ga, ga.c.W / GG::TC);
+        }
     }
     static int launch(int mode, const ColGroupArgs& ga, const TileMap& in, const TileMap& out, int ctas, cudaStream_t s) {
         static_assert(!ColWarpGeom<R, L>::OK || (ColWarpGeom<R, L>::TC == GG::TC && ColWarpGeom<R, L>::ROWB == GG::ROWB),
@@ -84,7 +86,6 @@ template <typename R, int L> struct GroupLaunch<R, L, true> {
         const long long tiles = (long long)ga.c.B * (ga.c.W / GG::TC);
         const dim3 grid((unsigned)(tiles < ctas ? tiles : ctas)), block(GG::THREADS);
         run<CGM_GS>(mode, ga, in, out, grid, block, s);
-        run<CGM_GD>(mode, ga, in, out, grid, block, s);
         run<CGM_STATS>(mode, ga, in, out, grid, block, s);
         run<CGM_STATS_KEEP>(mode, ga, in, out, grid, block, s);
         run<CGM_GD_POST>(mode, ga, in, out, grid, block, s);

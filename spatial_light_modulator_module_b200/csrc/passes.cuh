@@ -124,27 +124,35 @@ SLM_DEV double collect_sum(int t, const double* plane_partials, int tiles) {
     for (int m = 16; m >= 1; m >>= 1) q += shfl_xor(q, m);
     return q;
 }
-// Publish this tile's partial; returns (to every thread) whether this CTA is the last of its plane,
-// in which case thread 0 of it receives the plane total in `total`.
-template <int NT, int FIELDS> SLM_DEV bool publish_and_collect(Partial mine, int t, Partial* plane_partials, int tile, int tiles,
-                                                               unsigned* counter, Partial& total) {
-    SLM_STATIC_SMEM int is_last;
-    if (t == 0) {
-        plane_partials[tile] = mine;
-        fence_device();
-        const unsigned ticket = atomic_inc_wrap(counter, (unsigned)tiles - 1);   // wraps to 0: reusable
-        is_last = (ticket == (unsigned)tiles - 1);
+
+// ---- closing a plane's Fourier-plane pass ---------------------------------------------------------------
+// The Partial fields the tiles reduce for a closing of kind KIND (PlaneClose)
+SLM_HOSTDEV constexpr int close_fields(int kind) { return kind == CLOSE_GS ? F_ALL : (kind == CLOSE_GD ? F_A : F_MX); }
+// GS error of an iteration from sums taken against the scale s0 of the previous one (a = sum d^2, b = sum d u,
+// c = sum u^2 with u = s0 I, d = u - T): with the exact scale s, sum((s I - T)^2) / HW (algorithms.py:38,162)
+SLM_DEV double gs_error(double a, double b, double c, double s, double s0, double hw) {
+    const double dl = (s0 != 0.0) ? s / s0 - 1.0 : 0.0;
+    return (a + 2.0 * dl * b + dl * dl * c) / hw;
+}
+// One thread closes plane `st` from the total of its tiles' sums: max and scale, and for an iteration the error, its
+// entry in the plane's error curve `err_row`, the iteration count and the loop condition.  s0 / norm: the plane's
+// scale and norm as read by the tiles, which computed in R.
+template <typename R, int KIND>
+SLM_DEV void close_plane(PlaneStats* st, const Partial& tot, double s0, double norm, double hw, double* err_row, double tolerance) {
+    double err = 0;
+    if constexpr (KIND == CLOSE_GD) {
+        err = tot.a / hw;                                        // algorithms.py:92
+    } else {
+        const double s = norm / tot.mx;                          // algorithms.py:37
+        if constexpr (KIND == CLOSE_GS) err = gs_error(tot.a, tot.b, tot.c, s, (double)(R)s0, hw);
+        st->imax = tot.mx; st->scale = s;
     }
-    sync_cta();
-    const bool last = is_last != 0;
-    if (!last) return false;
-    fence_device();
-    if (t < 32) {
-        Partial q; q.mx = 0; q.a = 0; q.b = 0; q.c = 0;
-        for (int i = t; i < tiles; i += 32) q = combine<FIELDS>(q, ld_partial(plane_partials + i));
-        total = warp_reduce<FIELDS>(q);
+    if constexpr (KIND != CLOSE_MAX) {
+        const int k = st->iters;
+        err_row[k] = err;
+        st->err = err; st->iters = k + 1;
+        st->done = !(err > tolerance);                           // loop condition, algorithms.py:29,83
     }
-    return true;
 }
 
 // ---- geometry --------------------------------------------------------------------------------------
@@ -342,7 +350,7 @@ SLM_DEV void col_pass_tile(const ColArgs& a, int b, int tile, int tiles, cpx<R>*
         const R m2 = cnorm2(v[r]);                              // |C|^2, algorithms.py:36 / :85
         if (ALG == ALG_GS || GSW) {
             // error of this iteration against the scale s0 of the previous one; the exact scale
-            // s = norm/max is folded in by the last tile (see finish below).
+            // s = norm/max is folded in by the last tile (gs_error).
             const R u = s0r * m2, d = u - tv[r];
             mx = fmax(mx, m2); sa += d * d; sb += d * u; sc += u * u;
             R amp = aux[r];
@@ -369,7 +377,7 @@ SLM_DEV void col_pass_tile(const ColArgs& a, int b, int tile, int tiles, cpx<R>*
             v[r] = cscale(cscale(v[r], aux[r]), d);              // mask * med_output * (output - T), :88
         }
     }
-    constexpr int FIELDS = ALG == ALG_GD ? F_A : F_ALL;
+    constexpr int KIND = ALG == ALG_GD ? CLOSE_GD : CLOSE_GS, FIELDS = close_fields(KIND);
     Partial p; p.mx = (double)mx; p.a = (double)sa; p.b = (double)sb; p.c = (double)sc;
     p = block_reduce<G::THREADS, FIELDS, GSW ? 1 : 0>(p, t);
     double* sig_partials = GSW ? a.signal_partial + (size_t)b * tiles : nullptr;
@@ -394,23 +402,7 @@ SLM_DEV void col_pass_tile(const ColArgs& a, int b, int tile, int tiles, cpx<R>*
         const double psum = collect_sum(t, sig_partials, tiles);
         if (t == 0) a.signal_sum[b] = psum;
     }
-    if (t == 0) {
-        const double hw = (double)H * (double)W;
-        double err;
-        if (ALG != ALG_GD) {
-            const double s = norm / tot.mx;                      // algorithms.py:37
-            const double s0u = (double)s0r;                      // the scale the tiles actually used
-            const double dl = (s0u != 0.0) ? s / s0u - 1.0 : 0.0;
-            err = (tot.a + 2.0 * dl * tot.b + dl * dl * tot.c) / hw;   // == sum((s*I - T)^2)/HW, :38,:162
-            st->imax = tot.mx; st->scale = s;
-        } else {
-            err = tot.a / hw;                                    // algorithms.py:92
-        }
-        const int k = st->iters;
-        a.err_curve[(size_t)b * a.max_loops + k] = err;
-        st->err = err; st->iters = k + 1;
-        st->done = !(err > a.tolerance);                         // loop condition, algorithms.py:29,83
-    }
+    if (t == 0) close_plane<R, KIND>(st, tot, s0, norm, (double)H * (double)W, a.err_curve + (size_t)b * a.max_loops, a.tolerance);
 }
 
 // One column tile of a plain transform: complex out, max-only, or normalised intensity out.
@@ -444,14 +436,15 @@ SLM_DEV void col_plain_tile(const PlainColArgs& a, int b, int tile, int tiles, c
 #pragma unroll
         for (int r = 0; r < E; ++r) mx = fmax(mx, cnorm2(v[r]));
         p.mx = (double)mx;
-        p = block_reduce<G::THREADS, F_MX>(p, t);
+        constexpr int FIELDS = close_fields(CLOSE_MAX);
+        p = block_reduce<G::THREADS, FIELDS>(p, t);
         if (t >= 32) return;
         Partial* plane_partials = a.partial + (size_t)b * tiles;
         unsigned ticket = 0;
         if (t == 0) ticket = publish_partial(p, plane_partials, tile, tiles, a.counter + b);
         Partial tot;
-        if (!collect_if_last<F_MX>(ticket, t, plane_partials, tiles, tot)) return;
-        if (t == 0) { st->imax = tot.mx; st->scale = ld_ro(a.norm + b) / tot.mx; }
+        if (!collect_if_last<FIELDS>(ticket, t, plane_partials, tiles, tot)) return;
+        if (t == 0) close_plane<R, CLOSE_MAX>(st, tot, 0.0, ld_ro(a.norm + b), 0.0, nullptr, 0.0);
     } else {
         double* out = static_cast<double*>(a.out) + off;
         const double imax = ld_cg(&st->imax), scale = ld_cg(&st->scale), norm = ld_ro(a.norm + b);
@@ -532,8 +525,9 @@ SLM_GLOBAL void SLM_LAUNCH_BOUNDS((ColGeom<R, H>::THREADS), 1) col_gsw_stats_ker
                 mx = fmax(mx, m2);
                 if (sig[r]) sp += m2;
             }
+            constexpr int FIELDS = close_fields(CLOSE_MAX);
             Partial p; p.mx = (double)mx; p.a = 0; p.b = 0; p.c = 0;
-            p = block_reduce<G::THREADS, F_MX, 1>(p, t);
+            p = block_reduce<G::THREADS, FIELDS, 1>(p, t);
             Partial q; q.mx = 0; q.a = 0; q.b = (double)sp; q.c = 0;
             q = block_reduce<G::THREADS, F_B, 1>(q, t);
             if (t >= 32) return;
@@ -545,11 +539,10 @@ SLM_GLOBAL void SLM_LAUNCH_BOUNDS((ColGeom<R, H>::THREADS), 1) col_gsw_stats_ker
                 ticket = publish_partial(p, plane_partials, tile, tiles, a.counter + b);
             }
             Partial tot;
-            if (!collect_if_last<F_MX>(ticket, t, plane_partials, tiles, tot)) return;
+            if (!collect_if_last<FIELDS>(ticket, t, plane_partials, tiles, tot)) return;
             const double psum = collect_sum(t, sig_partials, tiles);
             if (t == 0) {
-                PlaneStats* st = a.stats + b;
-                st->imax = tot.mx; st->scale = ld_ro(a.norm + b) / tot.mx;
+                close_plane<R, CLOSE_MAX>(a.stats + b, tot, 0.0, ld_ro(a.norm + b), 0.0, nullptr, 0.0);
                 a.signal_sum[b] = psum;
             }
         });

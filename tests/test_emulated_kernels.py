@@ -78,6 +78,37 @@ def test_warp_column_kernel_gd_pipelined_one_pass_form(monkeypatch, rows, batch)
         np.testing.assert_array_equal(out["pipe"][i], out["two_pass"][i])
 
 
+@pytest.mark.parametrize("shape,precision,gd_form", [((1024, 64), "fp32", "two_pass"), ((1024, 64), "fp32", "pipe"),
+                                                     ((128, 128), "fp64", None)])
+def test_deferred_and_in_kernel_closing_agree(monkeypatch, shape, precision, gd_form):
+    """When a batch has more tiles than 4 per CTA, the planes are closed by a kernel behind the column pass;
+    SLM_NO_DEFER_CLOSE=1 has the publisher warp of the pass close them.  Same bits for GS and GD from both persistent
+    column kernels: the warp-per-column kernel (fp32 1024 rows; GD in two passes or pipelined) and the column-group
+    kernel (fp64 128 rows)."""
+    import numpy as np
+    from spatial_light_modulator_module_b200 import host_logic as hl, synthetic
+    if gd_form:
+        monkeypatch.setenv("SLM_GD_FORM", gd_form)
+    batch, loops = 2, 3
+    t = np.stack([synthetic.noise_target(shape, seed=i) for i in range(batch)])
+    x0 = np.stack([hl.host_initial_guess("random", shape, 42 + i) for i in range(batch)])
+    during, _ = hl.learning_rate_schedule(0.005, 0, loops)
+    out = {}
+    for name in ("deferred", "in_kernel"):
+        if name == "in_kernel":
+            monkeypatch.setenv("SLM_NO_DEFER_CLOSE", "1")
+        eng = make_engine(shape, precision, batch)
+        n0 = eng.launch_count()
+        g = eng.gs(t, loops)
+        r, _ = eng.gd(t, x0.copy(), during, loops)
+        out[name] = ([np.array(g.errors), eng.to_host(g.hologram), eng.to_host(g.expected),
+                      np.array(r.errors), eng.to_host(r.hologram), eng.to_host(r.expected)], eng.launch_count() - n0)
+        eng.close()
+    assert out["deferred"][1] > out["in_kernel"][1]                # the closing kernels ran
+    for a, b in zip(out["deferred"][0], out["in_kernel"][0]):
+        np.testing.assert_array_equal(a, b)
+
+
 def test_warp_column_kernel_gd_pipelined_tolerance(monkeypatch):
     monkeypatch.setenv("SLM_GD_FORM", "pipe")
     pc.check_gd_tolerance_and_batch(make_engine, "fp32", shape=(768, 64), loops=6)
