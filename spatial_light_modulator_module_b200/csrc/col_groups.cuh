@@ -334,17 +334,11 @@ col_group_kernel(ColGroupArgs ga, const SLM_GRID_CONSTANT TileMap tm_in, const S
 #pragma unroll
             for (int r = 0; r < E; ++r) {
                 const R m2 = cnorm2(v[r]);
-                if (MODE == CGM_GS) {                                 // algorithms.py:33,36-38 (see col_pass_tile)
-                    const R u = s0r * m2, d = u - tv[r];
-                    mx = fmax(mx, m2); sa += d * d; sb += d * u; sc += u * u;
-                    v[r] = (m2 == (R)0) ? mk<R>(copysign(aux[r], v[r].x), (R)0) : cscale(v[r], aux[r] * rsqrt_fast(m2));
-                } else {                                              // algorithms.py:85-88,92
-                    R I;
-                    if (sizeof(R) == 8) I = (R)(((double)m2 * norm) / imax);
-                    else I = m2 * gdk;
-                    const R d = I - tv[r];
-                    sa += d * d;
-                    v[r] = cscale(cscale(v[r], aux[r]), d);
+                if (MODE == CGM_GS) {
+                    gs_sums(m2, tv[r], s0r, mx, sa, sb, sc);
+                    replace_amplitude(v[r], m2, aux[r]);
+                } else {
+                    v[r] = gd_point(v[r], gd_output(m2, gdk, norm, imax), tv[r], aux[r], sa);
                 }
             }
         } else if (IS_STATS) {

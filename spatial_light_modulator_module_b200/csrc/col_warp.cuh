@@ -207,6 +207,58 @@ SLM_DEV void close_fused_max(const ColArgs& a, int b, double norm) {
     *plane_max_word(a, b) = 0u; *plane_count_word(a, b) = 0u;
 }
 
+// The one-pass GD forms' share of a plane's max |F|^2 (algorithms.py:86).  A column's max on side B, in every lane.
+template <typename R> SLM_DEV R side_b_max(const cpx<R>* v, bool active) {
+    R m = 0;
+#pragma unroll
+    for (int r = 0; r < 32; ++r) m = fmax(m, cnorm2(v[r]));
+    if (!active) m = 0;                                          // lanes outside side B hold no points
+#pragma unroll
+    for (int sh = 16; sh >= 1; sh >>= 1) m = fmax(m, shfl_xor(m, sh));
+    return m;
+}
+// A tile's column maxima fmx[0..TC) -> its plane's max word, then its arrival count.
+template <int TC> SLM_DEV void add_tile_max(const ColArgs& a, int b, const float* fmx) {
+    float mm = fmx[0];
+#pragma unroll
+    for (int i = 1; i < TC; ++i) mm = fmax(mm, fmx[i]);
+    atomic_max_u32(plane_max_word(a, b), __float_as_uint(mm));  // |F|^2 >= 0: ordered like its bit pattern
+    fence_device();
+    atomic_add_u32(plane_count_word(a, b), 1u);
+}
+
+// One lane waits until every tile of plane b has contributed; -> the bits of the plane's max.  Should the other tiles not
+// come (the CTAs of the launch not all resident: a foreign kernel holding SMs for good), it gives up after ~2 s with the
+// time-out flag set instead of hanging the device.  PAUSE: back off between polls (the pipelined form's waiting lane).
+template <bool PAUSE> SLM_DEV unsigned wait_plane_max(const ColArgs& a, int b, int tiles) {
+    const long long t0 = clock_now();
+    unsigned max_bits;
+    while (!plane_complete(a, b, tiles, max_bits)) {
+        if (PAUSE) spin_pause();
+        if (clock_now() - t0 > (1ll << 32)) { atomic_max_u32(plane_timeout_flag(a), 1u); break; }
+    }
+    return max_bits;
+}
+
+// The targets of side-B rows lane + RA (r0 + i), i < 8, of a column: grey level and table entry from the tile's grey rows
+// (gsrc: the lane's first), or T and the second plane from global memory at goff (zero in lanes outside side B).
+template <int RA, int TC, typename R>
+SLM_DEV void side_b_targets(const ColArgs& a, bool use_t8, bool active, const uint8_t* gsrc, const R* lut_s, size_t goff, int r0,
+                            R* tv, R* aux) {
+    if (use_t8) {
+#pragma unroll
+        for (int i = 0; i < 8; ++i) { const int gl = gsrc[(size_t)(r0 + i) * RA * TC]; tv[i] = (R)gl; aux[i] = lut_s[gl]; }
+    } else {
+        const R* T = static_cast<const R*>(a.Treal) + goff;
+        const R* Q = static_cast<const R*>(a.plane2) + goff;
+#pragma unroll
+        for (int i = 0; i < 8; ++i) {
+            tv[i] = active ? ld_ro(T + (size_t)(r0 + i) * RA * a.W) : (R)0;
+            aux[i] = active ? ld_ro(Q + (size_t)(r0 + i) * RA * a.W) : (R)0;
+        }
+    }
+}
+
 template <typename R, int H, int MODE>
 SLM_GLOBAL void SLM_LAUNCH_BOUNDS((ColWarpGeom<R, H>::THREADS), 1)
 col_warp_kernel(ColGroupArgs ga, const SLM_GRID_CONSTANT TileMap tm_in, const SLM_GRID_CONSTANT TileMap tm_out) {
@@ -301,15 +353,7 @@ col_warp_kernel(ColGroupArgs ga, const SLM_GRID_CONSTANT TileMap tm_in, const SL
                 if (ev & EV_FSTOP) fend = true;
                 if (ev & EV_FWD) {
                     const int s = (int)(kf % NBUF);
-                    if (lane == 0) {
-                        const int b = (int)(desc[s].g / tiles);
-                        float mm = fmx[s * (TC + 2)];
-#pragma unroll
-                        for (int i = 1; i < TC; ++i) mm = fmax(mm, fmx[s * (TC + 2) + i]);
-                        atomic_max_u32(plane_max_word(a, b), __float_as_uint(mm));  // |F|^2 >= 0: ordered like its bit pattern
-                        fence_device();
-                        atomic_add_u32(plane_count_word(a, b), 1u);
-                    }
+                    if (lane == 0) add_tile_max<TC>(a, (int)(desc[s].g / tiles), fmx + s * (TC + 2));
                     ++kf;
                 }
                 if (ev & EV_DSTOP) break;
@@ -498,12 +542,7 @@ col_warp_kernel(ColGroupArgs ga, const SLM_GRID_CONSTANT TileMap tm_in, const SL
                 sync_named(pair_bar, 64);                    // the partner holds its column too: the pair's chunk is free
                 warp_fft_forward<RA>(v, buf, lm, sm, w1);
                 SLM_STAMP(t == 0, k, 2);
-                R m = 0;
-#pragma unroll
-                for (int r = 0; r < 32; ++r) m = fmax(m, cnorm2(v[r]));
-                if (!active) m = 0;
-#pragma unroll
-                for (int sh = 16; sh >= 1; sh >>= 1) m = fmax(m, shfl_xor(m, sh));
+                const R m = side_b_max(v, active);
                 if (lane == 0) fmx[s * (TC + 2) + c] = m;
                 sync_named(pair_bar, 64);                    // the partner is through its exchange: its rows of my column are free
                 if (active) {
@@ -528,48 +567,25 @@ col_warp_kernel(ColGroupArgs ga, const SLM_GRID_CONSTANT TileMap tm_in, const SL
             SLM_STAMP(t == G::GROUP_THREADS, k, 5);
 #pragma unroll
             for (int q = 0; q < 32; ++q) v[q] = *reinterpret_cast<const cpx<R>*>(buf + my + 64u * RA * q);
-            if (c == 0 && lane == 0) {
-                // the plane's other tiles: counted already, or being transformed on other SMs right now (cooperative
-                // launch: every CTA is resident).  The time-out only guards against a broken launch.
-                const long long t0 = clock_now();
-                unsigned max_bits;
-                while (!plane_complete(a, b, tiles, max_bits)) {
-                    spin_pause();
-                    if (clock_now() - t0 > (1ll << 32)) { atomic_max_u32(plane_timeout_flag(a), 1u); break; }
-                }
-                fmx[s * (TC + 2) + TC] = __uint_as_float(max_bits);
-            }
+            // the plane's other tiles: counted already, or being transformed on other SMs right now (cooperative launch:
+            // every CTA is resident).  The time-out only guards against a broken launch.
+            if (c == 0 && lane == 0) fmx[s * (TC + 2) + TC] = __uint_as_float(wait_plane_max<true>(a, b, tiles));
             sync_named(10, G::GROUP_THREADS);
             SLM_STAMP(t == G::GROUP_THREADS, k, 6);
-            const R gdk = (R)(d.norm / (double)fmx[s * (TC + 2) + TC]);
+            const double pmax = (double)fmx[s * (TC + 2) + TC];
+            const R gdk = (R)(d.norm / pmax);
             sync_named(pair_bar, 64);                        // the partner holds its column too: the pair's chunk is free
             R sa = 0;
-            {
-                const uint8_t* gsrc = grey_buf(s) + (size_t)lane * TC + c;
-                const size_t goff = (size_t)b * H * a.W + (size_t)lane * a.W + tile * TC + c;
+            const uint8_t* gsrc = grey_buf(s) + (size_t)lane * TC + c;
+            const size_t goff = (size_t)b * H * a.W + (size_t)lane * a.W + tile * TC + c;
 #pragma unroll
-                for (int r0 = 0; r0 < 32; r0 += 8) {
-                    R tv[8], aux[8];
-                    if (use_t8) {
+            for (int r0 = 0; r0 < 32; r0 += 8) {
+                R tv[8], aux[8];
+                side_b_targets<RA, TC>(a, use_t8, active, gsrc, lut_s, goff, r0, tv, aux);
 #pragma unroll
-                        for (int i = 0; i < 8; ++i) { const int gl = gsrc[(size_t)(r0 + i) * RA * TC]; tv[i] = (R)gl; aux[i] = lut_s[gl]; }
-                    } else {
-                        const R* T = static_cast<const R*>(a.Treal) + goff;
-                        const R* Q = static_cast<const R*>(a.plane2) + goff;
-#pragma unroll
-                        for (int i = 0; i < 8; ++i) {
-                            tv[i] = active ? ld_ro(T + (size_t)(r0 + i) * RA * a.W) : (R)0;
-                            aux[i] = active ? ld_ro(Q + (size_t)(r0 + i) * RA * a.W) : (R)0;
-                        }
-                    }
-#pragma unroll
-                    for (int i = 0; i < 8; ++i) {            // algorithms.py:85-88,92
-                        const int r = r0 + i;
-                        const R I = cnorm2(v[r]) * gdk;
-                        const R dd = I - tv[i];
-                        sa += dd * dd;
-                        v[r] = cscale(cscale(v[r], aux[i]), dd);
-                    }
+                for (int i = 0; i < 8; ++i) {
+                    const int r = r0 + i;
+                    v[r] = gd_point(v[r], gd_output(cnorm2(v[r]), gdk, d.norm, pmax), tv[i], aux[i], sa);
                 }
             }
             if (!active) sa = 0;                             // lanes outside side B hold no points
@@ -610,31 +626,13 @@ col_warp_kernel(ColGroupArgs ga, const SLM_GRID_CONSTANT TileMap tm_in, const SL
         // ---- CGM_GD_FUSED: max |F|^2 of the whole plane (algorithms.py:86), across the CTAs holding its tiles ----
         double plane_max = d.imax;
         if (FUSED) {
-            R m = 0;
-#pragma unroll
-            for (int r = 0; r < 32; ++r) m = fmax(m, cnorm2(v[r]));
-            if (!active) m = 0;
-#pragma unroll
-            for (int sh = 16; sh >= 1; sh >>= 1) m = fmax(m, shfl_xor(m, sh));
+            const R m = side_b_max(v, active);
             float* const fmx = reinterpret_cast<float*>(raw + G::OFF_FMX) + s * (TC + 2);
             if (lane == 0) fmx[c] = m;
             sync_named(9 + grp, G::GROUP_THREADS);
             if (c == 0 && lane == 0) {
-                float mm = fmx[0];
-#pragma unroll
-                for (int i = 1; i < TC; ++i) mm = fmax(mm, fmx[i]);
-                atomic_max_u32(plane_max_word(a, b), __float_as_uint(mm));  // |F|^2 >= 0: ordered like its bit pattern
-                fence_device();
-                atomic_add_u32(plane_count_word(a, b), 1u);
-                // the plane's other tiles are in flight on other SMs; should they not be (the CTAs of this launch not all
-                // resident: a foreign kernel holding SMs for good), give up after ~2 s with the error flag set instead of
-                // hanging the device
-                const long long t0 = clock_now();
-                unsigned max_bits;
-                while (!plane_complete(a, b, tiles, max_bits)) {
-                    if (clock_now() - t0 > (1ll << 32)) { atomic_max_u32(plane_timeout_flag(a), 1u); break; }
-                }
-                fmx[TC] = __uint_as_float(max_bits);
+                add_tile_max<TC>(a, b, fmx);
+                fmx[TC] = __uint_as_float(wait_plane_max<false>(a, b, tiles));   // the plane's other tiles are in flight on other SMs
             }
             sync_named(9 + grp, G::GROUP_THREADS);
             plane_max = (double)fmx[TC];
@@ -651,31 +649,16 @@ col_warp_kernel(ColGroupArgs ga, const SLM_GRID_CONSTANT TileMap tm_in, const SL
 #pragma unroll
             for (int r0 = 0; r0 < 32; r0 += 8) {
                 R tv[8], aux[8];
-                if (use_t8) {
-#pragma unroll
-                    for (int i = 0; i < 8; ++i) { const int gl = gsrc[(size_t)(r0 + i) * RA * TC]; tv[i] = (R)gl; aux[i] = lut_s[gl]; }
-                } else {
-                    const R* T = static_cast<const R*>(a.Treal) + goff;
-                    const R* Q = static_cast<const R*>(a.plane2) + goff;
-#pragma unroll
-                    for (int i = 0; i < 8; ++i) {
-                        tv[i] = active ? ld_ro(T + (size_t)(r0 + i) * RA * a.W) : (R)0;
-                        aux[i] = active ? ld_ro(Q + (size_t)(r0 + i) * RA * a.W) : (R)0;
-                    }
-                }
+                side_b_targets<RA, TC>(a, use_t8, active, gsrc, lut_s, goff, r0, tv, aux);
 #pragma unroll
                 for (int i = 0; i < 8; ++i) {
                     const int r = r0 + i;
                     const R m2 = cnorm2(v[r]);
-                    if (MODE == CGM_GS) {                                 // algorithms.py:33,36-38
-                        const R u = s0r * m2, dd = u - tv[i];
-                        mx = fmax(mx, m2); sa += dd * dd; sb += dd * u; sc += u * u;
-                        v[r] = (m2 == (R)0) ? mk<R>(copysign(aux[i], v[r].x), (R)0) : cscale(v[r], aux[i] * rsqrt_fast(m2));
-                    } else {                                              // algorithms.py:85-88,92
-                        const R I = m2 * gdk;
-                        const R dd = I - tv[i];
-                        sa += dd * dd;
-                        v[r] = cscale(cscale(v[r], aux[i]), dd);
+                    if (MODE == CGM_GS) {
+                        gs_sums(m2, tv[i], s0r, mx, sa, sb, sc);
+                        replace_amplitude(v[r], m2, aux[i]);
+                    } else {
+                        v[r] = gd_point(v[r], gd_output(m2, gdk, d.norm, plane_max), tv[i], aux[i], sa);
                     }
                 }
             }

@@ -56,6 +56,32 @@ template <typename R> SLM_DEV cpx<R> tangent_step(cpx<R> x, cpx<R> g, R lr) {
     return pk_fma(mk<R>(step, step), tang, x);                     // x - lr * tang / |x|
 }
 
+// The Fourier-plane step of one point, shared by the kernels that iterate (row_fourier_kernel writes out its GD step).
+// m2 = |C|^2 (GS) / |F|^2 (GD).
+// GS error sums (algorithms.py:36-38), taken against the scale s0 of the previous iteration: u = s0 |C|^2, d = u - T;
+// max |C|^2, sum d^2, sum d u, sum u^2.  The exact scale s = norm/max is folded in when the plane closes (gs_error).
+// t may be a grey level (an integer): it is converted to R where d is formed.
+template <typename R, typename T> SLM_DEV void gs_sums(R m2, T t, R s0r, R& mx, R& sa, R& sb, R& sc) {
+    const R u = s0r * m2, d = u - (R)t;
+    mx = fmax(mx, m2); sa += d * d; sb += d * u; sc += u * u;
+}
+// D = |amp| * exp(1j*angle(C)), algorithms.py:33
+template <typename R> SLM_DEV void replace_amplitude(cpx<R>& v, R m2, R amp) {
+    if (m2 == (R)0) v = mk<R>(copysign(amp, v.x), (R)0);
+    else v = cscale(v, amp * rsqrt_fast(m2));
+}
+// GD output = |F|^2 * norm / max, algorithms.py:85-86.  fp32: gdk = (R)(norm / max), formed once per plane.
+template <typename R> SLM_DEV R gd_output(R m2, R gdk, double norm, double imax) {
+    if (sizeof(R) == 8) return (R)(((double)m2 * norm) / imax);
+    return m2 * gdk;
+}
+// mask * med_output * (output - T), algorithms.py:88, and its error sum sum (output - T)^2, :92
+template <typename R> SLM_DEV cpx<R> gd_point(cpx<R> v, R output, R t, R mask, R& sa) {
+    const R d = output - t;
+    sa += d * d;
+    return cscale(cscale(v, mask), d);
+}
+
 // ---- deterministic reductions ---------------------------------------------------------------------
 // FIELDS selects which members of Partial a kernel actually uses (bit 0 mx, 1 a, 2 b, 3 c) so the
 // shuffle trees only move those.
@@ -347,12 +373,9 @@ SLM_DEV void col_pass_tile(const ColArgs& a, int b, int tile, int tiles, cpx<R>*
     const R wlo = GSW ? (R)(1.0 / a.weight_limit) : (R)0, whi = GSW ? (R)a.weight_limit : (R)0;
 #pragma unroll
     for (int r = 0; r < E; ++r) {
-        const R m2 = cnorm2(v[r]);                              // |C|^2, algorithms.py:36 / :85
+        const R m2 = cnorm2(v[r]);
         if (ALG == ALG_GS || GSW) {
-            // error of this iteration against the scale s0 of the previous one; the exact scale
-            // s = norm/max is folded in by the last tile (gs_error).
-            const R u = s0r * m2, d = u - tv[r];
-            mx = fmax(mx, m2); sa += d * d; sb += d * u; sc += u * u;
+            gs_sums(m2, tv[r], s0r, mx, sa, sb, sc);
             R amp = aux[r];
             if (GSW) {
                 // the weights are read here, after the forward transform, not before it like the target: held through
@@ -366,15 +389,9 @@ SLM_DEV void col_pass_tile(const ColArgs& a, int b, int tile, int tiles, cpx<R>*
                 st_cg(wp, w);
                 amp = aux[r] * w;
             }
-            // D = |amp| * exp(1j*angle(C)), algorithms.py:33
-            v[r] = (m2 == (R)0) ? mk<R>(copysign(amp, v[r].x), (R)0) : cscale(v[r], amp * rsqrt_fast(m2));
+            replace_amplitude(v[r], m2, amp);
         } else {
-            R I;                                                 // output, algorithms.py:86
-            if (sizeof(R) == 8) I = (R)(((double)m2 * norm) / imax);
-            else I = m2 * gdk;
-            const R d = I - tv[r];
-            sa += d * d;
-            v[r] = cscale(cscale(v[r], aux[r]), d);              // mask * med_output * (output - T), :88
+            v[r] = gd_point(v[r], gd_output(m2, gdk, norm, imax), tv[r], aux[r], sa);
         }
     }
     constexpr int KIND = ALG == ALG_GD ? CLOSE_GD : CLOSE_GS, FIELDS = close_fields(KIND);
@@ -678,12 +695,13 @@ SLM_GLOBAL void SLM_LAUNCH_BOUNDS((RowGeom<R, W>::THREADS), (RowGeom<R, W>::MIN_
         const int grey = (int)((grey4[r / 4] >> (8 * (r % 4))) & 0xffu);
         if (MODE == RF_GS) {
             const R amp = lut_s[grey];
-            const R u = s0r * m2, d = u - (R)grey;
-            mx = fmax(mx, m2); sa += d * d; sb += d * u; sc += u * u;
-            v[r] = (m2 == (R)0) ? mk<R>(copysign(amp, v[r].x), (R)0) : cscale(v[r], amp * rsqrt_fast(m2));   // algorithms.py:33
+            gs_sums(m2, grey, s0r, mx, sa, sb, sc);
+            replace_amplitude(v[r], m2, amp);
         } else if (MODE == RF_GD_MAX) {
             mx = fmax(mx, m2);                                                 // amax(output_unnormed), algorithms.py:86
         } else {
+            // gd_output / gd_point written out: the table is read after the error sum here; a call reads it first, and that
+            // changes the compiled fp64 kernels
             R I;                                                               // output, algorithms.py:86
             if (sizeof(R) == 8) I = (R)(((double)m2 * a.norm) / gd_max);
             else I = m2 * gdk;
