@@ -12,7 +12,7 @@
  *   - "device" pointers are valid on the context's device; "host" pointers are ordinary memory
  *     read before the call returns.  Planes are row-major [batch][H][W].
  *   - complex<R>/real<R>: R = float for SLM_PREC_F32 contexts, double for SLM_PREC_F64 ones.
- *   - all work is enqueued on the context's stream; only slm_read_curves synchronises.
+ *   - all work is enqueued on the context's stream; only slm_read_curves and slm_rows_state synchronise.
  *   - a context is not thread-safe; no device allocation happens after slm_ctx_create.
  */
 #ifndef SLM_HOLO_H
@@ -146,39 +146,41 @@ int slm_rows_fft(slm_ctx* ctx, const void* in, const uint8_t* in_u8, const doubl
  * final_pass: write angle(A) to `hologram` (device double [rows][W]) instead of starting the next fft2. */
 int slm_rows_gs_row_pass(slm_ctx* ctx, const void* in, void* out, const void* inc_amp, int in_is_field, int final_pass,
                          double* hologram);
-/* Fourier-plane step (algorithms.py:31-38) on received columns in the exchange layout: finishes fft2, replaces
- * the amplitude, starts ifft2; per-line sums (max |C|^2, sum r^2, sum r*u, sum u^2 against the previous iteration's
- * scale, read from device memory at scale_prev_dev: the loop state stays on the device, see slm_rows_close) go to
- * partial[rows][4]; intensity (nullable, device double, same layout) receives |C|^2. */
-int slm_rows_gs_fourier_pass(slm_ctx* ctx, const void* in, void* out, int block_w, const uint8_t* target_u8,
-                             const double* amp_lut, const double* scale_prev_dev, double* partial, double* intensity);
+/* Fourier-plane step on received columns in the exchange layout (block_w: the block width), by `mode`:
+ *   0 (GS, algorithms.py:31-38): finish fft2, replace the amplitude (lut: host double[256], amplitude by grey level),
+ *     start ifft2; per-line sums max |C|^2, sum r^2, sum r*u, sum u^2 against the scale of the previous iteration;
+ *   1 (GD max, :84-86): finish fft2, keep the transform (out), max |F|^2 per line into partial[.][0];
+ *   2 (GD step on the kept transform, after slm_rows_close kind 0 has closed mode 1's maxima: :85-88,92): output,
+ *     error sum into partial[.][1], mask * F * (output - T) (lut: the mask by grey level), first half of ifft2.
+ * Modes 0 and 2 need target_u8 and lut; norm = amax(T) (read by mode 2).  Scale and max come from the context's loop
+ * state (slm_rows_close), which stays on the device.  partial: device double[rows][4]; intensity (nullable, device
+ * double, same layout as `in`; modes 0 and 2) receives |C|^2 (GD: the expected outcome = that * norm / max). */
+int slm_rows_fourier_pass(slm_ctx* ctx, int mode, const void* in, void* out, int block_w, const uint8_t* target_u8,
+                          const double* lut, double norm, double* partial, double* intensity);
 /* partial[rows][4] -> out4 (device double[4]: max, three sums) by one CTA in a fixed order.  With n_peers > 0 the four
  * numbers are also stored into every peer's gathered[self] (peer_gathered[r] = rank r's device double[n_peers][4],
  * mapped into this process: peer memory over NVLink) -- otherwise the caller all-gathers out4. */
 int slm_rows_reduce(slm_ctx* ctx, const double* partial, int rows, double* out4, const void* const* peer_gathered,
                     int n_peers, int self);
-/* Close one GS iteration of the distributed plane from every rank's four numbers (gathered: device double[world][4],
- * rank order): scale = norm / max (algorithms.py:37), error (algorithms.py:38,162) appended to err_curve (device),
- * loop condition (algorithms.py:29).  state: device double[8] = {scale (in: the one the pass used; out: the new one),
- * last error, iterations done, loop-ended flag, max |C|^2, -, -, -}.  form 0: a GS iteration; 1: only scale and max (the
- * exact scale of GS iteration 0, the max pass of a GD iteration); 2: a GD iteration (error = sum (output - T)^2 / HW). */
-int slm_rows_close(slm_ctx* ctx, const double* gathered, int world, double norm, double hw, int form, double tolerance,
-                   double* state, double* err_curve);
-/* Gradient descent (algorithms.py:60-112) on the distributed plane, same exchange as GS:
+/* Close a Fourier-plane pass of the distributed plane from every rank's four numbers (gathered: device double[world][4],
+ * added in rank order) into the context's loop state.  kind 0: the max and the scale norm / max only (the exact scale
+ * of GS iteration 0, the max pass of a GD iteration); 1: a GS iteration (scale, error algorithms.py:37-38,162);
+ * 2: a GD iteration (error = sum (output - T)^2 / HW, :92).  Kinds 1 and 2 append the error to err_curve (device
+ * double[max_loops]), count the iteration and set the loop-ended flag (algorithms.py:29,83). */
+int slm_rows_close(slm_ctx* ctx, const double* gathered, int world, double norm, double hw, int kind, double tolerance,
+                   double* err_curve);
+/* The context's loop state, read back (synchronises the stream; every output nullable): scale and max of the latest
+ * closing, iterations closed, loop-ended flag. */
+int slm_rows_state(slm_ctx* ctx, double* scale, double* imax, int* iters, int* done);
+/* Gradient descent (algorithms.py:60-112) on the distributed plane, same exchange as GS and two Fourier-plane passes
+ * (modes 1 and 2, each closed by slm_rows_close: kind 0, then kind 2) per iteration:
  *   slm_rows_reset           zero the context's loop state before a run;
  *   slm_rows_gd_row_pass     SLM-plane pass on this rank's rows: finish ifft2 along the rows (in: lines back from the exchange),
  *                            dEdX + update of x in place with lr_dev[iteration] (:87-91,179-185), x/|x| and the row half of fft2
  *                            (:84) into out; first != 0: no update yet (the run's first pass); final_pass != 0: the last update,
- *                            then angle(x) into hologram (:111) instead of a transform;
- *   slm_rows_gd_fourier_pass stage 0: finish fft2 along the received lines, keep the transform (out), max |F|^2 per line into
- *                            partial[.][0] (:84-86); stage 1 (after slm_rows_close form 1 has put norm/max and max into state):
- *                            output, error sum into partial[.][1], mask * F * (output - T), first half of ifft2 (:85-88,92);
- *                            intensity (nullable): |F|^2 of the lines (expected outcome = that * norm / max);
- *   slm_rows_close           form 1 after stage 0, form 2 after stage 1 (error curve, iteration count, loop condition). */
+ *                            then angle(x) into hologram (:111) instead of a transform. */
 int slm_rows_reset(slm_ctx* ctx);
 int slm_rows_gd_row_pass(slm_ctx* ctx, const void* in, void* x, void* out, const double* lr_dev, int first, int final_pass, double* hologram);
-int slm_rows_gd_fourier_pass(slm_ctx* ctx, const void* in, void* out, int block_w, const uint8_t* target_u8, const double* mask_lut,
-                             double norm, const double* state_dev, double* partial, double* intensity, int stage);
 /* row slab [rows][W] <-> exchange layout [W/rows][rows][rows] (each block transposed); elem_bytes 1, 8 or 16. */
 int slm_transpose_blocks(slm_ctx* ctx, const void* in, void* out, int rows, int W, int elem_bytes, int from_exchange);
 

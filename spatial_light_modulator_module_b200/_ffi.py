@@ -14,6 +14,8 @@ LIB_PATH = os.path.join(_HERE, "lib", "libslmholo.so")
 
 PREC_F32, PREC_F64 = 0, 1
 QUANT_ROUND_WRAP, QUANT_PIL_FLOAT, QUANT_FLOOR, QUANT_PREVIEW = 1, 2, 3, 5
+RF_GS, RF_GD_MAX, RF_GD_POST = 0, 1, 2          # slm_rows_fourier_pass modes
+CLOSE_MAX, CLOSE_GS, CLOSE_GD = 0, 1, 2         # slm_rows_close kinds
 
 _vp, _i, _d, _ll = C.c_void_p, C.c_int, C.c_double, C.c_longlong
 _dp, _ip = C.POINTER(C.c_double), C.POINTER(C.c_int)
@@ -42,12 +44,12 @@ SIGNATURES = {
     "slm_rows_create": (_i, [C.POINTER(_vp), _i, _i, _i, _i, _vp]),
     "slm_rows_fft": (_i, [_vp, _vp, _vp, _dp, _vp, _i, _i, _i]),
     "slm_rows_gs_row_pass": (_i, [_vp, _vp, _vp, _vp, _i, _i, _vp]),
-    "slm_rows_gs_fourier_pass": (_i, [_vp, _vp, _vp, _i, _vp, _dp, _vp, _vp, _vp]),
+    "slm_rows_fourier_pass": (_i, [_vp, _i, _vp, _vp, _i, _vp, _dp, _d, _vp, _vp]),
     "slm_rows_reduce": (_i, [_vp, _vp, _i, _vp, _vp, _i, _i]),
-    "slm_rows_close": (_i, [_vp, _vp, _i, _d, _d, _i, _d, _vp, _vp]),
+    "slm_rows_close": (_i, [_vp, _vp, _i, _d, _d, _i, _d, _vp]),
+    "slm_rows_state": (_i, [_vp, _dp, _dp, _ip, _ip]),
     "slm_rows_reset": (_i, [_vp]),
     "slm_rows_gd_row_pass": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _vp]),
-    "slm_rows_gd_fourier_pass": (_i, [_vp, _vp, _vp, _i, _vp, _dp, _d, _vp, _vp, _vp, _i]),
     "slm_transpose_blocks": (_i, [_vp, _vp, _vp, _i, _i, _i, _i]),
     "slm_transpose_blocks_peer": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i, _i]),
     "slm_read_curves": (_i, [_vp, _i, _i, _dp, _ip]),

@@ -272,7 +272,7 @@ SLM_GLOBAL void transpose_blocks_peer_kernel(const T* in, PeerPtrs peers, int h,
     }
 }
 
-// ---- loop state of the row-slab GS on the device (no host round trip per iteration) ---------------------------------
+// ---- loop state of the row-slab GS and GD on the device (no host round trip per iteration) --------------------------
 // partial[rows][4] (max |C|^2, sum r^2, sum r*u, sum u^2 per line) -> out[4] for this rank: ONE CTA, fixed order.
 SLM_GLOBAL void rows_reduce_kernel(const double* partial, int rows, double* out, PeerPtrs peers, int n_peers, int self) {
     Partial q; q.mx = 0; q.a = 0; q.b = 0; q.c = 0;
@@ -289,34 +289,17 @@ SLM_GLOBAL void rows_reduce_kernel(const double* partial, int rows, double* out,
         }
     }
 }
-// gathered[world][4] -> the plane's max and sums (rank order: the same bits on every rank); closes the iteration like
-// close_plane<CLOSE_GS>: state[0] = scale (in: the one the pass used, out: norm / max), state[1] = error, state[2] = iterations
-// done (as a double), state[3] = loop-ended flag.  prepass: only the scale (exact scale of iteration 0).
-// form: 0 GS iteration; 1 only the scale and the max (GS iteration 0's exact scale; the max pass of every GD iteration,
-// algorithms.py:86); 2 GD iteration: error = sum (output - T)^2 / HW (algorithms.py:92), scale and max stay.  `stats`
-// (nullable): the context's PlaneStats, which the GD SLM-plane pass reads (iteration count -> learning rate, loop ended).
-SLM_GLOBAL void rows_close_kernel(const double* gathered, int world, double norm, double hw, int form, int as_float,
-                                  double tolerance, double* state, double* err_curve, PlaneStats* stats) {
+// gathered[world][4] -> the plane's max and sums, added in rank order (the same bits on every rank) -> the plane's
+// closing of kind KIND (close_plane) in the context's PlaneStats; the Fourier-plane pass used the scale held there.
+template <typename R, int KIND>
+SLM_GLOBAL void rows_close_kernel(const double* gathered, int world, double norm, double hw, double tolerance,
+                                  double* err_curve, PlaneStats* st) {
     if (threadIdx.x != 0 || blockIdx.x != 0) return;
-    double mx = 0, a = 0, b = 0, c = 0;
+    Partial tot; tot.mx = 0; tot.a = 0; tot.b = 0; tot.c = 0;
     for (int r = 0; r < world; ++r) {
-        mx = fmax(mx, gathered[4 * r]); a += gathered[4 * r + 1]; b += gathered[4 * r + 2]; c += gathered[4 * r + 3];
+        tot.mx = fmax(tot.mx, gathered[4 * r]); tot.a += gathered[4 * r + 1]; tot.b += gathered[4 * r + 2]; tot.c += gathered[4 * r + 3];
     }
-    if (form == 1) { state[0] = norm / mx; state[4] = mx; return; }
-    double err;
-    if (form == 0) {
-        const double s = norm / mx;                               // algorithms.py:37
-        const double s0u = as_float ? (double)(float)state[0] : state[0];      // the scale the kernel used
-        err = gs_error(a, b, c, s, s0u, hw);
-        state[0] = s; state[4] = mx;
-    } else {
-        err = a / hw;                                             // algorithms.py:92
-    }
-    const int k = (int)state[2];
-    err_curve[k] = err;
-    state[1] = err; state[2] = (double)(k + 1);
-    state[3] = !(err > tolerance) ? 1.0 : 0.0;                    // loop condition, algorithms.py:29,83
-    if (stats) { stats->err = err; stats->iters = k + 1; stats->done = !(err > tolerance); }
+    close_plane<R, KIND>(st, tot, st->scale, norm, hw, err_curve, tolerance);
 }
 
 // complex<R> <-> complex128 / real conversions at the boundary (numpy hands over complex128)

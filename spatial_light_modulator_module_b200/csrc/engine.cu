@@ -399,7 +399,7 @@ template <class F> static int replay_iterations(slm_ctx* c, int batch, int times
 }
 
 extern "C" const char* slm_last_error(void) { return g_err.c_str(); }
-extern "C" int slm_version(void) { return 103; }
+extern "C" int slm_version(void) { return 104; }
 extern "C" int slm_supported_lengths(int* out, int cap) { return supported_lengths(out, cap); }
 
 extern "C" void slm_ctx_destroy(slm_ctx* c) {
@@ -895,11 +895,11 @@ extern "C" int slm_rows_create(slm_ctx** out, int device, int rows, int W, int p
     row->prepare();
     int rc = 0;
     auto A = [&](void** p, size_t n) { if (!rc) rc = dev_alloc(c, p, n); };
-    A((void**)&c->stats, sizeof(PlaneStats));
+    A((void**)&c->stats, 2 * sizeof(PlaneStats));           // [0] the loop state, [1] stays zero (slm_rows_gs_row_pass)
     A(&c->lut, 256 * real_size(precision));
     A((void**)&c->lut32, 256 * sizeof(float));
     if (!rc) rc = make_twiddles(c, W, precision, &c->tw_row);
-    if (!rc && cudaMemset(c->stats, 0, sizeof(PlaneStats)) != cudaSuccess) rc = fail(SLM_ERR_CUDA, "cudaMemset(stats)");
+    if (!rc && cudaMemset(c->stats, 0, 2 * sizeof(PlaneStats)) != cudaSuccess) rc = fail(SLM_ERR_CUDA, "cudaMemset(stats)");
     if (rc) { std::string keep = g_err; slm_ctx_destroy(c); g_err = keep; return rc; }
     *out = c;
     return 0;
@@ -931,7 +931,10 @@ extern "C" int slm_rows_gs_row_pass(slm_ctx* c, const void* in, void* out, const
     if (!c || !in || (final_pass ? !hologram : !out)) return fail(SLM_ERR_ARG, "slm_rows_gs_row_pass: bad argument");
     SLM_CUDA(cudaSetDevice(c->device));
     RowArgs ra{};
-    ra.B = 1; ra.H = c->H; ra.Y = in; ra.field = in; ra.X = out; ra.inc = inc_amp; ra.stats = c->stats; ra.hologram = hologram;
+    // A GS run on the slab ends where the caller stops issuing iterations: with tolerance <= 0 it runs them all and cuts
+    // the error curve itself.  So its row passes read the record that stays zero, not the loop-ended flag, which an error
+    // of exactly 0 sets (one bright pixel at the origin), and which would stop them while the Fourier-plane passes go on.
+    ra.B = 1; ra.H = c->H; ra.Y = in; ra.field = in; ra.X = out; ra.inc = inc_amp; ra.stats = c->stats + 1; ra.hologram = hologram;
     ra.inv_hw = 1.0; ra.tw = c->tw_row; ra.final_pass = final_pass;
     ra.A32 = in;
     ra.source = in_is_field == 2 ? ROW_FROM_A32 : (in_is_field ? ROW_FROM_A : ROW_FROM_Y);
@@ -939,17 +942,19 @@ extern "C" int slm_rows_gs_row_pass(slm_ctx* c, const void* in, void* out, const
     return 0;
 }
 
-extern "C" int slm_rows_gs_fourier_pass(slm_ctx* c, const void* in, void* out, int block_w, const uint8_t* target_u8,
-                                        const double* amp_lut, const double* scale_prev_dev, double* partial, double* intensity) {
-    if (!c || !in || !out || !target_u8 || !amp_lut || !partial || !scale_prev_dev) return fail(SLM_ERR_ARG, "slm_rows_gs_fourier_pass: bad argument");
+extern "C" int slm_rows_fourier_pass(slm_ctx* c, int mode, const void* in, void* out, int block_w, const uint8_t* target_u8,
+                                     const double* lut, double norm, double* partial, double* intensity) {
+    if (!c || !in || !out || !partial || mode < RF_GS || mode > RF_GD_POST) return fail(SLM_ERR_ARG, "slm_rows_fourier_pass: bad argument");
+    const bool has_target = mode != RF_GD_MAX;
+    if (has_target && (!target_u8 || !lut)) return fail(SLM_ERR_ARG, "slm_rows_fourier_pass: this mode needs the target and its table");
     if (!block_width_ok(c, block_w))
-        return fail(SLM_ERR_SHAPE, "slm_rows_gs_fourier_pass: the exchange block width must be a power-of-two multiple of the line's thread count");
+        return fail(SLM_ERR_SHAPE, "slm_rows_fourier_pass: the exchange block width must be a power-of-two multiple of the line's thread count");
     SLM_CUDA(cudaSetDevice(c->device));
-    SLM_TRY(upload_lut(c, amp_lut));
+    if (has_target) SLM_TRY(upload_lut(c, lut));
     RowFourierArgs fa{};
-    fa.rows = c->H; fa.block_w = block_w; fa.in = in; fa.out = out; fa.T8 = target_u8; fa.lut = c->lut; fa.s0_dev = scale_prev_dev;
-    fa.partial = partial; fa.intensity = intensity; fa.tw = c->tw_row;
-    SLM_TIMED(K_COL_PASS, c->row->row_fourier(fa, c->stream));
+    fa.rows = c->H; fa.block_w = block_w; fa.in = in; fa.out = out; fa.T8 = target_u8; fa.lut = c->lut; fa.stats = c->stats;
+    fa.mode = mode; fa.norm = norm; fa.partial = partial; fa.intensity = intensity; fa.tw = c->tw_row;
+    SLM_TIMED(mode == RF_GD_MAX ? K_COL_STATS : K_COL_PASS, c->row->row_fourier(fa, c->stream));
     return 0;
 }
 
@@ -970,12 +975,17 @@ extern "C" int slm_rows_reduce(slm_ctx* c, const double* partial, int rows, doub
     return 0;
 }
 
-extern "C" int slm_rows_close(slm_ctx* c, const double* gathered, int world, double norm, double hw, int form, double tolerance,
-                              double* state, double* err_curve) {
-    if (!c || !gathered || !state || world < 1 || form < 0 || form > 2 || (form != 1 && !err_curve)) return fail(SLM_ERR_ARG, "slm_rows_close: bad argument");
+extern "C" int slm_rows_close(slm_ctx* c, const double* gathered, int world, double norm, double hw, int kind, double tolerance,
+                              double* err_curve) {
+    if (!c || !gathered || world < 1 || kind < CLOSE_MAX || kind > CLOSE_GD || (kind != CLOSE_MAX && !err_curve))
+        return fail(SLM_ERR_ARG, "slm_rows_close: bad argument");
     SLM_CUDA(cudaSetDevice(c->device));
-    { LaunchTimer t_(c, K_ELEMENTWISE); SLM_LAUNCH(rows_close_kernel, dim3(1), dim3(32), 0, c->stream, gathered, world, norm, hw, form,
-                                                    c->prec == PREC_F32 ? 1 : 0, tolerance, state, err_curve, form == 2 ? c->stats : nullptr); }
+    using CloseKernel = void (*)(const double*, int, double, double, double, double*, PlaneStats*);
+    static const CloseKernel kernels[2][3] = {     // [precision][kind]
+        {rows_close_kernel<float, CLOSE_MAX>, rows_close_kernel<float, CLOSE_GS>, rows_close_kernel<float, CLOSE_GD>},
+        {rows_close_kernel<double, CLOSE_MAX>, rows_close_kernel<double, CLOSE_GS>, rows_close_kernel<double, CLOSE_GD>}};
+    { LaunchTimer t_(c, K_ELEMENTWISE); SLM_LAUNCH(kernels[c->prec][kind], dim3(1), dim3(32), 0, c->stream, gathered, world, norm, hw,
+                                                    tolerance, err_curve, c->stats); }
     SLM_CUDA(cudaGetLastError());
     return 0;
 }
@@ -984,6 +994,19 @@ extern "C" int slm_rows_reset(slm_ctx* c) {
     if (!c) return fail(SLM_ERR_ARG, "slm_rows_reset: null context");
     SLM_CUDA(cudaSetDevice(c->device));
     SLM_CUDA(cudaMemsetAsync(c->stats, 0, sizeof(PlaneStats), c->stream));
+    return 0;
+}
+
+extern "C" int slm_rows_state(slm_ctx* c, double* scale, double* imax, int* iters, int* done) {
+    if (!c) return fail(SLM_ERR_ARG, "slm_rows_state: null context");
+    SLM_CUDA(cudaSetDevice(c->device));
+    PlaneStats st;
+    SLM_CUDA(cudaMemcpyAsync(&st, c->stats, sizeof st, cudaMemcpyDeviceToHost, c->stream));
+    SLM_CUDA(cudaStreamSynchronize(c->stream));
+    if (scale) *scale = st.scale;
+    if (imax) *imax = st.imax;
+    if (iters) *iters = st.iters;
+    if (done) *done = st.done;
     return 0;
 }
 
@@ -997,21 +1020,6 @@ extern "C" int slm_rows_gd_row_pass(slm_ctx* c, const void* in, void* x, void* o
     ra.tw = c->tw_row; ra.final_pass = final_pass;
     ra.source = first ? ROW_FROM_FIELD : ROW_FROM_Y;
     SLM_TIMED(K_ROW_PASS, c->row->row_pass(ALG_GD, ra, c->stream));
-    return 0;
-}
-
-extern "C" int slm_rows_gd_fourier_pass(slm_ctx* c, const void* in, void* out, int block_w, const uint8_t* target_u8, const double* mask_lut,
-                                        double norm, const double* state_dev, double* partial, double* intensity, int stage) {
-    if (!c || !in || !out || !partial || (stage != 0 && stage != 1)) return fail(SLM_ERR_ARG, "slm_rows_gd_fourier_pass: bad argument");
-    if (stage == 1 && (!target_u8 || !mask_lut || !state_dev)) return fail(SLM_ERR_ARG, "slm_rows_gd_fourier_pass: the gradient stage needs target, table and state");
-    if (!block_width_ok(c, block_w))
-        return fail(SLM_ERR_SHAPE, "slm_rows_gd_fourier_pass: the exchange block width must be a power-of-two multiple of the line's thread count");
-    SLM_CUDA(cudaSetDevice(c->device));
-    if (stage == 1) SLM_TRY(upload_lut(c, mask_lut));
-    RowFourierArgs fa{};
-    fa.rows = c->H; fa.block_w = block_w; fa.in = in; fa.out = out; fa.T8 = target_u8; fa.lut = c->lut; fa.partial = partial; fa.intensity = intensity;
-    fa.tw = c->tw_row; fa.mode = stage == 0 ? RF_GD_MAX : RF_GD_POST; fa.norm = norm; fa.state = state_dev;
-    SLM_TIMED(stage == 0 ? K_COL_STATS : K_COL_PASS, c->row->row_fourier(fa, c->stream));
     return 0;
 }
 

@@ -164,10 +164,10 @@ struct RowFourierArgs {
     void* out;               // complex<R>: lines ready for the return exchange
     const uint8_t* T8;       // target, same layout as `in`
     const void* lut;         // R[256] amplitude by grey level
-    const double* s0_dev;    // RF_GS: scale of the previous iteration (algorithms.py:37), in device memory (loop state)
+    const PlaneStats* stats; // the context's loop state (slm_rows_close): RF_GS reads the previous iteration's scale
+                             // (algorithms.py:37), RF_GD_POST this iteration's norm / max and max
     int mode;                // RowFourierMode
     double norm;             // RF_GD_POST: amax(T) (algorithms.py:74)
-    const double* state;     // RF_GD_POST: device loop state {norm/max, error, iterations, ended, max} (slm_rows_close)
     double* partial;         // device [rows][4]: max |C|^2, sum r^2, sum r*u, sum u^2 per line
     double* intensity;       // device double, same layout, or null: |C|^2 (final expected_outcome, unscaled)
     const void* tw;

@@ -574,7 +574,7 @@ SLM_DEV size_t line_offset(int wb, int rows, int W, long long row, int n) {
 
 // The same for the E points j + r*M (r < E) one thread of the slab path's Fourier-plane kernel holds, without a
 // division per point: a block is a whole power-of-two number q of M-element runs (the host checks this:
-// slm_rows_gs_fourier_pass), so point r lies in block r / q at run r % q; 32-bit element offsets (one slab has
+// slm_rows_fourier_pass), so point r lies in block r / q at run r % q; 32-bit element offsets (one slab has
 // fewer than 2^32 elements).  With the general div / mod form inlined at each of its ~100 uses the 16384-point
 // kernel was 9000 instructions and its warps waited for instruction fetches (ncu: no_instruction 38 %);
 // 3.8 -> 3.1 ms per pass, 136 -> 145 iterations/s on one GPU (same box, two runs each).
@@ -674,8 +674,8 @@ SLM_GLOBAL void SLM_LAUNCH_BOUNDS((RowGeom<R, W>::THREADS), (RowGeom<R, W>::MIN_
     // (one CTA per SM and nothing to hide a global load behind)
     SLM_STATIC_SMEM R lut_s[256];
     if (HAS_T) for (int i = t; i < 256; i += G::THREADS) lut_s[i] = ld_ro(lut + i);
-    const R s0r = MODE == RF_GS ? (R)ld_cg(a.s0_dev) : (R)0;
-    const double gd_scale = MODE == RF_GD_POST ? ld_cg(a.state) : 0.0, gd_max = MODE == RF_GD_POST ? ld_cg(a.state + 4) : 0.0;
+    const R s0r = MODE == RF_GS ? (R)ld_cg(&a.stats->scale) : (R)0;
+    const double gd_scale = MODE == RF_GD_POST ? ld_cg(&a.stats->scale) : 0.0, gd_max = MODE == RF_GD_POST ? ld_cg(&a.stats->imax) : 0.0;
     sync_cta();
     cpx<R> v[E];
     unsigned grey4[(E + 3) / 4];                              // the points' grey levels, four to a register (they wait through a transform)

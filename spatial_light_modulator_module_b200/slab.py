@@ -12,8 +12,9 @@ Rank p owns rows [p*h, (p+1)*h) of the N x N field, h = N / world.  One GS itera
     exchange      all-to-all back -> unpack into the row slab
 
 i.e. two all-to-alls and one tiny all-gather per iteration; the target is exchanged once.  All array work is done by
-kernels of libslmholo (``slm_rows_*``, ``slm_transpose_blocks*``).  The loop state (scale, error curve, iteration
-count) lives on the device: with ``tolerance <= 0`` -- every caller of the reference -- no iteration waits for the host.
+kernels of libslmholo (``slm_rows_*``, ``slm_transpose_blocks*``).  The loop state (the context's scale, max, iteration
+count and loop-ended flag, and the run's error curve) lives on the device: with ``tolerance <= 0`` -- every caller of the
+reference -- no iteration waits for the host.
 
 Two ways of moving the blocks:
 
@@ -204,7 +205,7 @@ class SlabEngine(Engine):
     # ---- what a GS and a GD run share ---------------------------------------------------------------------------------
     def _begin(self, target_slab, max_loops: int, want_expected: bool) -> SimpleNamespace:
         """Check this rank's uint8 target rows (host array or device buffer), take the plane's max over the ranks, exchange
-        the target once into the column layout, allocate the run's buffers and loop state and reset the context's."""
+        the target once into the column layout, allocate the run's buffers and reset the context's loop state."""
         if self._mem_is_device(target_slab):
             T = target_slab
             if tuple(T.shape) != self.shape or self._mem_np_dtype(T) != np.uint8:
@@ -228,8 +229,7 @@ class SlabEngine(Engine):
         r.S = self._mem_empty(blocks, self.complex_dtype)                 # exchange layout: lines (and the send side of the collectives)
         r.Rv = buf("Rv", blocks, self.complex_dtype)                      # receive side
         r.partial = self._mem_empty((self.rows, 4), np.float64)
-        # loop state on the device: {scale, last error, iterations done, loop ended, max}, the error curve, the ranks' sums
-        r.state = self._mem_upload(np.array([1.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0]))
+        # the error curve and the ranks' sums (the rest of the loop state is the context's)
         r.curve = self._mem_empty((max_loops,), np.float64)
         r.mine = self._mem_empty((4,), np.float64)
         # (two slots used in turn: a rank may run one closing step ahead of a peer that is still reading the previous one)
@@ -239,9 +239,9 @@ class SlabEngine(Engine):
         self._check(self._lib.slm_rows_reset(self._ctx))                 # (a finished run's flags would stop the row passes)
         return r
 
-    def _close(self, r, form: int, tolerance: float):
-        """this rank's sums -> every rank -> scale / error / loop condition in ``r.state`` (all on the device); ``form``: that
-        of slm_rows_close (0: GS iteration, 1: scale and max only, 2: GD iteration)"""
+    def _close(self, r, kind: int, tolerance: float):
+        """this rank's sums -> every rank -> the closing ``kind`` (``_ffi.CLOSE_*``) of slm_rows_close in the context's
+        loop state (all on the device)"""
         peer = self._peer is not None
         slot, self._slot = self._slot, self._slot ^ 1
         self._check(self._lib.slm_rows_reduce(self._ctx, self._mem_ptr(r.partial), self.rows, self._mem_ptr(r.mine),
@@ -251,17 +251,22 @@ class SlabEngine(Engine):
             self._peer_barrier()
         else:
             self._all_gather4(r.mine, r.gathered[slot])
-        self._check(self._lib.slm_rows_close(self._ctx, self._mem_ptr(r.gathered[slot]), self.world, r.norm, r.hw, form,
-                                             float(tolerance), self._mem_ptr(r.state), self._mem_ptr(r.curve)))
+        self._check(self._lib.slm_rows_close(self._ctx, self._mem_ptr(r.gathered[slot]), self.world, r.norm, r.hw, kind,
+                                             float(tolerance), self._mem_ptr(r.curve)))
+
+    def _state(self):
+        """(scale, max, loop ended) of the context's loop state, read back"""
+        scale, imax, done = C.c_double(), C.c_double(), C.c_int()
+        self._check(self._lib.slm_rows_state(self._ctx, C.byref(scale), C.byref(imax), None, C.byref(done)))
+        return scale.value, imax.value, done.value != 0
 
     def _curve(self, r, done_iters: int, tolerance: float):
-        """(error curve, loop state), read back; the curve cut where the reference stops (tolerance <= 0: the loop ran on)"""
+        """the error curve, read back and cut where the reference stops (tolerance <= 0: the loop ran on)"""
         errors = [np.float64(e) for e in self.to_host(r.curve)[:done_iters]]
         for i, e in enumerate(errors):
             if not (e > tolerance):
-                errors = errors[:i + 1]
-                break
-        return errors, self.to_host(r.state)
+                return errors[:i + 1]
+        return errors
 
     def _expected(self, r, on_device: bool, scale: float, divisor: float = None):
         """the intensity the run kept, back in rows, times ``scale`` and then over ``divisor`` (GD: times norm, over the max,
@@ -317,21 +322,21 @@ class SlabEngine(Engine):
             self._check(self._lib.slm_rows_gs_row_pass(self._ctx, self._mem_ptr(src), self._mem_ptr(cur), self._mem_ptr(inc), int(field), 0, None))
             self._exchange(cur, r.S, r.Rv, cs, "Rv")
             if k == 0:                                                        # exact scale of iteration 0: max pre-pass
-                self._fourier(r, None)
-                self._close(r, 1, tolerance)
+                self._fourier(r, _ffi.RF_GS, r.Rv, self._amp_lut)
+                self._close(r, _ffi.CLOSE_MAX, tolerance)
             last = k == max_loops - 1
-            self._fourier(r, r.inten if (last or check_every or k == 0) else None)
-            self._close(r, 0, tolerance)
+            self._fourier(r, _ffi.RF_GS, r.Rv, self._amp_lut, r.inten if (last or check_every or k == 0) else None)
+            self._close(r, _ffi.CLOSE_GS, tolerance)
             self._exchange_back(r.S, r.Rv, cur, cs, "X" if cur is r.X else "Y")   # D with the columns inverse-transformed
             src, field, done_iters = cur, 0, k + 1
             if check_every or (k == 0 and not r.norm > 0):                    # (an all-zero target ends the loop at once: 0/0, algorithms.py:29,37)
-                if self.to_host(r.state)[3] != 0.0:
+                if self._state()[2]:
                     break
         self.enqueue_s = time.perf_counter() - t_loop                        # host time to issue the loop (measurements: is the host the bound?)
-        errors, st = self._curve(r, done_iters, tolerance)
+        errors = self._curve(r, done_iters, tolerance)
         holo = self._mem_empty(self.shape, np.float64)
         self._check(self._lib.slm_rows_gs_row_pass(self._ctx, self._mem_ptr(src), None, None, 0, 1, self._mem_ptr(holo)))
-        expected = self._expected(r, on_device, float(st[0]))                # expected_outcome *= norm / max, :37
+        expected = self._expected(r, on_device, self._state()[0])            # expected_outcome *= norm / max, :37
         return (holo if on_device else self.to_host(holo)), expected, errors
 
     # ---- gradient descent on the distributed plane (algorithms.py:60-112) ------------------------------------------------
@@ -352,7 +357,7 @@ class SlabEngine(Engine):
         if lr.shape != (max_loops,):
             raise ValueError("lr_schedule must have max_loops entries")
         r = self._begin(target_slab, max_loops, want_expected)
-        h, cs = self.rows, np.dtype(self.complex_dtype).itemsize
+        cs = np.dtype(self.complex_dtype).itemsize
         if x_on_device:                                                   # (the row pass updates x in place: work on a copy)
             x = self._mem_empty(self.shape, self.complex_dtype)
             self._copy(x0, x)
@@ -368,25 +373,21 @@ class SlabEngine(Engine):
                                                        int(k == 0), 0, None))
             self._exchange(r.X, r.S, r.Rv, cs, "Rv")
             # the plane's max (the transform is kept in S), then the gradient step on it
-            self._check(self._lib.slm_rows_gd_fourier_pass(self._ctx, self._mem_ptr(r.Rv), self._mem_ptr(r.S), h, None, None, r.norm, None,
-                                                           self._mem_ptr(r.partial), None, 0))
-            self._close(r, 1, tolerance)
+            self._fourier(r, _ffi.RF_GD_MAX, r.Rv)
+            self._close(r, _ffi.CLOSE_MAX, tolerance)
             last = k == max_loops - 1
-            want_i = r.inten if (last or check_every or k == 0) else None
-            self._check(self._lib.slm_rows_gd_fourier_pass(self._ctx, self._mem_ptr(r.S), self._mem_ptr(r.S), h, self._mem_ptr(r.Tx),
-                                                           self._dp(mask_lut), r.norm, self._mem_ptr(r.state), self._mem_ptr(r.partial),
-                                                           self._mem_ptr(want_i), 1))
-            self._close(r, 2, tolerance)
+            self._fourier(r, _ffi.RF_GD_POST, r.S, mask_lut, r.inten if (last or check_every or k == 0) else None)
+            self._close(r, _ffi.CLOSE_GD, tolerance)
             self._exchange_back(r.S, r.Rv, r.Y, cs, "Y")
             done_iters = k + 1
             if check_every or (k == 0 and not r.norm > 0):
-                if self.to_host(r.state)[3] != 0.0:
+                if self._state()[2]:
                     break
-        errors, st = self._curve(r, done_iters, tolerance)
+        errors = self._curve(r, done_iters, tolerance)
         holo = self._mem_empty(self.shape, np.float64)
         self._check(self._lib.slm_rows_gd_row_pass(self._ctx, self._mem_ptr(r.Y), self._mem_ptr(x), None, self._mem_ptr(lr_dev), 0, 1,
                                                    self._mem_ptr(holo)))
-        expected = self._expected(r, on_device, r.norm, float(st[4]))      # output_unnormed * norm / amax, algorithms.py:86
+        expected = self._expected(r, on_device, r.norm, self._state()[1])  # output_unnormed * norm / amax, algorithms.py:86
         return (holo if on_device else self.to_host(holo)), expected, errors
 
     def _setup_field(self, T, X, S, Rv, peer_recv=None, peer_slab=None):
@@ -397,10 +398,12 @@ class SlabEngine(Engine):
         self._rows_fft(Rv, S, True, block_in=h, block_out=h)
         self._exchange_back(S, Rv, X, cs, peer_slab)
 
-    def _fourier(self, r, inten):
-        self._check(self._lib.slm_rows_gs_fourier_pass(self._ctx, self._mem_ptr(r.Rv), self._mem_ptr(r.S), self.rows, self._mem_ptr(r.Tx),
-                                                       self._dp(self._amp_lut), self._mem_ptr(r.state), self._mem_ptr(r.partial),
-                                                       self._mem_ptr(inten)))
+    def _fourier(self, r, mode, src, lut=None, inten=None):
+        """Fourier-plane pass ``mode`` (``_ffi.RF_*``) over the received lines ``src`` into r.S (``lut``: the target's
+        table by grey level, GS amplitude or GD mask)"""
+        self._check(self._lib.slm_rows_fourier_pass(self._ctx, mode, self._mem_ptr(src), self._mem_ptr(r.S), self.rows,
+                                                    self._mem_ptr(r.Tx), None if lut is None else self._dp(lut), r.norm,
+                                                    self._mem_ptr(r.partial), self._mem_ptr(inten)))
 
     def close(self):
         self._peer = None                     # (releases this rank's symmetric allocation)

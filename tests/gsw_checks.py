@@ -186,7 +186,7 @@ def check_argument_errors(make_engine, shape, precision):
                                   eng._dp(norms), None, None, 1, 2, 0.0, eng._mem_ptr(holo), None, eng._dp(sums),
                                   eng._mem_ptr(w), c)
         assert rc == -1 and b"weight_limit" in eng._lib.slm_last_error()
-    assert eng._lib.slm_version() == 103
+    assert eng._lib.slm_version() == 104
     eng.close()
 
 

@@ -75,6 +75,32 @@ def test_slab_gs_single_rank_equals_plane_engine(precision):
     np.testing.assert_array_equal(h, ref.to_host(r.hologram)[0])
     np.testing.assert_array_equal(e, ref.to_host(r.expected)[0])
     assert np.max(np.abs(np.array(errs) - r.errors[0]) / r.errors[0]) < 1e-12
+    # a tolerance between two errors of the curve ends the loop where the ordinary engine ends it (algorithms.py:29)
+    stop_at = float(0.5 * (errs[0] + errs[1]))
+    r2 = ref.gs(t, 4, tolerance=stop_at)
+    h2, _, errs2 = eng.gs(t, 4, tolerance=stop_at)
+    assert len(errs2) == len(r2.errors[0]) == 2
+    assert np.max(np.abs(np.array(errs2) - r2.errors[0]) / r2.errors[0]) < 1e-12
+    np.testing.assert_array_equal(h2, ref.to_host(r2.hologram)[0])
+    eng.close(); ref.close()
+
+
+@pytest.mark.parametrize("precision", ["fp32", "fp64"])
+def test_slab_gs_exact_zero_error(precision):
+    """One bright pixel at the origin is a fixed point of GS: the first error is exactly 0, so the default tolerance 0
+    ends the loop there.  The slab path, which runs every iteration and cuts the curve, gives the ordinary engine's
+    hologram, expected outcome and curve."""
+    from tests.emu.emu_engine import EmuEngine, EmuSlabEngine
+    n = 256
+    t = np.zeros((n, n), np.uint8)
+    t[0, 0] = 255
+    ref = EmuEngine((n, n), precision, 1)
+    r = ref.gs(t, 2)
+    eng = EmuSlabEngine(n, 1, 0, precision)
+    h, e, errs = eng.gs(t, 2)
+    assert errs == [0.0] and list(r.errors[0]) == [0.0]
+    np.testing.assert_array_equal(h, ref.to_host(r.hologram)[0])
+    np.testing.assert_array_equal(e, ref.to_host(r.expected)[0])
     eng.close(); ref.close()
 
 
