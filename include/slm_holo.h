@@ -91,6 +91,27 @@ int slm_gsw_run(slm_ctx* ctx, int batch, const uint8_t* target_u8, const void* t
                 int max_loops, double tolerance, double* hologram_out, double* expected_out,
                 const double* target_sum, void* weights, double weight_limit);
 
+/* Multi-plane Gerchberg-Saxton (Haist et al., Opt. Commun. 140, 299 (1997)): one phase hologram for K target planes at
+ * different focus, plane k being the plane a lens of phase alpha_k * rho^2 brings into focus (rho^2 = (y - H/2)^2 +
+ * (x - W/2)^2 in pixels^2; alpha_k = -pi px^2 / (lambda f_k), 0 for the Fourier plane).  With L_k = exp(i alpha_k rho^2):
+ *     setup      A = sum_k ifft2(amp_k) conj(L_k)               (ifft2 as slm_gs_run's setup)
+ *     iteration  B = inc exp(i angle(A));  per plane C_k = fft2(B L_k), D_k = amp_k C_k/|C_k|, error and expected
+ *                outcome of plane k as GS's;  A = sum_k ifft2(D_k) conj(L_k)
+ *     hologram   angle(A) after the last iteration
+ * A hologram iterates until the error of EVERY one of its planes is <= tolerance (or max_loops): its K error curves
+ * have the same length.  planes = 1 with alpha = 0 is slm_gs_run, bit for bit.
+ * Arguments as slm_gs_run, with the batch made of `holograms` x `planes` planes, plane k of hologram g at g*planes + k:
+ *   holograms, planes   1 <= planes <= 8, holograms * planes <= max_batch (else SLM_ERR_ARG)
+ *   target_u8 / target_real / amp_real / norm / expected_out   per plane
+ *   defocus        host double[planes]: alpha_k in radians per pixel^2, finite (else SLM_ERR_ARG), shared by the holograms
+ *   phasor0        device complex<R> [holograms][H][W] or NULL: B of iteration 0
+ *   hologram_out   device double [holograms][H][W]
+ * Error curves: slm_read_curves over holograms * planes planes. */
+int slm_gs_multiplane_run(slm_ctx* ctx, int holograms, int planes, const uint8_t* target_u8, const void* target_real,
+                          const void* amp_real, const double* amp_lut, const double* norm, const double* defocus,
+                          const void* inc_amp, const void* phasor0, int setup_c64, int max_loops, double tolerance,
+                          double* hologram_out, double* expected_out);
+
 /* gradient_descent(demanded_output, args) -- algorithms.py:60-112 (+ dEdX_complex :179-185).
  *   x              device complex<R> [batch][H][W]: the initial guess (algorithms.py:75), updated in place
  *   mask_lut       host double[256]: 1 + white_attention*g/255 for g = 0..255 as numpy computes it

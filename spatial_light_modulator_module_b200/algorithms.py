@@ -20,10 +20,10 @@ import os
 
 import numpy as np
 
-from . import host_logic as hl
+from . import constants, host_logic as hl
 from .engine import Engine, get_engine
 
-__all__ = ["gerchberg_saxton", "weighted_gerchberg_saxton", "gradient_descent", "make_initial_guess", "error_f", "printout",
+__all__ = ["gerchberg_saxton", "weighted_gerchberg_saxton", "multiplane_gerchberg_saxton", "gradient_descent", "make_initial_guess", "error_f", "printout",
            "complex_to_real_phase", "dEdX_complex", "add_gif_image"]
 
 
@@ -107,6 +107,41 @@ def weighted_gerchberg_saxton(demanded_output, args):
     return _gs_family(demanded_output, args, lambda eng, target, n, inc, phasor0:
                       eng.gsw(target, n, float(args.tolerance), inc_amp=inc, phasor0=phasor0,
                               weight_limit=float(getattr(args, "weight_limit", 10.0)))[0])
+
+
+def multiplane_gerchberg_saxton(demanded_outputs, focal_lengths, args):
+    """Multi-plane Gerchberg-Saxton (Haist et al., Opt. Commun. 140, 299 (1997)): one phase hologram for several target
+    images, image k in focus where ``add_lens(hologram, focal_lengths[k])`` would bring the Fourier plane (None or inf:
+    the Fourier plane itself) -- traps in 3-D.  ``demanded_outputs``: K images of one shape (a list or a [K,H,W]
+    array), K <= 8.  Returns ``(hologram, expected[K,H,W], [errors_k])``: each plane's expected outcome and error curve
+    as :func:`gerchberg_saxton` computes them, every curve of the same length (the loop runs while any plane's error is
+    above ``args.tolerance``).  Lenses use the paraxial phase -pi r^2 / (lambda f) at the pixel pitch and wavelength of
+    ``constants``; a focal length short enough to alias at the plane's edge is refused (ValueError), as are
+    ``args.gif``, an all-zero target image and a count of focal lengths other than K."""
+    if getattr(args, "gif", False):
+        raise ValueError("multiplane_gerchberg_saxton does not offer GIF snapshots (args.gif)")
+    targets = np.stack([np.asarray(t) for t in demanded_outputs])
+    focal_lengths = list(focal_lengths)
+    if len(focal_lengths) != len(targets):
+        raise ValueError(f"{len(targets)} target images need {len(targets)} focal lengths, not {len(focal_lengths)}")
+    for k, t in enumerate(targets):
+        if not np.any(t):
+            raise ValueError(f"target image {k} is all zero: it has no intensity to place")
+    inc = _illumination(args, targets.shape[1:])
+    if args.max_loops < 1 or not (args.tolerance + 1 > args.tolerance):
+        print()
+        raise UnboundLocalError("cannot access local variable 'expected_outcome' where it is not associated with a value")
+    alphas = [hl.defocus_coefficient(f, constants.px_distance, constants.wavelength) for f in focal_lengths]
+    eng = _engine(targets.shape[1:], args, batch=len(targets))
+    res = eng.gs_multiplane(targets, alphas, int(args.max_loops), float(args.tolerance), inc_amp=inc)
+    hologram, expected = (a[0] for a in eng.to_host_many([res.hologram, res.expected]))
+    errors = [[np.float64(e) for e in curve] for curve in res.errors[0]]
+    _progress(len(errors[0]), args.max_loops)
+    if args.print_info:
+        for k, curve in enumerate(errors):
+            print(f"\nplane {k}")
+            printout(curve[-1], len(curve), curve, args.plot_error)
+    return hologram, expected, errors
 
 
 def gradient_descent(demanded_output, args):

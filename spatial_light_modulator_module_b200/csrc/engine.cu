@@ -12,6 +12,7 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include <cmath>
 #include <string>
 #include <vector>
 
@@ -50,6 +51,12 @@ struct slm_ctx {
     double *err_curve = nullptr, *lr = nullptr, *norm = nullptr;
     // weighted GS, allocated by the first slm_gsw_run: [max_batch] S_T, [max_batch] P, [max_batch][tiles] partials of P
     double *target_sum = nullptr, *signal_sum = nullptr, *signal_partial = nullptr;
+    // multi-plane GS, allocated by the first slm_gs_multiplane_run: defocus tables [kMaxPlanes][H] and [kMaxPlanes][W]
+    // complex<R>, the alphas they hold, and their host staging (lives as long as the context, like lut_host_f)
+    void *lens_y = nullptr, *lens_x = nullptr;
+    std::vector<double> lens_alpha;
+    std::vector<double> lens_host_d;
+    std::vector<float> lens_host_f;
     void* lut = nullptr;
     float* lut32 = nullptr;
     double lut_host[256];                                 // the table the device copies hold (upload_lut)
@@ -656,15 +663,19 @@ template <class F> static int run_loop(slm_ctx* c, int batch, const char* family
 // every batch size, with the GSW forms of the max pre-pass and of the column pass (col_pass_tile<ALG_GSW>).  The
 // persistent column kernels have no room for a weight tile (col_warp.cuh: three 64 KB tile buffers), so the context's
 // batch does not choose a kernel for it.
+//
+// Multi-plane GS (ra.planes > 0) is GS with the multi-plane row pass (ALG_MP): `batch` counts planes, ra.B holograms.
 static int gs_loop(slm_ctx* c, int batch, bool weighted, RowArgs& ra, ColArgs& ca, const uint8_t* T8, const void* amp_real,
                    const void* phasor0, int setup_c64, double* expected_out) {
+    const bool multiplane = ra.planes > 0;
+    const int row_alg = multiplane ? ALG_MP : ALG_GS;
     if (phasor0) { ra.source = ROW_FROM_FIELD; ra.field = phasor0; }
     else {
         int src = 0;
         SLM_TRY(setup_field(c, batch, T8, amp_real, setup_c64, &src));
         ra.source = src; ra.A32 = c->Y; ra.field = c->Y;
     }
-    SLM_TIMED(K_ROW_PASS, c->row->row_pass(ALG_GS, ra, c->stream));
+    SLM_TIMED(K_ROW_PASS, c->row->row_pass(row_alg, ra, c->stream));
     // Fewer tiles than SMs (one SLM-size plane): the persistent tile pipeline of the column-group kernels has nothing to
     // pipeline, and the plain column kernel -- one CTA per tile, CTA-wide transforms -- has the shorter latency
     // (measured per 100 iterations of one 1024^2 plane: 1.91 against 2.11 ms; 512^2 x 20: 0.35 against 0.39 ms; from
@@ -680,7 +691,8 @@ static int gs_loop(slm_ctx* c, int batch, bool weighted, RowArgs& ra, ColArgs& c
     else SLM_TIMED(K_COL_STATS, c->col->col_plain(stats_args(c, batch, OUT_STATS, nullptr), c->stream));
 
     const int col_alg = weighted ? ALG_GSW : ALG_GS;
-    SLM_TRY(run_loop(c, batch, weighted ? "gsw/plain" : (groups ? "gs/pipeline" : "gs/plain"), ALG_GS, ra, ca, [&]() -> int {
+    const char* family = weighted ? "gsw/plain" : multiplane ? (groups ? "mp/pipeline" : "mp/plain") : (groups ? "gs/pipeline" : "gs/plain");
+    SLM_TRY(run_loop(c, batch, family, row_alg, ra, ca, [&]() -> int {
         if (groups) SLM_TRY(launch_group(c, CGM_GS, batch, &ca, &c->map_y, 0, 1.0));
         else SLM_TIMED(K_COL_PASS, c->col->col_pass(col_alg, ca, c->stream));
         return 0;
@@ -726,6 +738,65 @@ extern "C" int slm_gsw_run(slm_ctx* c, int batch, const uint8_t* T8, const void*
     ca.weights = weights; ca.target_sum = c->target_sum; ca.signal_sum = c->signal_sum; ca.signal_partial = c->signal_partial;
     ca.weight_limit = weight_limit;
     return gs_loop(c, batch, true, ra, ca, T8, amp_real, phasor0, setup_c64, expected_out);
+}
+
+// Multi-plane GS: the defocus tables lens_y[k][i] = exp(i alpha_k (i - H/2)^2) and lens_x[k][j] (W) of `planes` planes, in
+// the context's precision.  Phases are evaluated in extended precision and reduced mod 2 pi before sin / cos, as in
+// make_twiddles.  Uploaded when the alphas differ from those of the previous run.
+static const int kMaxPlanes = 8;
+static int upload_lenses(slm_ctx* c, int planes, const double* alpha) {
+    const size_t cs = 2 * real_size(c->prec);
+    if (!c->lens_y) {
+        SLM_TRY(dev_alloc(c, &c->lens_y, (size_t)kMaxPlanes * c->H * cs));
+        SLM_TRY(dev_alloc(c, &c->lens_x, (size_t)kMaxPlanes * c->W * cs));
+    }
+    if (c->lens_alpha.size() == (size_t)planes && memcmp(c->lens_alpha.data(), alpha, planes * sizeof(double)) == 0) return 0;
+    c->lens_alpha.assign(alpha, alpha + planes);
+    const long double two_pi = 6.283185307179586476925286766559005768L;
+    for (int axis = 0; axis < 2; ++axis) {
+        const int n = axis == 0 ? c->H : c->W;
+        c->lens_host_d.resize(2 * (size_t)planes * n);
+        c->lens_host_f.resize(2 * (size_t)planes * n);
+        for (int k = 0; k < planes; ++k) {
+            for (int i = 0; i < n; ++i) {
+                const long double d = (long double)i - (long double)n / 2;        // lens_kernel's centre (elementwise.cuh)
+                const long double ph = fmodl((long double)alpha[k] * (d * d), two_pi);
+                const size_t q = 2 * ((size_t)k * n + i);
+                c->lens_host_d[q] = (double)cosl(ph); c->lens_host_d[q + 1] = (double)sinl(ph);
+                c->lens_host_f[q] = (float)cosl(ph); c->lens_host_f[q + 1] = (float)sinl(ph);
+            }
+        }
+        // (a copy from pageable memory is staged by the driver before the call returns, see upload_lut)
+        const void* src = c->prec == PREC_F64 ? (const void*)c->lens_host_d.data() : (const void*)c->lens_host_f.data();
+        SLM_CUDA(cudaMemcpyAsync(axis == 0 ? c->lens_y : c->lens_x, src, (size_t)planes * n * cs, cudaMemcpyHostToDevice, c->stream));
+    }
+    return 0;
+}
+
+extern "C" int slm_gs_multiplane_run(slm_ctx* c, int holograms, int planes, const uint8_t* T8, const void* Treal,
+                                     const void* amp_real, const double* amp_lut, const double* norm, const double* defocus,
+                                     const void* inc_amp, const void* phasor0, int setup_c64, int max_loops, double tolerance,
+                                     double* hologram_out, double* expected_out) {
+    const std::string who = "slm_gs_multiplane_run";
+    if (!c) return fail(SLM_ERR_ARG, who + ": null context");
+    if (planes < 1 || planes > kMaxPlanes) return fail(SLM_ERR_ARG, who + ": planes must be in 1.." + std::to_string(kMaxPlanes));
+    if (holograms < 1 || (long long)holograms * planes > c->max_batch)
+        return fail(SLM_ERR_ARG, who + ": holograms * planes must be in 1..max_batch of the context");
+    std::string refused;
+    if (!defocus) refused = "defocus is required";
+    for (int k = 0; defocus && k < planes && refused.empty(); ++k)
+        if (!std::isfinite(defocus[k])) refused = "defocus[" + std::to_string(k) + "] is not finite";
+    if (refused.empty() && c->row && c->row->rows_only) refused = "no multi-plane pass for rows of " + std::to_string(c->W) + " points";
+    RowArgs ra; ColArgs ca;
+    SLM_TRY(begin_loop(c, holograms * planes, who.c_str(), "max_loops must be >= 1 (the reference raises UnboundLocalError for 0)",
+                       norm && hologram_out, "norm and hologram_out", "give target_u8 + amp_lut, or target_real + amp_real",
+                       refused.empty() ? nullptr : refused.c_str(),
+                       T8, Treal, amp_real, amp_lut, norm, inc_amp, max_loops, tolerance, hologram_out, &ra, &ca));
+    SLM_TRY(upload_lenses(c, planes, defocus));
+    ra.B = holograms; ra.planes = planes; ra.lens_y = c->lens_y; ra.lens_x = c->lens_x;
+    for (int k = 0; k < planes; ++k)
+        if (defocus[k] != 0.0) ra.lens_mask |= 1 << k;
+    return gs_loop(c, holograms * planes, false, ra, ca, T8, amp_real, phasor0, setup_c64, expected_out);
 }
 
 extern "C" int slm_gd_run(slm_ctx* c, int batch, const uint8_t* T8, const void* Treal, const void* mask_real,

@@ -7,8 +7,9 @@ namespace slm {
 
 enum Precision { PREC_F32 = 0, PREC_F64 = 1 };
 // ALG_GSW: weighted GS (per-pixel amplitude feedback, DESIGN.md); ALG_GSW_STATS selects its iteration-0 pre-pass
-// (col_gsw_stats_kernel) in LineTable::col_pass
-enum Algorithm { ALG_GS = 0, ALG_GD = 1, ALG_GSW = 2, ALG_GSW_STATS = 3 };
+// (col_gsw_stats_kernel) in LineTable::col_pass.  ALG_MP: the SLM-plane pass of multi-plane GS (row_multiplane_kernel)
+// in LineTable::row_pass; its Fourier-plane side is GS's.
+enum Algorithm { ALG_GS = 0, ALG_GD = 1, ALG_GSW = 2, ALG_GSW_STATS = 3, ALG_MP = 4 };
 
 // ---- per-plane loop state, device resident --------------------------------------------------
 // Written only by the last column tile of a plane to finish a Fourier-plane pass.
@@ -49,6 +50,13 @@ struct RowArgs {
     const PlaneStats* stats;
     double* hologram;        // [B][H][W], final pass
     const void* tw;          // complex<R> [W] row twiddles exp(-2 pi i q / W)
+    // multi-plane GS (ALG_MP); appended so that the offsets the other kernels read stay where they were.  B counts
+    // holograms, plane k of hologram g is plane g * planes + k of Y, X and stats; field (ROW_FROM_FIELD) and hologram
+    // hold one plane per hologram.
+    int planes;              // K, 1..8
+    int lens_mask;           // bit k: plane k has a defocus (alpha_k != 0); a clear bit skips the products with L_k
+    const void* lens_y;      // complex<R> [K][H]: exp(i alpha_k (y - H/2)^2)
+    const void* lens_x;      // complex<R> [K][W]: exp(i alpha_k (x - W/2)^2);  L_k(y, x) = lens_y[k][y] * lens_x[k][x]
 };
 
 // ---- Fourier-plane (column) pass -----------------------------------------------------------------

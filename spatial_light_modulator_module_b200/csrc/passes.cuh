@@ -197,6 +197,9 @@ template <typename R, int L> struct RowGeom {
     // (<= 128 registers) for the 32-point long lines
     static constexpr int BUDGET = P::E == 32 ? 512 : SLM_ROW_THREADS_PER_SM;
     static constexpr int MIN_CTAS = sizeof(R) == 4 ? (BUDGET / THREADS > 0 ? BUDGET / THREADS : 1) : 1;
+    // the multi-plane row pass holds the field sum S[E] beside the plane being transformed: 512 threads (<= 128
+    // registers) in fp32
+    static constexpr int MP_MIN_CTAS = sizeof(R) == 4 ? (512 / THREADS > 0 ? 512 / THREADS : 1) : 1;
     // rows are transformed independently: the threads of LPG rows (whole warps) share a named barrier
     static constexpr int LPG = M % 32 == 0 ? 1 : (M % 16 == 0 ? 2 : (M % 8 == 0 ? 4 : 8));
     static constexpr int GROUPS = NR / LPG;
@@ -320,6 +323,123 @@ SLM_GLOBAL void SLM_LAUNCH_BOUNDS((RowGeom<R, W>::THREADS), (RowGeom<R, W>::MIN_
     cpx<R>* X = static_cast<cpx<R>*>(a.X) + base;
 #pragma unroll
     for (int r = 0; r < E; ++r) st_plane(X + r * M, v[r]);
+}
+
+// ---- multi-plane SLM-plane pass ------------------------------------------------------------------
+// Multi-plane GS (Haist et al., Opt. Commun. 140, 299 (1997)): K target planes at defocus L_k = exp(i alpha_k rho^2)
+// share one hologram.  Their Fourier-plane steps are K planes of GS's column pass; this pass joins them.  A CTA takes
+// NR rows of hologram g and, plane by plane (b = g K + k), finishes the inverse transform, takes off the defocus and
+// adds the field into S[E]:  S = sum_k ifft2(D_k) conj(L_k).  Then B = inc exp(i angle(S)), and per plane the rows of
+// B L_k are forward-transformed into X.  FINAL = 1 writes angle(S) to the hologram instead.
+// Other sources: ROW_FROM_A32 / ROW_FROM_A sum the setup's A_k (already transformed) the same way; ROW_FROM_FIELD
+// takes B of iteration 0 from `field` (one plane per hologram).
+// K = 1 with alpha = 0 is GS's arithmetic: S starts from the first term (not 0 + term), a plane without defocus is not
+// multiplied, and the phasor and `inc` are applied as row_pass_kernel applies them.
+// Loop condition: each plane's column pass closes with its own `done`; a hologram iterates while any of its planes
+// has not converged.  All flags set: return; otherwise every CTA of the hologram clears them (all CTAs decide alike,
+// in any order: a flag that was clear stays clear), so the planes keep iterating together and their curves stay
+// equal in length.
+template <typename R, int W, int FINAL>
+SLM_GLOBAL void SLM_LAUNCH_BOUNDS((RowGeom<R, W>::THREADS), (RowGeom<R, W>::MP_MIN_CTAS)) row_multiplane_kernel(RowArgs a) {
+    using G = RowGeom<R, W>;
+    using P = FftPlan<W>;
+    constexpr int E = P::E, M = P::M;
+    SLM_DYN_SMEM(raw);
+    const int t = threadIdx.x, rr = t / M, j = t % M;
+    const long long grow = (long long)blockIdx.x * G::NR + rr;
+    const int g = (int)(grow / a.H), y = (int)(grow % a.H);
+    const int K = a.planes;
+    griddep_launch();
+    griddep_wait();
+    if (!FINAL) {
+        // (the PlaneStats of the context, handed over as const for the single-plane passes)
+        PlaneStats* st = const_cast<PlaneStats*>(a.stats) + (size_t)g * K;
+        bool all = true;
+        for (int k = 0; k < K; ++k) all = all && ld_cg(&st[k].done) != 0;
+        if (all) return;                              // uniform: a CTA never straddles holograms
+        if (t == 0)
+            for (int k = 0; k < K; ++k) st[k].done = 0;
+    }
+    cpx<R>* line = reinterpret_cast<cpx<R>*>(raw) + (size_t)rr * P::NP;
+    const typename G::Sync sync{1 + rr / G::LPG};
+    const cpx<R>* tw = static_cast<const cpx<R>*>(a.tw);
+    const cpx<R>* ly = static_cast<const cpx<R>*>(a.lens_y);
+    const cpx<R>* lx = static_cast<const cpx<R>*>(a.lens_x) + j;
+    const size_t plane = (size_t)a.H * W, pix = (size_t)y * W + j;
+    const size_t gbase = (size_t)g * plane + pix;                   // one plane per hologram (field, hologram)
+    const size_t kbase = (size_t)g * K * plane + pix;               // plane 0 of the hologram's K planes
+    const R* inc = static_cast<const R*>(a.inc);
+    cpx<R> s[E], v[E];
+
+    if (a.source == ROW_FROM_FIELD) {
+        const cpx<R>* F = static_cast<const cpx<R>*>(a.field) + gbase;
+#pragma unroll
+        for (int r = 0; r < E; ++r) s[r] = ld_plane(F + r * M);
+    } else if (a.source == ROW_FROM_A32 && K == 1 && !(a.lens_mask & 1)) {
+        // GS's first phasor, in complex64 (row_pass_kernel)
+        const cpx<float>* A = static_cast<const cpx<float>*>(a.A32) + kbase;
+#pragma unroll
+        for (int r = 0; r < E; ++r) {
+            cpx<float> z = ld_plane(A + r * M);
+            if (!FINAL) z = unit_phasor(z);
+            s[r].x = (R)z.x; s[r].y = (R)z.y;
+        }
+    } else {
+        for (int k = 0; k < K; ++k) {
+            const size_t off = kbase + (size_t)k * plane;
+            if (a.source == ROW_FROM_Y) {
+                const cpx<R>* Y = static_cast<const cpx<R>*>(a.Y) + off;
+#pragma unroll
+                for (int r = 0; r < E; ++r) v[r] = ld_plane(Y + r * M);
+                line_fft<R, W, +1, 1>(v, line, j, tw, sync);       // A_k = ifft2(D_k) up to a positive scale
+            } else if (a.source == ROW_FROM_A32) {
+                const cpx<float>* A = static_cast<const cpx<float>*>(a.A32) + off;
+#pragma unroll
+                for (int r = 0; r < E; ++r) { const cpx<float> z = ld_plane(A + r * M); v[r].x = (R)z.x; v[r].y = (R)z.y; }
+            } else {
+                const cpx<R>* A = static_cast<const cpx<R>*>(a.field) + off;
+#pragma unroll
+                for (int r = 0; r < E; ++r) v[r] = ld_plane(A + r * M);
+            }
+            if (a.lens_mask & (1 << k)) {
+                const cpx<R> cy = ld_const(ly + (size_t)k * a.H + y);
+#pragma unroll
+                for (int r = 0; r < E; ++r) v[r] = cmul(v[r], cconj(cmul(cy, ld_const(lx + (size_t)k * W + r * M))));
+            }
+#pragma unroll
+            for (int r = 0; r < E; ++r) s[r] = k ? cadd(s[r], v[r]) : v[r];
+        }
+        if (!FINAL) {
+            if (a.source == ROW_FROM_Y) unit_phasors<E>(s);
+            else {
+#pragma unroll
+                for (int r = 0; r < E; ++r) s[r] = unit_phasor(s[r]);
+            }
+        }
+    }
+    if (FINAL) {                                       // hologram = angle(S)
+        double* h = a.hologram + gbase;
+#pragma unroll
+        for (int r = 0; r < E; ++r) h[r * M] = atan2((double)s[r].y, (double)s[r].x);
+        return;
+    }
+    if (inc && a.source != ROW_FROM_FIELD) {
+#pragma unroll
+        for (int r = 0; r < E; ++r) s[r] = cscale(s[r], ld_ro(inc + pix + r * M));
+    }
+    for (int k = 0; k < K; ++k) {                      // X_k = rows of fft2(B L_k)
+#pragma unroll
+        for (int r = 0; r < E; ++r) v[r] = s[r];
+        if (a.lens_mask & (1 << k)) {
+            const cpx<R> cy = ld_const(ly + (size_t)k * a.H + y);
+#pragma unroll
+            for (int r = 0; r < E; ++r) v[r] = cmul(v[r], cmul(cy, ld_const(lx + (size_t)k * W + r * M)));
+        }
+        line_fft<R, W, -1, 1>(v, line, j, tw, sync);
+        cpx<R>* X = static_cast<cpx<R>*>(a.X) + kbase + (size_t)k * plane;
+#pragma unroll
+        for (int r = 0; r < E; ++r) st_plane(X + r * M, v[r]);
+    }
 }
 
 // ---- Fourier-plane pass ---------------------------------------------------------------------------

@@ -30,6 +30,15 @@ class LoopResult:
     iterations: np.ndarray           # int [B]
 
 
+@dataclass
+class MultiplaneResult:
+    """Results of a multi-plane GS run of G holograms with K target planes each (device buffers unless converted)."""
+    hologram: object                 # [G,H,W] float64: angle(A)
+    expected: Optional[object]       # [G,K,H,W] float64 or None: each plane's expected outcome
+    errors: List[List[np.ndarray]]   # errors[g][k]: error_evolution of plane k; the K curves of a hologram have one length
+    iterations: np.ndarray           # int [G]
+
+
 class Engine:
     """Device context for planes of one shape.
 
@@ -245,14 +254,14 @@ class Engine:
     # what _begin hands a run: the targets (fields of _targets), the illumination and the result buffers
     _Begun = namedtuple("_Begun", "batch t8 treal amp norms c64 inc hologram expected")
 
-    def _begin(self, targets, max_loops, unbound, inc_amp, norms, want_expected):
-        """What gs, gsw and gd do first.  ``unbound``: the reference's variable that a run without iterations
-        leaves unbound."""
+    def _begin(self, targets, max_loops, unbound, inc_amp, norms, want_expected, holograms=None):
+        """What gs, gsw, gs_multiplane and gd do first.  ``unbound``: the reference's variable that a run without
+        iterations leaves unbound.  ``holograms``: hologram planes to allocate (default: one per target plane)."""
         if max_loops < 1:
             raise UnboundLocalError(f"cannot access local variable '{unbound}' where it is not associated with a value")
         batch, t8, treal, amp, norms, c64 = self._targets(targets, norms)
         inc_dev = self._as_device(inc_amp, self.real_dtype, "inc_amp")
-        holo = self._mem_empty((batch,) + self.shape, np.float64)
+        holo = self._mem_empty((holograms or batch,) + self.shape, np.float64)
         exp = self._mem_empty((batch,) + self.shape, np.float64) if want_expected else None
         return self._Begun(batch, t8, treal, amp, norms, c64, inc_dev, holo, exp)
 
@@ -299,6 +308,46 @@ class Engine:
         res = self._gs_run(self._lib.slm_gsw_run, b, phasor0, max_loops, tolerance,
                            self._dp(sums), self._mem_ptr(w), float(weight_limit))
         return res, w
+
+    def gs_multiplane(self, targets, defocus, max_loops: int, tolerance: float = 0.0, inc_amp=None, phasor0=None,
+                      want_expected: bool = True, norms=None) -> MultiplaneResult:
+        """Multi-plane GS (include/slm_holo.h slm_gs_multiplane_run): one hologram for K target planes at different
+        focus.  ``targets``: [K,H,W] (one hologram) or [G,K,H,W]; ``defocus``: K coefficients alpha_k [rad / pixel^2]
+        shared by the holograms (host_logic.defocus_coefficient; 0 = the Fourier plane), each with |alpha_k| max(H, W)
+        <= pi.  A hologram iterates while any of its planes' error is above ``tolerance``.  ``phasor0``: B of
+        iteration 0, [G,H,W].  K = 1 with alpha = 0 gives :meth:`gs`'s results bit for bit."""
+        shape = tuple(int(s) for s in targets.shape) if hasattr(targets, "shape") else np.shape(targets)
+        if len(shape) not in (3, 4):
+            raise ValueError(f"targets must be [K,H,W] or [G,K,H,W], not of shape {tuple(shape)}")
+        g, k = (1, shape[0]) if len(shape) == 3 else shape[:2]
+        alpha = np.ascontiguousarray(np.asarray(defocus, dtype=np.float64).reshape(-1))
+        if max_loops >= 1:                                            # (max_loops < 1 raises first, in _begin)
+            if alpha.shape != (k,):
+                raise ValueError(f"{k} target planes need {k} defocus coefficients, not {alpha.size}")
+            if not 1 <= k <= 8:
+                raise ValueError(f"multi-plane GS takes 1 to 8 target planes, not {k}")
+            if g * k > self.max_batch:
+                raise ValueError(f"{g} holograms of {k} planes exceed the engine's max_batch ({self.max_batch})")
+            from . import constants
+            hl.check_defocus(alpha, self.shape, constants.px_distance, constants.wavelength)
+        flat = targets.reshape((g * k,) + tuple(shape[-2:])) if self._mem_is_device(targets) else \
+            np.asarray(targets).reshape((g * k,) + tuple(shape[-2:]))
+        b = self._begin(flat, max_loops, "expected_outcome", inc_amp, norms, want_expected, holograms=g)
+        ph_dev = self._as_device(phasor0, self.complex_dtype, "phasor0")
+        if ph_dev is not None:
+            if tuple(ph_dev.shape) == self.shape and g == 1:
+                ph_dev = ph_dev.reshape((1,) + self.shape)
+            if tuple(ph_dev.shape) != (g,) + self.shape:
+                raise ValueError(f"phasor0 must have shape {(g,) + self.shape}, not {tuple(ph_dev.shape)}")
+        amp_dev = self._mem_upload(b.amp.astype(self.real_dtype)) if b.amp is not None else None
+        self._check(self._lib.slm_gs_multiplane_run(
+            self._ctx, g, k, self._mem_ptr(b.t8), self._mem_ptr(b.treal), self._mem_ptr(amp_dev), self._dp(self._amp_lut),
+            self._dp(b.norms), self._dp(alpha), self._mem_ptr(b.inc), self._mem_ptr(ph_dev), int(b.c64), int(max_loops),
+            float(tolerance), self._mem_ptr(b.hologram), self._mem_ptr(b.expected)))
+        res = self._collect(b.batch, max_loops, b.hologram, b.expected)
+        expected = None if b.expected is None else b.expected.reshape((g, k) + self.shape)
+        return MultiplaneResult(b.hologram, expected, [res.errors[i * k:(i + 1) * k] for i in range(g)],
+                                res.iterations[::k].copy())
 
     # ---- gradient descent (algorithms.py:60-112) --------------------------------------------------------
     def gd(self, targets, x0, lr_schedule, max_loops: int, tolerance: float = 0.0, white_attention=1,

@@ -153,6 +153,30 @@ def lens_scalars(focal_length, wavelength):
     return float(2 * np.pi * focal_length / wavelength), float(focal_length ** 2)
 
 
+def defocus_coefficient(focal_length, px_distance, wavelength) -> float:
+    """Multi-plane GS: alpha = -pi px^2 / (lambda f) [rad / pixel^2], the paraxial form of the reference's ``lens(f)``
+    (generate_hologram.py:189-203, phase k (1 - sqrt(1 + r^2/f^2)) ~ -pi r^2 / (lambda f)): the target plane that
+    ``add_lens(hologram, f)`` brings into focus.  f = None or infinite: 0, the Fourier plane."""
+    if focal_length is None or np.isinf(focal_length):
+        return 0.0
+    return float(-np.pi * px_distance ** 2 / (wavelength * focal_length))
+
+
+def check_defocus(alphas, shape, px_distance, wavelength) -> None:
+    """Multi-plane GS: refuse a defocus that aliases.  The phase alpha rho^2 steps by |alpha| max(H, W) per pixel at the
+    plane's edge; above pi the sampled lens is a different lens.  The message names the plane and the shortest focal
+    length allowed at ``px_distance`` and ``wavelength``."""
+    n = max(shape)
+    for k, a in enumerate(alphas):
+        if not np.isfinite(a):
+            raise ValueError(f"defocus of plane {k} is not finite: {a!r}")
+        if abs(a) * n > np.pi:
+            f_min = px_distance ** 2 * n / wavelength
+            raise ValueError(f"the defocus of plane {k} aliases: its phase steps by |alpha| * max(H, W) = {abs(a) * n:.4g} rad "
+                             f"per pixel at the edge of a {shape[0]}x{shape[1]} plane (at most pi); the shortest focal length "
+                             f"allowed is |f| >= {f_min:.3g} m (pixel pitch {px_distance:g} m, wavelength {wavelength:g} m)")
+
+
 # --------------------------------------------------------------------------------------------
 # frame sharding (generate_hologram_sequence over ranks)
 # --------------------------------------------------------------------------------------------
