@@ -126,6 +126,33 @@ int slm_gd_run(slm_ctx* ctx, int batch, const uint8_t* target_u8, const void* ta
 int slm_fourier_guess(slm_ctx* ctx, int batch, const uint8_t* target_u8, const void* amp_real, const double* amp_lut,
                       const void* inc_amp, int setup_c64, void* x_out);
 
+/* Multi-plane gradient descent: one phase hologram for K target planes at different focus (plane k and L_k as in
+ * slm_gs_multiplane_run), by gradient descent on the mean of the planes' errors.  Each iteration:
+ *     B = x/|x| inc;  per plane F_k = fft2(B L_k), out_k = |F_k|^2 norm_k / max |F_k|^2,
+ *                     G_k = ifft2(mask_k F_k (out_k - T_k)), error and expected outcome of plane k as GD's
+ *     dEdF = (sum_k G_k conj(L_k)) inc / K;  x -= lr_i dEdX_complex(dEdF, x)
+ *     hologram   angle(x) after the last update
+ * A hologram iterates until the error of EVERY one of its planes is <= tolerance (or max_loops); the update of the
+ * iteration that ends the loop is applied.  planes = 1 with alpha = 0 runs slm_gd_run's passes: its results, bit for bit.
+ * Arguments as slm_gd_run, with the batch made of `holograms` x `planes` planes (g*planes + k), and as
+ * slm_gs_multiplane_run for holograms, planes and defocus (same refusals):
+ *   target_u8 / target_real / mask_real / norm / expected_out   per plane
+ *   x              device complex<R> [holograms][H][W]: one initial guess per hologram, updated in place
+ *   lr_schedule    host double[max_loops], shared by the holograms
+ *   hologram_out   device double [holograms][H][W]
+ * Error curves: slm_read_curves over holograms * planes planes. */
+int slm_gd_multiplane_run(slm_ctx* ctx, int holograms, int planes, const uint8_t* target_u8, const void* target_real,
+                          const void* mask_real, const double* mask_lut, const double* norm, const double* defocus,
+                          const void* inc_amp, void* x, const double* lr_schedule, int max_loops, double tolerance,
+                          double* hologram_out, double* expected_out);
+
+/* "fourier" initial guess of multi-plane GD: x = inc exp(i angle(sum_k ifft2(sqrt(T_k)) conj(L_k))), the setup sum of
+ * slm_gs_multiplane_run (ifft2 as slm_fourier_guess's).  Arguments as slm_fourier_guess per plane, and holograms,
+ * planes, defocus as slm_gs_multiplane_run (same refusals); x_out: device complex<R> [holograms][H][W]. */
+int slm_multiplane_fourier_guess(slm_ctx* ctx, int holograms, int planes, const uint8_t* target_u8, const void* amp_real,
+                                 const double* amp_lut, const double* defocus, const void* inc_amp, int setup_c64,
+                                 void* x_out);
+
 /* make_initial_guess("random" | "zeros", ...) -- algorithms.py:118-124,145-151: exp(1j*2*pi*u) / divide_by
  * from the MT19937 stream `u` (device double[n], drawn on the host exactly as random.random() does);
  * x_out: device complex<R>[n]. */

@@ -37,6 +37,8 @@ SIGNATURES = {
     "slm_gs_multiplane_run": (_i, [_vp, _i, _i, _vp, _vp, _vp, _dp, _dp, _dp, _vp, _vp, _i, _i, _d, _vp, _vp]),
     "slm_gd_run": (_i, [_vp, _i, _vp, _vp, _vp, _dp, _dp, _vp, _vp, _dp, _i, _d, _vp, _vp]),
     "slm_fourier_guess": (_i, [_vp, _i, _vp, _vp, _dp, _vp, _i, _vp]),
+    "slm_gd_multiplane_run": (_i, [_vp, _i, _i, _vp, _vp, _vp, _dp, _dp, _dp, _vp, _vp, _dp, _i, _d, _vp, _vp]),
+    "slm_multiplane_fourier_guess": (_i, [_vp, _i, _i, _vp, _vp, _dp, _dp, _vp, _i, _vp]),
     "slm_random_phasor": (_i, [_vp, _vp, _vp, _ll, _d]),
     "slm_mt19937_uniform": (_i, [_vp, _vp, _i, _vp, _ll, _vp]),
     "slm_phase_phasor": (_i, [_vp, _vp, _vp, _vp, _ll, _ll]),

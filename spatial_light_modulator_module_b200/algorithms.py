@@ -23,8 +23,9 @@ import numpy as np
 from . import constants, host_logic as hl
 from .engine import Engine, get_engine
 
-__all__ = ["gerchberg_saxton", "weighted_gerchberg_saxton", "multiplane_gerchberg_saxton", "gradient_descent", "make_initial_guess", "error_f", "printout",
-           "complex_to_real_phase", "dEdX_complex", "add_gif_image"]
+__all__ = ["gerchberg_saxton", "weighted_gerchberg_saxton", "multiplane_gerchberg_saxton", "gradient_descent",
+           "multiplane_gradient_descent", "make_initial_guess", "error_f", "printout", "complex_to_real_phase", "dEdX_complex",
+           "add_gif_image"]
 
 
 def _precision(args) -> str:
@@ -118,8 +119,22 @@ def multiplane_gerchberg_saxton(demanded_outputs, focal_lengths, args):
     above ``args.tolerance``).  Lenses use the paraxial phase -pi r^2 / (lambda f) at the pixel pitch and wavelength of
     ``constants``; a focal length short enough to alias at the plane's edge is refused (ValueError), as are
     ``args.gif``, an all-zero target image and a count of focal lengths other than K."""
+    targets, focal_lengths = _multiplane_targets("multiplane_gerchberg_saxton", demanded_outputs, focal_lengths, args)
+    inc = _illumination(args, targets.shape[1:])
+    if args.max_loops < 1 or not (args.tolerance + 1 > args.tolerance):
+        print()
+        raise UnboundLocalError("cannot access local variable 'expected_outcome' where it is not associated with a value")
+    alphas = _alphas(focal_lengths)
+    eng = _engine(targets.shape[1:], args, batch=len(targets))
+    res = eng.gs_multiplane(targets, alphas, int(args.max_loops), float(args.tolerance), inc_amp=inc)
+    return _multiplane_report(args, eng, res)
+
+
+def _multiplane_targets(name, demanded_outputs, focal_lengths, args):
+    """The multi-plane drop-ins' refusals (``name`` in the messages) -> (targets as one [K,H,W] array, focal lengths
+    as a list)."""
     if getattr(args, "gif", False):
-        raise ValueError("multiplane_gerchberg_saxton does not offer GIF snapshots (args.gif)")
+        raise ValueError(f"{name} does not offer GIF snapshots (args.gif)")
     targets = np.stack([np.asarray(t) for t in demanded_outputs])
     focal_lengths = list(focal_lengths)
     if len(focal_lengths) != len(targets):
@@ -127,13 +142,16 @@ def multiplane_gerchberg_saxton(demanded_outputs, focal_lengths, args):
     for k, t in enumerate(targets):
         if not np.any(t):
             raise ValueError(f"target image {k} is all zero: it has no intensity to place")
-    inc = _illumination(args, targets.shape[1:])
-    if args.max_loops < 1 or not (args.tolerance + 1 > args.tolerance):
-        print()
-        raise UnboundLocalError("cannot access local variable 'expected_outcome' where it is not associated with a value")
-    alphas = [hl.defocus_coefficient(f, constants.px_distance, constants.wavelength) for f in focal_lengths]
-    eng = _engine(targets.shape[1:], args, batch=len(targets))
-    res = eng.gs_multiplane(targets, alphas, int(args.max_loops), float(args.tolerance), inc_amp=inc)
+    return targets, focal_lengths
+
+
+def _alphas(focal_lengths):
+    return [hl.defocus_coefficient(f, constants.px_distance, constants.wavelength) for f in focal_lengths]
+
+
+def _multiplane_report(args, eng, res):
+    """The multi-plane drop-ins' epilogue: (hologram, expected[K,H,W], [errors_k]) on the host, progress line, and
+    the reference's printout per plane with ``args.print_info``."""
     hologram, expected = (a[0] for a in eng.to_host_many([res.hologram, res.expected]))
     errors = [[np.float64(e) for e in curve] for curve in res.errors[0]]
     _progress(len(errors[0]), args.max_loops)
@@ -170,6 +188,41 @@ def gradient_descent(demanded_output, args):
         hologram, expected, errors = _to_host(eng, chunk(int(args.max_loops), 0))
     args.learning_rate = after[len(errors)]
     return _report(args, hologram, expected, errors)
+
+
+def multiplane_gradient_descent(demanded_outputs, focal_lengths, args):
+    """Multi-plane gradient descent: one phase hologram for several target images, image k in focus where
+    ``add_lens(hologram, focal_lengths[k])`` would bring the Fourier plane (None or inf: the Fourier plane itself) --
+    :func:`gradient_descent` for traps in 3-D.  It descends on the mean of the planes' errors, so
+    ``args.learning_rate`` means what it means for one plane.  Arguments as :func:`gradient_descent`
+    (``initial_guess``, ``random_seed``, ``learning_rate``, ``unsettle``, ``white_attention``,
+    ``incomming_intensity``; one initial guess for the hologram, "fourier" being taken from the sum of the planes'
+    setup fields as multi-plane GS takes it), targets and focal lengths as :func:`multiplane_gerchberg_saxton`, with its
+    refusals.  Returns ``(hologram, expected[K,H,W], [errors_k])``, every curve of the same length (the loop runs while
+    any plane's error is above ``args.tolerance``); ``args.learning_rate`` is updated as :func:`gradient_descent`
+    updates it.  One plane with focal length None gives :func:`gradient_descent`'s results bit for bit, except from
+    the "fourier" guess, whose phase is taken through the multi-plane setup sum."""
+    targets, focal_lengths = _multiplane_targets("multiplane_gradient_descent", demanded_outputs, focal_lengths, args)
+    alphas = _alphas(focal_lengths)
+    inc = _illumination(args, targets.shape[1:])
+    eng = _engine(targets.shape[1:], args, batch=len(targets))
+    if args.initial_guess == "fourier":
+        hl.host_initial_guess("fourier", targets.shape[1:], args.random_seed)     # seeds `random` as make_initial_guess does
+        x = eng.multiplane_fourier_guess(targets, alphas, inc)
+    else:
+        inc_amp = np.float64(1.0) if inc is None else inc
+        x = make_initial_guess(args.initial_guess, inc_amp, targets[0], args.random_seed, _engine_hint=eng, _device=True)
+    if args.print_info:
+        print("computing hologram")
+    if args.max_loops < 1 or not (args.tolerance + 1 > args.tolerance):
+        print()
+        raise UnboundLocalError("cannot access local variable 'output' where it is not associated with a value")
+    during, after = hl.learning_rate_schedule(args.learning_rate, args.unsettle, int(args.max_loops))
+    res, _ = eng.gd_multiplane(targets, alphas, x, during, int(args.max_loops), float(args.tolerance),
+                               white_attention=args.white_attention, inc_amp=inc)
+    out = _multiplane_report(args, eng, res)
+    args.learning_rate = after[len(out[2][0])]
+    return out
 
 
 def make_initial_guess(initial_guess_type, incomming_amplitude, demanded_output, seed, _engine_hint=None, _device=False):

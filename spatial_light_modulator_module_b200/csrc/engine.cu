@@ -773,44 +773,55 @@ static int upload_lenses(slm_ctx* c, int planes, const double* alpha) {
     return 0;
 }
 
+// The multi-plane entry points' own refusals (after the context): `planes` outside 1..kMaxPlanes and `holograms` x
+// `planes` above the context's batch fail at once; a missing or non-finite defocus, or a rows-only context, is left
+// in `refused` for begin_loop, which names the entry point.
+static int check_multiplane(slm_ctx* c, const std::string& who, int holograms, int planes, const double* defocus,
+                            std::string* refused) {
+    if (!c) return fail(SLM_ERR_ARG, who + ": null context");
+    if (planes < 1 || planes > kMaxPlanes) return fail(SLM_ERR_ARG, who + ": planes must be in 1.." + std::to_string(kMaxPlanes));
+    if (holograms < 1 || (long long)holograms * planes > c->max_batch)
+        return fail(SLM_ERR_ARG, who + ": holograms * planes must be in 1..max_batch of the context");
+    if (!defocus) *refused = "defocus is required";
+    for (int k = 0; defocus && k < planes && refused->empty(); ++k)
+        if (!std::isfinite(defocus[k])) *refused = "defocus[" + std::to_string(k) + "] is not finite";
+    if (refused->empty() && c->row && c->row->rows_only) *refused = "no multi-plane pass for rows of " + std::to_string(c->W) + " points";
+    return 0;
+}
+
+// The defocus tables and the multi-plane fields of the row arguments: ra.B counts holograms from here on.
+static int multiplane_rows(slm_ctx* c, RowArgs& ra, int holograms, int planes, const double* defocus) {
+    SLM_TRY(upload_lenses(c, planes, defocus));
+    ra.B = holograms; ra.planes = planes; ra.lens_y = c->lens_y; ra.lens_x = c->lens_x;
+    for (int k = 0; k < planes; ++k)
+        if (defocus[k] != 0.0) ra.lens_mask |= 1 << k;
+    return 0;
+}
+
 extern "C" int slm_gs_multiplane_run(slm_ctx* c, int holograms, int planes, const uint8_t* T8, const void* Treal,
                                      const void* amp_real, const double* amp_lut, const double* norm, const double* defocus,
                                      const void* inc_amp, const void* phasor0, int setup_c64, int max_loops, double tolerance,
                                      double* hologram_out, double* expected_out) {
     const std::string who = "slm_gs_multiplane_run";
-    if (!c) return fail(SLM_ERR_ARG, who + ": null context");
-    if (planes < 1 || planes > kMaxPlanes) return fail(SLM_ERR_ARG, who + ": planes must be in 1.." + std::to_string(kMaxPlanes));
-    if (holograms < 1 || (long long)holograms * planes > c->max_batch)
-        return fail(SLM_ERR_ARG, who + ": holograms * planes must be in 1..max_batch of the context");
     std::string refused;
-    if (!defocus) refused = "defocus is required";
-    for (int k = 0; defocus && k < planes && refused.empty(); ++k)
-        if (!std::isfinite(defocus[k])) refused = "defocus[" + std::to_string(k) + "] is not finite";
-    if (refused.empty() && c->row && c->row->rows_only) refused = "no multi-plane pass for rows of " + std::to_string(c->W) + " points";
+    SLM_TRY(check_multiplane(c, who, holograms, planes, defocus, &refused));
     RowArgs ra; ColArgs ca;
     SLM_TRY(begin_loop(c, holograms * planes, who.c_str(), "max_loops must be >= 1 (the reference raises UnboundLocalError for 0)",
                        norm && hologram_out, "norm and hologram_out", "give target_u8 + amp_lut, or target_real + amp_real",
                        refused.empty() ? nullptr : refused.c_str(),
                        T8, Treal, amp_real, amp_lut, norm, inc_amp, max_loops, tolerance, hologram_out, &ra, &ca));
-    SLM_TRY(upload_lenses(c, planes, defocus));
-    ra.B = holograms; ra.planes = planes; ra.lens_y = c->lens_y; ra.lens_x = c->lens_x;
-    for (int k = 0; k < planes; ++k)
-        if (defocus[k] != 0.0) ra.lens_mask |= 1 << k;
+    SLM_TRY(multiplane_rows(c, ra, holograms, planes, defocus));
     return gs_loop(c, holograms * planes, false, ra, ca, T8, amp_real, phasor0, setup_c64, expected_out);
 }
 
-extern "C" int slm_gd_run(slm_ctx* c, int batch, const uint8_t* T8, const void* Treal, const void* mask_real,
-                          const double* mask_lut, const double* norm, const void* inc_amp, void* x,
-                          const double* lr_schedule, int max_loops, double tolerance, double* hologram_out,
-                          double* expected_out) {
-    RowArgs ra; ColArgs ca;
-    SLM_TRY(begin_loop(c, batch, "slm_gd_run", "max_loops must be >= 1 (the reference raises UnboundLocalError for 0)",
-                       norm && hologram_out && x && lr_schedule, "norm, x, lr_schedule and hologram_out",
-                       "give target_u8 + mask_lut, or target_real + mask_real", nullptr,
-                       T8, Treal, mask_real, mask_lut, norm, inc_amp, max_loops, tolerance, hologram_out, &ra, &ca));
-    SLM_CUDA(cudaMemcpyAsync(c->lr, lr_schedule, (size_t)max_loops * sizeof(double), cudaMemcpyHostToDevice, c->stream));
-    ra.x = x; ra.lr = c->lr; ra.source = ROW_FROM_FIELD;
-    SLM_TIMED(K_ROW_PASS, c->row->row_pass(ALG_GD, ra, c->stream));
+// GD and multi-plane GD after begin_loop, with ra.x and ra.lr set: the first pass, the choice of the Fourier-plane form,
+// the loop and the expected outcome.  Multi-plane GD (ra.planes > 0) is GD with the multi-plane row pass (ALG_MPGD):
+// `batch` counts planes, ra.B holograms; its kept graphs have families of their own.
+static int gd_loop(slm_ctx* c, int batch, RowArgs& ra, ColArgs& ca, double* expected_out) {
+    const bool multiplane = ra.planes > 0;
+    const int row_alg = multiplane ? ALG_MPGD : ALG_GD;
+    ra.source = ROW_FROM_FIELD;
+    SLM_TIMED(K_ROW_PASS, c->row->row_pass(row_alg, ra, c->stream));
     // The fused pass saves a launch and a trip of the field through L2/HBM per iteration, but its CTAs wait for each
     // other once per plane and it leaves the SMs beyond a whole number of planes idle: measured faster for a few
     // planes (latency bound: 2.9 vs 3.3 ms per 100-iteration hologram), slower for a large batch (47.9 vs 46.4 ms).
@@ -826,7 +837,8 @@ extern "C" int slm_gd_run(slm_ctx* c, int batch, const uint8_t* T8, const void* 
     }
     // two-pass form without the column groups: the max pass keeps the transformed field in X (below)
     if (!c->use_groups) ca.skip_forward = 1;
-    SLM_TRY(run_loop(c, batch, fused ? "gdf" : (pipe ? "gdp" : "gd2"), ALG_GD, ra, ca, [&]() -> int {
+    const char* family = multiplane ? (fused ? "mgdf" : (pipe ? "mgdp" : "mgd2")) : (fused ? "gdf" : (pipe ? "gdp" : "gd2"));
+    SLM_TRY(run_loop(c, batch, family, row_alg, ra, ca, [&]() -> int {
         if (fused) {
             // one Fourier-plane pass: the tiles of a plane agree on amax(output_unnormed) (algorithms.py:86) between
             // their forward transforms and the gradient step
@@ -858,6 +870,45 @@ extern "C" int slm_gd_run(slm_ctx* c, int batch, const uint8_t* T8, const void* 
     return 0;
 }
 
+extern "C" int slm_gd_run(slm_ctx* c, int batch, const uint8_t* T8, const void* Treal, const void* mask_real,
+                          const double* mask_lut, const double* norm, const void* inc_amp, void* x,
+                          const double* lr_schedule, int max_loops, double tolerance, double* hologram_out,
+                          double* expected_out) {
+    RowArgs ra; ColArgs ca;
+    SLM_TRY(begin_loop(c, batch, "slm_gd_run", "max_loops must be >= 1 (the reference raises UnboundLocalError for 0)",
+                       norm && hologram_out && x && lr_schedule, "norm, x, lr_schedule and hologram_out",
+                       "give target_u8 + mask_lut, or target_real + mask_real", nullptr,
+                       T8, Treal, mask_real, mask_lut, norm, inc_amp, max_loops, tolerance, hologram_out, &ra, &ca));
+    SLM_CUDA(cudaMemcpyAsync(c->lr, lr_schedule, (size_t)max_loops * sizeof(double), cudaMemcpyHostToDevice, c->stream));
+    ra.x = x; ra.lr = c->lr;
+    return gd_loop(c, batch, ra, ca, expected_out);
+}
+
+extern "C" int slm_gd_multiplane_run(slm_ctx* c, int holograms, int planes, const uint8_t* T8, const void* Treal,
+                                     const void* mask_real, const double* mask_lut, const double* norm, const double* defocus,
+                                     const void* inc_amp, void* x, const double* lr_schedule, int max_loops, double tolerance,
+                                     double* hologram_out, double* expected_out) {
+    const std::string who = "slm_gd_multiplane_run";
+    std::string refused;
+    SLM_TRY(check_multiplane(c, who, holograms, planes, defocus, &refused));
+    RowArgs ra; ColArgs ca;
+    SLM_TRY(begin_loop(c, holograms * planes, who.c_str(), "max_loops must be >= 1 (the reference raises UnboundLocalError for 0)",
+                       norm && hologram_out && x && lr_schedule, "norm, x, lr_schedule and hologram_out",
+                       "give target_u8 + mask_lut, or target_real + mask_real", refused.empty() ? nullptr : refused.c_str(),
+                       T8, Treal, mask_real, mask_lut, norm, inc_amp, max_loops, tolerance, hologram_out, &ra, &ca));
+    SLM_CUDA(cudaMemcpyAsync(c->lr, lr_schedule, (size_t)max_loops * sizeof(double), cudaMemcpyHostToDevice, c->stream));
+    ra.x = x; ra.lr = c->lr;
+    // One plane at the Fourier plane is GD itself: it runs GD's row pass, so it gives GD's bits at GD's rate.  (The
+    // multi-plane pass at K = 1 ran at 0.70-0.81 of GD's plane rate, DESIGN.md §4, and its fp64 results differed
+    // from GD's in the last bit: the same arithmetic, compiled into a different kernel.)
+    if (planes > 1 || defocus[0] != 0.0) {
+        SLM_TRY(multiplane_rows(c, ra, holograms, planes, defocus));
+        // the cost is the mean of the planes' errors: dEdF = sum_k G_k conj(L_k) inc / K
+        ra.inv_hw = 1.0 / ((double)planes * c->H * c->W);
+    }
+    return gd_loop(c, holograms * planes, ra, ca, expected_out);
+}
+
 extern "C" int slm_fourier_guess(slm_ctx* c, int batch, const uint8_t* T8, const void* amp_real, const double* amp_lut,
                                  const void* inc_amp, int setup_c64, void* x_out) {
     SLM_TRY(check_batch(c, batch, "slm_fourier_guess"));
@@ -881,6 +932,31 @@ extern "C" int slm_fourier_guess(slm_ctx* c, int batch, const uint8_t* T8, const
     }
     SLM_CUDA(cudaGetLastError());
     return 0;
+}
+
+// "fourier" initial guess of multi-plane GD: x = inc exp(i angle(sum_k ifft2(amp_k) conj(L_k))), multi-plane GS's setup
+// sum.  The setup field of every plane, then the multi-plane row pass in its final form writes the phase of the sum
+// into X (G double planes fit in the context's max_batch complex planes), and slm_phase_phasor makes x of it.
+extern "C" int slm_multiplane_fourier_guess(slm_ctx* c, int holograms, int planes, const uint8_t* T8, const void* amp_real,
+                                            const double* amp_lut, const double* defocus, const void* inc_amp, int setup_c64,
+                                            void* x_out) {
+    const std::string who = "slm_multiplane_fourier_guess";
+    std::string refused;
+    SLM_TRY(check_multiplane(c, who, holograms, planes, defocus, &refused));
+    SLM_TRY(check_batch(c, holograms * planes, who.c_str()));
+    if (!refused.empty()) return fail(SLM_ERR_ARG, who + ": " + refused);
+    if (!x_out || (T8 ? !amp_lut : !amp_real)) return fail(SLM_ERR_ARG, who + ": x_out, and target_u8 + amp_lut or amp_real, are required");
+    if (T8) SLM_TRY(upload_lut(c, amp_lut));
+    RowArgs ra;
+    memset(&ra, 0, sizeof ra);
+    int src = 0;
+    SLM_TRY(setup_field(c, holograms * planes, T8, amp_real, setup_c64, &src));
+    SLM_TRY(multiplane_rows(c, ra, holograms, planes, defocus));
+    ra.H = c->H; ra.source = src; ra.A32 = c->Y; ra.field = c->Y; ra.tw = c->tw_row;
+    ra.hologram = static_cast<double*>(c->X); ra.final_pass = 1;
+    SLM_TIMED(K_ROW_PASS, c->row->row_pass(ALG_MP, ra, c->stream));
+    const long long plane = (long long)c->H * c->W;
+    return slm_phase_phasor(c, static_cast<const double*>(c->X), inc_amp, x_out, plane * holograms, plane);
 }
 
 extern "C" int slm_random_phasor(slm_ctx* c, const double* u, void* x_out, long long n, double divide_by) {

@@ -7,9 +7,9 @@ namespace slm {
 
 enum Precision { PREC_F32 = 0, PREC_F64 = 1 };
 // ALG_GSW: weighted GS (per-pixel amplitude feedback, DESIGN.md); ALG_GSW_STATS selects its iteration-0 pre-pass
-// (col_gsw_stats_kernel) in LineTable::col_pass.  ALG_MP: the SLM-plane pass of multi-plane GS (row_multiplane_kernel)
-// in LineTable::row_pass; its Fourier-plane side is GS's.
-enum Algorithm { ALG_GS = 0, ALG_GD = 1, ALG_GSW = 2, ALG_GSW_STATS = 3, ALG_MP = 4 };
+// (col_gsw_stats_kernel) in LineTable::col_pass.  ALG_MP / ALG_MPGD: the SLM-plane pass of multi-plane GS / GD
+// (row_multiplane_kernel) in LineTable::row_pass; their Fourier-plane side is GS's / GD's.
+enum Algorithm { ALG_GS = 0, ALG_GD = 1, ALG_GSW = 2, ALG_GSW_STATS = 3, ALG_MP = 4, ALG_MPGD = 5 };
 
 // ---- per-plane loop state, device resident --------------------------------------------------
 // Written only by the last column tile of a plane to finish a Fourier-plane pass.
@@ -46,13 +46,13 @@ struct RowArgs {
     void* x;                 // GD: complex<R> [B][H][W], updated in place
     const void* inc;         // real<R> [H][W] illumination amplitude or null (uniform)
     const double* lr;        // GD: learning rate of iteration k at lr[k]
-    double inv_hw;           // 1/(H*W): scipy's ifft2 normalisation (matters for GD only)
+    double inv_hw;           // 1/(H*W): scipy's ifft2 normalisation (read by GD only); multi-plane GD: 1/(K*H*W)
     const PlaneStats* stats;
     double* hologram;        // [B][H][W], final pass
     const void* tw;          // complex<R> [W] row twiddles exp(-2 pi i q / W)
-    // multi-plane GS (ALG_MP); appended so that the offsets the other kernels read stay where they were.  B counts
-    // holograms, plane k of hologram g is plane g * planes + k of Y, X and stats; field (ROW_FROM_FIELD) and hologram
-    // hold one plane per hologram.
+    // multi-plane GS and GD (ALG_MP, ALG_MPGD); appended so that the offsets the other kernels read stay where they
+    // were.  B counts holograms, plane k of hologram g is plane g * planes + k of Y, X and stats; field (ROW_FROM_FIELD),
+    // x (GD) and hologram hold one plane per hologram.
     int planes;              // K, 1..8
     int lens_mask;           // bit k: plane k has a defocus (alpha_k != 0); a clear bit skips the products with L_k
     const void* lens_y;      // complex<R> [K][H]: exp(i alpha_k (y - H/2)^2)

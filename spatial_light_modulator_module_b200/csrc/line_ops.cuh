@@ -97,14 +97,16 @@ template <typename R, int L> struct GroupLaunch<R, L, true> {
 // Row (line-contiguous) kernels: available for every line length.
 template <typename R, int L> struct RowLaunch {
     using RG = RowGeom<R, L>;
-    // multi-plane GS (row_multiplane_kernel): built where a line is 16 points per thread or fewer, i.e. not for the
-    // row-only long lines
+    // multi-plane GS and GD (row_multiplane_kernel): built where a line is 16 points per thread or fewer, i.e. not for
+    // the row-only long lines
     static constexpr bool MP = FftPlan<L>::E <= 16;
     static int check() { cudaError_t e = cudaGetLastError(); return e == cudaSuccess ? 0 : -(int)e - 1000; }
     static void prepare() {
         if constexpr (MP) {
-            cudaFuncSetAttribute(row_multiplane_kernel<R, L, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RG::SMEM);
-            cudaFuncSetAttribute(row_multiplane_kernel<R, L, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RG::SMEM);
+            cudaFuncSetAttribute(row_multiplane_kernel<R, L, ALG_MP, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RG::SMEM);
+            cudaFuncSetAttribute(row_multiplane_kernel<R, L, ALG_MP, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RG::SMEM);
+            cudaFuncSetAttribute(row_multiplane_kernel<R, L, ALG_MPGD, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RG::SMEM);
+            cudaFuncSetAttribute(row_multiplane_kernel<R, L, ALG_MPGD, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RG::SMEM);
         }
         cudaFuncSetAttribute(row_pass_kernel<R, L, ALG_GS, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RG::SMEM);
         cudaFuncSetAttribute(row_pass_kernel<R, L, ALG_GS, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RG::SMEM);
@@ -117,10 +119,13 @@ template <typename R, int L> struct RowLaunch {
     }
     static int row_pass(int alg, const RowArgs& a, cudaStream_t s) {
         const dim3 grid((unsigned)((long long)a.B * a.H / RG::NR)), block(RG::THREADS);
-        if (alg == ALG_MP) {
+        if (alg == ALG_MP || alg == ALG_MPGD) {
             if constexpr (MP) {
-                if (a.final_pass) SLM_LAUNCH_PDL((row_multiplane_kernel<R, L, 1>), grid, block, RG::SMEM, s, a);
-                else SLM_LAUNCH_PDL((row_multiplane_kernel<R, L, 0>), grid, block, RG::SMEM, s, a);
+                if (alg == ALG_MPGD) {
+                    if (a.final_pass) SLM_LAUNCH_PDL((row_multiplane_kernel<R, L, ALG_MPGD, 1>), grid, block, RG::SMEM, s, a);
+                    else SLM_LAUNCH_PDL((row_multiplane_kernel<R, L, ALG_MPGD, 0>), grid, block, RG::SMEM, s, a);
+                } else if (a.final_pass) SLM_LAUNCH_PDL((row_multiplane_kernel<R, L, ALG_MP, 1>), grid, block, RG::SMEM, s, a);
+                else SLM_LAUNCH_PDL((row_multiplane_kernel<R, L, ALG_MP, 0>), grid, block, RG::SMEM, s, a);
             } else {
                 return -1;
             }

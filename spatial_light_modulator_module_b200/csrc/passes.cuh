@@ -339,7 +339,16 @@ SLM_GLOBAL void SLM_LAUNCH_BOUNDS((RowGeom<R, W>::THREADS), (RowGeom<R, W>::MIN_
 // has not converged.  All flags set: return; otherwise every CTA of the hologram clears them (all CTAs decide alike,
 // in any order: a flag that was clear stays clear), so the planes keep iterating together and their curves stay
 // equal in length.
-template <typename R, int W, int FINAL>
+//
+// ALG = ALG_MPGD is multi-plane GD: the planes' Fourier-plane steps are K planes of GD's column pass, and the pass
+// takes the gradient of the mean of their errors.  From Y: S = sum_k ifft2(G_k) conj(L_k) as above, then x is loaded
+// (into the registers the plane's transform has freed) and takes row_pass_kernel<ALG_GD>'s step with dEdF = S inc /
+// (K H W) (ra.inv_hw = 1 / (K H W)) and lr[iters - 1]; ROW_FROM_FIELD takes x as given (iteration 0).  Then B =
+// x rsqrt(|x|^2) inc, forward-transformed per plane as above; FINAL = 1 writes angle(x) instead.  The FINAL pass does
+// not test the flags: it applies the update of the last iteration that ran, once, as row_pass_kernel<ALG_GD> does.
+// K = 1 with alpha = 0 is row_pass_kernel<ALG_GD>'s arithmetic; the engine runs that case with row_pass_kernel itself
+// (slm_gd_multiplane_run).
+template <typename R, int W, int ALG, int FINAL>
 SLM_GLOBAL void SLM_LAUNCH_BOUNDS((RowGeom<R, W>::THREADS), (RowGeom<R, W>::MP_MIN_CTAS)) row_multiplane_kernel(RowArgs a) {
     using G = RowGeom<R, W>;
     using P = FftPlan<W>;
@@ -371,7 +380,52 @@ SLM_GLOBAL void SLM_LAUNCH_BOUNDS((RowGeom<R, W>::THREADS), (RowGeom<R, W>::MP_M
     const R* inc = static_cast<const R*>(a.inc);
     cpx<R> s[E], v[E];
 
-    if (a.source == ROW_FROM_FIELD) {
+    if constexpr (ALG == ALG_MPGD) {
+        cpx<R>* xp = static_cast<cpx<R>*>(a.x) + gbase;
+        if (a.source == ROW_FROM_Y) {
+            for (int k = 0; k < K; ++k) {
+                const cpx<R>* Y = static_cast<const cpx<R>*>(a.Y) + kbase + (size_t)k * plane;
+#pragma unroll
+                for (int r = 0; r < E; ++r) v[r] = ld_plane(Y + r * M);
+                line_fft<R, W, +1, 1>(v, line, j, tw, sync);
+                if (a.lens_mask & (1 << k)) {
+                    const cpx<R> cy = ld_const(ly + (size_t)k * a.H + y);
+#pragma unroll
+                    for (int r = 0; r < E; ++r) v[r] = cmul(v[r], cconj(cmul(cy, ld_const(lx + (size_t)k * W + r * M))));
+                }
+#pragma unroll
+                for (int r = 0; r < E; ++r) s[r] = k ? cadd(s[r], v[r]) : v[r];
+            }
+            // the update of the iteration whose Fourier-plane passes produced Y: lr of THAT iteration (the K planes of
+            // a hologram count alike)
+            const R lr = (R)ld_ro(a.lr + (ld_cg(&a.stats[(size_t)g * K].iters) - 1));
+            const R nrm = (R)a.inv_hw;
+#pragma unroll
+            for (int r = 0; r < E; ++r) v[r] = ld_plane(xp + r * M);
+#pragma unroll
+            for (int r = 0; r < E; ++r) {
+                R gs = nrm;
+                if (inc) gs *= ld_ro(inc + pix + r * M);
+                v[r] = tangent_step(v[r], cscale(s[r], gs), lr);
+                st_plane(xp + r * M, v[r]);
+            }
+        } else {
+#pragma unroll
+            for (int r = 0; r < E; ++r) v[r] = ld_plane(xp + r * M);
+        }
+        if (FINAL) {                                   // hologram = angle(x)
+            double* h = a.hologram + gbase;
+#pragma unroll
+            for (int r = 0; r < E; ++r) h[r * M] = atan2((double)v[r].y, (double)v[r].x);
+            return;
+        }
+#pragma unroll
+        for (int r = 0; r < E; ++r) {                  // B = x / |x| inc
+            R inv = rsqrt_fast(cnorm2(v[r]));
+            if (inc) inv *= ld_ro(inc + pix + r * M);
+            s[r] = cscale(v[r], inv);
+        }
+    } else if (a.source == ROW_FROM_FIELD) {
         const cpx<R>* F = static_cast<const cpx<R>*>(a.field) + gbase;
 #pragma unroll
         for (int r = 0; r < E; ++r) s[r] = ld_plane(F + r * M);
@@ -417,13 +471,13 @@ SLM_GLOBAL void SLM_LAUNCH_BOUNDS((RowGeom<R, W>::THREADS), (RowGeom<R, W>::MP_M
             }
         }
     }
-    if (FINAL) {                                       // hologram = angle(S)
+    if (FINAL) {                                       // hologram = angle(S) (GD has returned above)
         double* h = a.hologram + gbase;
 #pragma unroll
         for (int r = 0; r < E; ++r) h[r * M] = atan2((double)s[r].y, (double)s[r].x);
         return;
     }
-    if (inc && a.source != ROW_FROM_FIELD) {
+    if (ALG == ALG_MP && inc && a.source != ROW_FROM_FIELD) {
 #pragma unroll
         for (int r = 0; r < E; ++r) s[r] = cscale(s[r], ld_ro(inc + pix + r * M));
     }

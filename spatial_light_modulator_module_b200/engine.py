@@ -32,8 +32,8 @@ class LoopResult:
 
 @dataclass
 class MultiplaneResult:
-    """Results of a multi-plane GS run of G holograms with K target planes each (device buffers unless converted)."""
-    hologram: object                 # [G,H,W] float64: angle(A)
+    """Results of a multi-plane GS or GD run of G holograms with K target planes each (device buffers unless converted)."""
+    hologram: object                 # [G,H,W] float64: angle(A) (GS), angle(x) (GD)
     expected: Optional[object]       # [G,K,H,W] float64 or None: each plane's expected outcome
     errors: List[List[np.ndarray]]   # errors[g][k]: error_evolution of plane k; the K curves of a hologram have one length
     iterations: np.ndarray           # int [G]
@@ -255,7 +255,7 @@ class Engine:
     _Begun = namedtuple("_Begun", "batch t8 treal amp norms c64 inc hologram expected")
 
     def _begin(self, targets, max_loops, unbound, inc_amp, norms, want_expected, holograms=None):
-        """What gs, gsw, gs_multiplane and gd do first.  ``unbound``: the reference's variable that a run without
+        """What gs, gsw, gd and their multi-plane forms do first.  ``unbound``: the reference's variable that a run without
         iterations leaves unbound.  ``holograms``: hologram planes to allocate (default: one per target plane)."""
         if max_loops < 1:
             raise UnboundLocalError(f"cannot access local variable '{unbound}' where it is not associated with a value")
@@ -309,6 +309,36 @@ class Engine:
                            self._dp(sums), self._mem_ptr(w), float(weight_limit))
         return res, w
 
+    def _multiplane_args(self, targets, defocus, max_loops, name):
+        """What gs_multiplane, gd_multiplane and multiplane_fourier_guess check first -> (G, K, alphas, targets as
+        [G*K,H,W]).  ``name``: the algorithm the messages name.  With max_loops < 1 nothing is checked: _begin raises
+        the reference's UnboundLocalError first."""
+        shape = tuple(int(s) for s in targets.shape) if hasattr(targets, "shape") else np.shape(targets)
+        if len(shape) not in (3, 4):
+            raise ValueError(f"targets must be [K,H,W] or [G,K,H,W], not of shape {tuple(shape)}")
+        g, k = (1, shape[0]) if len(shape) == 3 else shape[:2]
+        alpha = np.ascontiguousarray(np.asarray(defocus, dtype=np.float64).reshape(-1))
+        if max_loops >= 1:
+            if alpha.shape != (k,):
+                raise ValueError(f"{k} target planes need {k} defocus coefficients, not {alpha.size}")
+            if not 1 <= k <= 8:
+                raise ValueError(f"multi-plane {name} takes 1 to 8 target planes, not {k}")
+            if g * k > self.max_batch:
+                raise ValueError(f"{g} holograms of {k} planes exceed the engine's max_batch ({self.max_batch})")
+            from . import constants
+            hl.check_defocus(alpha, self.shape, constants.px_distance, constants.wavelength)
+        flat = targets.reshape((g * k,) + tuple(shape[-2:])) if self._mem_is_device(targets) else \
+            np.asarray(targets).reshape((g * k,) + tuple(shape[-2:]))
+        return g, k, alpha, flat
+
+    def _per_hologram(self, buf, g, what):
+        """A device buffer of one plane per hologram: [G,H,W], or [H,W] for G = 1."""
+        if tuple(buf.shape) == self.shape and g == 1:
+            buf = buf.reshape((1,) + self.shape)
+        if tuple(buf.shape) != (g,) + self.shape:
+            raise ValueError(f"{what} must have shape {(g,) + self.shape}, not {tuple(buf.shape)}")
+        return buf
+
     def gs_multiplane(self, targets, defocus, max_loops: int, tolerance: float = 0.0, inc_amp=None, phasor0=None,
                       want_expected: bool = True, norms=None) -> MultiplaneResult:
         """Multi-plane GS (include/slm_holo.h slm_gs_multiplane_run): one hologram for K target planes at different
@@ -316,34 +346,19 @@ class Engine:
         shared by the holograms (host_logic.defocus_coefficient; 0 = the Fourier plane), each with |alpha_k| max(H, W)
         <= pi.  A hologram iterates while any of its planes' error is above ``tolerance``.  ``phasor0``: B of
         iteration 0, [G,H,W].  K = 1 with alpha = 0 gives :meth:`gs`'s results bit for bit."""
-        shape = tuple(int(s) for s in targets.shape) if hasattr(targets, "shape") else np.shape(targets)
-        if len(shape) not in (3, 4):
-            raise ValueError(f"targets must be [K,H,W] or [G,K,H,W], not of shape {tuple(shape)}")
-        g, k = (1, shape[0]) if len(shape) == 3 else shape[:2]
-        alpha = np.ascontiguousarray(np.asarray(defocus, dtype=np.float64).reshape(-1))
-        if max_loops >= 1:                                            # (max_loops < 1 raises first, in _begin)
-            if alpha.shape != (k,):
-                raise ValueError(f"{k} target planes need {k} defocus coefficients, not {alpha.size}")
-            if not 1 <= k <= 8:
-                raise ValueError(f"multi-plane GS takes 1 to 8 target planes, not {k}")
-            if g * k > self.max_batch:
-                raise ValueError(f"{g} holograms of {k} planes exceed the engine's max_batch ({self.max_batch})")
-            from . import constants
-            hl.check_defocus(alpha, self.shape, constants.px_distance, constants.wavelength)
-        flat = targets.reshape((g * k,) + tuple(shape[-2:])) if self._mem_is_device(targets) else \
-            np.asarray(targets).reshape((g * k,) + tuple(shape[-2:]))
+        g, k, alpha, flat = self._multiplane_args(targets, defocus, max_loops, "GS")
         b = self._begin(flat, max_loops, "expected_outcome", inc_amp, norms, want_expected, holograms=g)
         ph_dev = self._as_device(phasor0, self.complex_dtype, "phasor0")
         if ph_dev is not None:
-            if tuple(ph_dev.shape) == self.shape and g == 1:
-                ph_dev = ph_dev.reshape((1,) + self.shape)
-            if tuple(ph_dev.shape) != (g,) + self.shape:
-                raise ValueError(f"phasor0 must have shape {(g,) + self.shape}, not {tuple(ph_dev.shape)}")
+            ph_dev = self._per_hologram(ph_dev, g, "phasor0")
         amp_dev = self._mem_upload(b.amp.astype(self.real_dtype)) if b.amp is not None else None
         self._check(self._lib.slm_gs_multiplane_run(
             self._ctx, g, k, self._mem_ptr(b.t8), self._mem_ptr(b.treal), self._mem_ptr(amp_dev), self._dp(self._amp_lut),
             self._dp(b.norms), self._dp(alpha), self._mem_ptr(b.inc), self._mem_ptr(ph_dev), int(b.c64), int(max_loops),
             float(tolerance), self._mem_ptr(b.hologram), self._mem_ptr(b.expected)))
+        return self._multiplane_result(b, g, k, max_loops)
+
+    def _multiplane_result(self, b, g, k, max_loops) -> MultiplaneResult:
         res = self._collect(b.batch, max_loops, b.hologram, b.expected)
         expected = None if b.expected is None else b.expected.reshape((g, k) + self.shape)
         return MultiplaneResult(b.hologram, expected, [res.errors[i * k:(i + 1) * k] for i in range(g)],
@@ -355,23 +370,61 @@ class Engine:
         """``x0``: complex initial guess [B,H,W] (host or device; a device tensor is updated in place).
         Returns (LoopResult, x_device)."""
         b = self._begin(targets, max_loops, "output", inc_amp, norms, want_expected)
+        x = self._as_device(x0, self.complex_dtype, "x0")
+        if len(x.shape) == 2:
+            x = x[None]
+        mask_lut, mask_dev, lr = self._gd_args(b, targets, white_attention, lr_schedule, max_loops)
+        self._check(self._lib.slm_gd_run(
+            self._ctx, b.batch, self._mem_ptr(b.t8), self._mem_ptr(b.treal), self._mem_ptr(mask_dev), self._dp(mask_lut),
+            self._dp(b.norms), self._mem_ptr(b.inc), self._mem_ptr(x), self._dp(lr), int(max_loops), float(tolerance),
+            self._mem_ptr(b.hologram), self._mem_ptr(b.expected)))
+        return self._collect(b.batch, max_loops, b.hologram, b.expected), x
+
+    def _gd_args(self, b, targets, white_attention, lr_schedule, max_loops):
+        """gd and gd_multiplane after :meth:`_begin` (``b``): (mask table, device mask plane of non-8-bit targets,
+        learning-rate schedule)."""
         if b.t8 is not None:
             mask_lut, mask_dev = hl.gd_mask_lut(white_attention), None
         else:
             mask_lut = np.zeros(256)
             mask_dev = self._mem_upload(np.asarray(1 + white_attention * np.asarray(targets).reshape((b.batch,) + self.shape) / 255,
                                                    dtype=self.real_dtype))
-        x = self._as_device(x0, self.complex_dtype, "x0")
-        if len(x.shape) == 2:
-            x = x[None]
         lr = np.ascontiguousarray(lr_schedule, dtype=np.float64)
         if lr.shape != (max_loops,):
             raise ValueError("lr_schedule must have max_loops entries")
-        self._check(self._lib.slm_gd_run(
-            self._ctx, b.batch, self._mem_ptr(b.t8), self._mem_ptr(b.treal), self._mem_ptr(mask_dev), self._dp(mask_lut),
-            self._dp(b.norms), self._mem_ptr(b.inc), self._mem_ptr(x), self._dp(lr), int(max_loops), float(tolerance),
-            self._mem_ptr(b.hologram), self._mem_ptr(b.expected)))
-        return self._collect(b.batch, max_loops, b.hologram, b.expected), x
+        return mask_lut, mask_dev, lr
+
+    def gd_multiplane(self, targets, defocus, x0, lr_schedule, max_loops: int, tolerance: float = 0.0,
+                      white_attention=1, inc_amp=None, want_expected: bool = True, norms=None):
+        """Multi-plane GD (include/slm_holo.h slm_gd_multiplane_run): one hologram for K target planes at different
+        focus, by gradient descent on the mean of the planes' errors.  ``targets``, ``defocus``: as
+        :meth:`gs_multiplane`; ``x0``: one complex initial guess per hologram, [G,H,W] (or [H,W] for one hologram; a
+        device tensor is updated in place); ``lr_schedule``: max_loops learning rates shared by the holograms.  A
+        hologram iterates while any of its planes' error is above ``tolerance``.  K = 1 with alpha = 0 gives
+        :meth:`gd`'s results bit for bit.  Returns (MultiplaneResult, x_device)."""
+        g, k, alpha, flat = self._multiplane_args(targets, defocus, max_loops, "GD")
+        b = self._begin(flat, max_loops, "output", inc_amp, norms, want_expected, holograms=g)
+        x = self._per_hologram(self._as_device(x0, self.complex_dtype, "x0"), g, "x0")
+        mask_lut, mask_dev, lr = self._gd_args(b, flat, white_attention, lr_schedule, max_loops)
+        self._check(self._lib.slm_gd_multiplane_run(
+            self._ctx, g, k, self._mem_ptr(b.t8), self._mem_ptr(b.treal), self._mem_ptr(mask_dev), self._dp(mask_lut),
+            self._dp(b.norms), self._dp(alpha), self._mem_ptr(b.inc), self._mem_ptr(x), self._dp(lr), int(max_loops),
+            float(tolerance), self._mem_ptr(b.hologram), self._mem_ptr(b.expected)))
+        return self._multiplane_result(b, g, k, max_loops), x
+
+    def multiplane_fourier_guess(self, targets, defocus, inc_amp=None):
+        """The "fourier" initial guess of :meth:`gd_multiplane` on the device (include/slm_holo.h
+        slm_multiplane_fourier_guess): inc exp(i angle(sum_k ifft2(sqrt(T_k)) conj(L_k))) -> complex [G,H,W].
+        ``targets``, ``defocus``: as :meth:`gs_multiplane`."""
+        g, k, alpha, flat = self._multiplane_args(targets, defocus, 1, "GD")
+        _batch, t8, _treal, amp, _norms, c64 = self._targets(flat)
+        amp_dev = self._mem_upload(amp.astype(self.real_dtype)) if amp is not None else None
+        inc_dev = self._as_device(inc_amp, self.real_dtype, "inc_amp")
+        x = self._mem_empty((g,) + self.shape, self.complex_dtype)
+        self._check(self._lib.slm_multiplane_fourier_guess(
+            self._ctx, g, k, self._mem_ptr(t8), self._mem_ptr(amp_dev), self._dp(self._amp_lut), self._dp(alpha),
+            self._mem_ptr(inc_dev), int(c64), self._mem_ptr(x)))
+        return x
 
     def random_phasor_guess(self, u, divide_by=1.0):
         """exp(1j*2*pi*u)/divide_by on the device from a host-drawn uniform stream ``u`` [B,H,W] or [H,W]
